@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """bench.py -- images/sec of MDC-Net's batched inference hot path (encode + greedy decode) on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 1|4|5] [--global-batch G]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 1|4|5] [--global-batch G] [--dump-outputs DIR]
+
+--dump-outputs DIR: after the timed steps, the results of the last one (tokens, confidences; boxes and max IoU for --config 5) as
+float32 DIR/<name>.npy.  Weights and inputs are seeded, so two builds run with the same arguments can be compared array for array.
 
 A "step" = one batch of synthetic NEU-DET-shaped images (200x200 gray u8 -> the reference transform -> 3x224x224) through
 encoder -> cross-K/V -> greedy decode.  Default workload = BASELINE.json configs[1]: config P, B = 64 per GPU, bf16, 99 new tokens.
@@ -316,8 +319,21 @@ def roofline_probe(M, dev, peaks, B):
 PIPE_KW = {}          # --decode-streams / --depth: GenerationPipeline operating point (defaults: 4 streams, 6 plans)
 
 
-def run_workload(M, wl, B, steps, warmup, dev, rank, world, dist, peaks, full):
-    """Returns the fields of one bench line for workload `wl` at per-rank batch B.  full: also serial / e2e / roofline extras."""
+def dump_outputs(M, d, last, T1, C, NB):
+    """Writes one step's packed results (every rank's rows) as float32 arrays DIR/<name>.npy: the tokens and confidences a caller of
+    the batch pipeline receives, and for the box workload the decoded boxes and their max IoU against the ground truth."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    tokens, confs, boxes, max_iou = M.parallel.unpack_results(last, T1, C, NB)
+    arrays = {"tokens": tokens, "confidences": confs, "boxes": boxes, "max_iou": max_iou}
+    for name, a in arrays.items():
+        if a is not None:
+            np.save(os.path.join(d, name + ".npy"), a.cpu().to(torch.float32).numpy())     # token ids < 2^24: exact in float32
+
+
+def run_workload(M, wl, B, steps, warmup, dev, rank, world, dist, peaks, full, dump=None):
+    """Returns the fields of one bench line for workload `wl` at per-rank batch B.  full: also serial / e2e / roofline extras.
+    dump: directory for the results of the last timed step (dump_outputs)."""
     T, S, img, top_k = wl["T"], wl["S"], wl["img"], wl["top_k"]
     geo = {k: wl[k] for k in ("dim", "heads", "layers", "vocab") if k in wl}
     model = build_model(M, img=img, S=S, max_len=wl["max_len"], **geo).to(dev).set_precision("bf16")
@@ -338,7 +354,8 @@ def run_workload(M, wl, B, steps, warmup, dev, rank, world, dist, peaks, full):
         gt[torch.rand(B, 5, generator=gg) < 0.3] = 0
         gt = gt.to(dev)
     pipe = M.GenerationPipeline(model, B, T, top_k=top_k, **PIPE_KW)
-    F = T1 + C + ((5 * max(1, (T1 + 4) // 5)) if with_boxes else 0)
+    NB = max(1, (T1 + 4) // 5) if with_boxes else 0          # box slots per image (Tokenizer.decode_bboxes_padded)
+    F = T1 + C + 5 * NB
 
     def steps_pipelined(k, sink):
         """k steps through the batch pipeline; every step packs its results (tokens, confidences[, boxes + max IoU]) into its rows of
@@ -377,6 +394,8 @@ def run_workload(M, wl, B, steps, warmup, dev, rank, world, dist, peaks, full):
     if world > 1:
         dist.barrier()
     clocks = sampler.stop()
+    if dump and rank == 0:                           # rows of the gathered buffer: rank-major, then step, then image
+        dump_outputs(M, dump, out.view(world, steps, B, F)[:, -1].reshape(world * B, F), T1, C, NB)
     t = torch.tensor([pa.elapsed_time(pb)], dtype=torch.float64, device=dev)
     mine = torch.tensor([pa.elapsed_time(pb), pa.elapsed_time(steps_pipelined.pre_gather)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -446,7 +465,8 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--decode-streams", type=int, default=0)
     ap.add_argument("--depth", type=int, default=0)
-    ap.add_argument("--steps", type=int, default=100)      # 100 steps ~ 0.5 s pipelined: the fill and drain of the 6-deep pipeline (~8 ms) stay below 2 %
+    # default 100 steps (~0.5 s pipelined: the fill and drain of the 6-deep pipeline, ~8 ms, stay below 2 %) for config 1, 20 for the others
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (batches) of the workload")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", type=int, default=1, choices=[1, 4, 5, 6], help="1: BASELINE configs[1] (default; configs[2] under torchrun), 4: configs[3], 5: configs[4], 6: the trained geometry (dim 1024)")
@@ -454,7 +474,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--profile", action="store_true", help="1 warm-up + 1 serial step only (for an ncu launch list)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 100 if args.config == 1 else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.profile):
+        ap.error("--dump-outputs writes the results of the batch pipeline: not with --impl reference or --profile")
     if args.decode_streams:
         PIPE_KW["decode_streams"] = args.decode_streams
     if args.depth:
@@ -507,8 +534,8 @@ def main():
         print(json.dumps({"profile_step_launches": int(M._lib.launch_count(dev) - n0)}))
         return
 
-    steps = args.steps if args.config == 1 else min(args.steps, 20)
-    res, model, xs_dev = run_workload(M, wl, B, steps, args.warmup, dev, rank, world, dist, peaks, full=(args.config == 1))
+    steps = args.steps
+    res, model, xs_dev = run_workload(M, wl, B, steps, args.warmup, dev, rank, world, dist, peaks, full=(args.config == 1), dump=args.dump_outputs)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
