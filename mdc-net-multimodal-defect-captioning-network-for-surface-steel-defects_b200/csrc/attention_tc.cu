@@ -13,28 +13,6 @@ namespace {
 
 constexpr int HD = 64;
 
-__device__ __forceinline__ void mma16816(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void ldsm_x4(uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3, uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_trans(uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3, uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ float ex2_fast(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }   // exp2f() adds denormal range handling the softmax does not need
-// byte offset of 16-byte chunk `c` (0..7) of row `r` in a swizzled [rows][64 bf16] panel
-__device__ __forceinline__ uint32_t swz(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
-
-__device__ __forceinline__ void cp_async16(uint32_t smem_dst, const void* gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gsrc) : "memory");
-}
-
 // One CTA = one (strip, head, chunk of up to 208 queries): 13 warps x 16 queries, compiled for TWO CTAs per SM (<= 72 registers), so
 // one CTA's K/V fetch overlaps the other's MMAs.  Keys are consumed in chunks of up to 208 staged in shared memory (a 197-token
 // ViT strip is one chunk and one query chunk -- the common case; a 1025-token strip of a 512x512 input is 5 x 5), the online
@@ -49,7 +27,7 @@ attn_tc_kernel(const bf16* __restrict__ qkv, int64_t ld, bf16* __restrict__ out,
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bf16* base = qkv + (int64_t)strip * S * ld + head * HD;
   const int D = H * HD;
-  const uint32_t ks_u32 = (uint32_t)__cvta_generic_to_shared(Ks), vs_u32 = (uint32_t)__cvta_generic_to_shared(Vs);
+  const uint32_t ks_u32 = smem_u32(Ks), vs_u32 = smem_u32(Vs);
   // Q fragments straight from global memory (A operand layout of m16n8k16)
   const int q0 = blockIdx.z * QCHUNK + warp * 16, r0 = q0 + (lane >> 2), r1 = r0 + 8;
   const bool active = q0 < S;           // warps past the strip's end only help staging
@@ -74,14 +52,14 @@ attn_tc_kernel(const bf16* __restrict__ qkv, int64_t ld, bf16* __restrict__ out,
   for (int i = tid; i < KC * 8; i += blockDim.x) {
     const int r = i >> 3, c = i & 7, gr = kc0 + r;
     if (gr < S) {
-      cp_async16(ks_u32 + swz(r, c), base + (int64_t)gr * ld + D + c * 8);
-      cp_async16(vs_u32 + swz(r, c), base + (int64_t)gr * ld + 2 * D + c * 8);
+      cp_async16(ks_u32 + swz<HD>(r, c), base + (int64_t)gr * ld + D + c * 8);
+      cp_async16(vs_u32 + swz<HD>(r, c), base + (int64_t)gr * ld + 2 * D + c * 8);
     } else {
-      *reinterpret_cast<uint4*>(Ks + swz(r, c)) = make_uint4(0, 0, 0, 0);
-      *reinterpret_cast<uint4*>(Vs + swz(r, c)) = make_uint4(0, 0, 0, 0);
+      *reinterpret_cast<uint4*>(Ks + swz<HD>(r, c)) = make_uint4(0, 0, 0, 0);
+      *reinterpret_cast<uint4*>(Vs + swz<HD>(r, c)) = make_uint4(0, 0, 0, 0);
     }
   }
-  asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
+  cp_async_wait_all();
   __syncthreads();
   const int nblk = active ? (min(KC, S - kc0) + 15) / 16 : 0;
   for (int kb = 0; kb < nblk; ++kb) {
@@ -94,10 +72,10 @@ attn_tc_kernel(const bf16* __restrict__ qkv, int64_t ld, bf16* __restrict__ out,
       for (int kp = 0; kp < 2; ++kp) {        // two k-steps (32 dims) per ldmatrix.x4
         // matrices: (dims 32kp..+7), (+8..15), (+16..23), (+24..31) of keys key0+8nt+0..7
         const int krow = lk0 + nt * 8 + (lane & 7), chunk = kp * 4 + (lane >> 3);
-        uint32_t b0, b1, b2, b3;
-        ldsm_x4(b0, b1, b2, b3, ks_base + swz(krow, chunk));
-        mma16816(s[nt], qa[2 * kp], b0, b1);
-        mma16816(s[nt], qa[2 * kp + 1], b2, b3);
+        uint32_t kf[4];
+        ldsm_x4(kf, ks_base + swz<HD>(krow, chunk));
+        mma_m16n8k16<bf16>(s[nt], qa[2 * kp], kf[0], kf[1]);
+        mma_m16n8k16<bf16>(s[nt], qa[2 * kp + 1], kf[2], kf[3]);
       }
     }
     // ---- mask + online softmax (exp2 domain) ------------------------------------------------------------------
@@ -112,14 +90,14 @@ attn_tc_kernel(const bf16* __restrict__ qkv, int64_t ld, bf16* __restrict__ out,
     mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1)); mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
     mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1)); mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
     const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);          // finite: key 0 of the first block is always valid
-    const float c0 = ex2_fast((m0 - mn0) * scale_log2e), c1 = ex2_fast((m1 - mn1) * scale_log2e);
+    const float c0 = ex2_approx((m0 - mn0) * scale_log2e), c1 = ex2_approx((m1 - mn1) * scale_log2e);
     m0 = mn0; m1 = mn1;
     const float ms0 = mn0 * scale_log2e, ms1 = mn1 * scale_log2e;
     float p[2][4];
 #pragma unroll
     for (int nt = 0; nt < 2; ++nt) {
-      p[nt][0] = ex2_fast(fmaf(s[nt][0], scale_log2e, -ms0)); p[nt][1] = ex2_fast(fmaf(s[nt][1], scale_log2e, -ms0));
-      p[nt][2] = ex2_fast(fmaf(s[nt][2], scale_log2e, -ms1)); p[nt][3] = ex2_fast(fmaf(s[nt][3], scale_log2e, -ms1));
+      p[nt][0] = ex2_approx(fmaf(s[nt][0], scale_log2e, -ms0)); p[nt][1] = ex2_approx(fmaf(s[nt][1], scale_log2e, -ms0));
+      p[nt][2] = ex2_approx(fmaf(s[nt][2], scale_log2e, -ms1)); p[nt][3] = ex2_approx(fmaf(s[nt][3], scale_log2e, -ms1));
     }
     l0 = l0 * c0 + (p[0][0] + p[0][1]) + (p[1][0] + p[1][1]);
     l1 = l1 * c1 + (p[0][2] + p[0][3]) + (p[1][2] + p[1][3]);
@@ -129,16 +107,16 @@ attn_tc_kernel(const bf16* __restrict__ qkv, int64_t ld, bf16* __restrict__ out,
     }
     // ---- O += P V : P is the A operand (rows = queries, k = these 16 keys) -----------------------------------------
     uint32_t pa[4];
-    pa[0] = pack_bf16(p[0][0], p[0][1]); pa[1] = pack_bf16(p[0][2], p[0][3]);
-    pa[2] = pack_bf16(p[1][0], p[1][1]); pa[3] = pack_bf16(p[1][2], p[1][3]);
+    pa[0] = pack_bf16x2(p[0][0], p[0][1]); pa[1] = pack_bf16x2(p[0][2], p[0][3]);
+    pa[2] = pack_bf16x2(p[1][0], p[1][1]); pa[3] = pack_bf16x2(p[1][2], p[1][3]);
 #pragma unroll
     for (int dp = 0; dp < 4; ++dp) {           // two 8-wide dim tiles per ldmatrix.x4.trans
       // matrices: (keys key0..+7, dims 16dp..+7), (keys +8..15, same dims), (keys key0..+7, dims 16dp+8..), (keys +8..15, dims 16dp+8..)
       const int vrow = lk0 + (lane & 7) + ((lane >> 3) & 1) * 8, chunk = dp * 2 + (lane >> 4);
-      uint32_t b0, b1, b2, b3;
-      ldsm_x4_trans(b0, b1, b2, b3, vs_base + swz(vrow, chunk));
-      mma16816(o[2 * dp], pa, b0, b1);
-      mma16816(o[2 * dp + 1], pa, b2, b3);
+      uint32_t vf[4];
+      ldsm_x4_trans(vf, vs_base + swz<HD>(vrow, chunk));
+      mma_m16n8k16<bf16>(o[2 * dp], pa, vf[0], vf[1]);
+      mma_m16n8k16<bf16>(o[2 * dp + 1], pa, vf[2], vf[3]);
     }
   }
   }
@@ -149,8 +127,8 @@ attn_tc_kernel(const bf16* __restrict__ qkv, int64_t ld, bf16* __restrict__ out,
   bf16* ob = out + (int64_t)strip * S * ldo + head * HD + 2 * (lane & 3);
 #pragma unroll
   for (int dt = 0; dt < 8; ++dt) {
-    if (r0 < S) *reinterpret_cast<uint32_t*>(ob + (int64_t)r0 * ldo + dt * 8) = pack_bf16(o[dt][0] * i0, o[dt][1] * i0);
-    if (r1 < S) *reinterpret_cast<uint32_t*>(ob + (int64_t)r1 * ldo + dt * 8) = pack_bf16(o[dt][2] * i1, o[dt][3] * i1);
+    if (r0 < S) *reinterpret_cast<uint32_t*>(ob + (int64_t)r0 * ldo + dt * 8) = pack_bf16x2(o[dt][0] * i0, o[dt][1] * i0);
+    if (r1 < S) *reinterpret_cast<uint32_t*>(ob + (int64_t)r1 * ldo + dt * 8) = pack_bf16x2(o[dt][2] * i1, o[dt][3] * i1);
   }
 }
 
@@ -169,10 +147,10 @@ int attn_tc_launch(mdc_ctx* ctx, const void* qkv, int64_t ld, void* out, int64_t
   dim3 grid(heads, n_strips, q_chunks), block(32 * (KC / 16));
   if (q_chunks == 1) {
     MDC_ENSURE_SMEM(attn_tc_kernel<false>, smem);
-    attn_tc_kernel<false><<<grid, block, smem, s>>>((const bf16*)qkv, ld, (bf16*)out, ldo, strip_len, heads, scale * 1.4426950408889634f, KC);
+    attn_tc_kernel<false><<<grid, block, smem, s>>>((const bf16*)qkv, ld, (bf16*)out, ldo, strip_len, heads, scale * LOG2E, KC);
   } else {
     MDC_ENSURE_SMEM(attn_tc_kernel<true>, smem);
-    attn_tc_kernel<true><<<grid, block, smem, s>>>((const bf16*)qkv, ld, (bf16*)out, ldo, strip_len, heads, scale * 1.4426950408889634f, KC);
+    attn_tc_kernel<true><<<grid, block, smem, s>>>((const bf16*)qkv, ld, (bf16*)out, ldo, strip_len, heads, scale * LOG2E, KC);
   }
   MDC_LAUNCH_CHECK(ctx);
   return 0;

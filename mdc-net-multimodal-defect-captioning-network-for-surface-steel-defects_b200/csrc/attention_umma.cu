@@ -24,87 +24,6 @@ constexpr int QROWS = 256;                 // query rows staged per item (two 12
 constexpr int N_SOFTMAX_WARPS = 16;
 constexpr int THREADS = 64 + N_SOFTMAX_WARPS * 32;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) { asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory"); }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
-// bounded wait (sleeping try_wait): a protocol bug traps instead of hanging the GPU box
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (true) {
-    asm volatile("{\n\t.reg .pred P1;\n\tmbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, P1;\n\t}\n"
-                 : "=r"(done) : "r"(bar), "r"(parity), "r"(1000000u) : "memory");
-    if (done) break;
-    if (++spins > 2000u) __trap();
-  }
-}
-__device__ __forceinline__ void tma_load_2d(const CUtensorMap* map, uint32_t bar, uint32_t dst, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-               ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// D[tmem] (+)= A[smem desc] . B[smem desc]
-__device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-               ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-// D[tmem] (+)= A[tmem] . B[smem desc]
-__device__ __forceinline__ void umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n"
-               ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t addr, uint32_t* v) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]) : "r"(addr));
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t addr, uint32_t* v) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-               "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-               "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                 "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-                 "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-                 "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-               : "r"(addr));
-}
-__device__ __forceinline__ void tmem_ld4(uint32_t addr, uint32_t* v) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(addr));
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t addr, uint32_t* v) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                 "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]) : "r"(addr));
-}
-__device__ __forceinline__ void tmem_st2(uint32_t addr, uint32_t a, uint32_t b) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_st4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ float ex2a(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) { __nv_bfloat162 h = __floats2bfloat162_rn(a, b); return *reinterpret_cast<uint32_t*>(&h); }
-
-// SWIZZLE_128B operand tile: rows of 128 B, 8-row groups 1024 B apart (SBO).  K-major use (Q, K): the rows are the M / N index;
-// MN-major use (V, selected by the instruction descriptor's transpose bit): the rows are the K index, the 64 elements of a row the N index.
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-// kind::f16 instruction descriptor: D = f32, A = B = bf16, N >> 3 at bit 17, M >> 4 at bit 24; bit 16 = B is MN-major
-__device__ __forceinline__ uint32_t make_idesc(int M, int N, bool b_mn_major) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((b_mn_major ? 1u : 0u) << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
 struct SmemLayout {          // per item buffer: Q | K | V, each 1024-aligned
   int q_bytes, kv_bytes, buf_bytes;
 };
@@ -134,13 +53,13 @@ attn_umma_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constan
       mbar_init(smem_u32(&full[i]), 1); mbar_init(smem_u32(&sfree[i]), 1); mbar_init(smem_u32(&s_ready[i]), 1);
       mbar_init(smem_u32(&p_ready[i]), N_SOFTMAX_WARPS * 32); mbar_init(smem_u32(&o_ready[i]), 1); mbar_init(smem_u32(&t_free[i]), N_SOFTMAX_WARPS * 32);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_q) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_kv) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&map_q);
+    prefetch_tmap(&map_kv);
   }
   if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr_smem)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(smem_u32(tmem_ptr_smem), 512);
+    tmem_relinquish<1>();
   }
   tc_fence_before();
   __syncthreads();
@@ -167,7 +86,7 @@ attn_umma_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constan
   } else if (warp == 0) {
     // ===== MMA issuer (one thread) =====
     if (lane == 0) {
-      const uint32_t idesc_qk = make_idesc(128, NK, false), idesc_pv = make_idesc(128, HD, true);
+      const uint32_t idesc_qk = make_idesc(128, NK), idesc_pv = make_idesc(128, HD, false, true);
       int n = 0;
       for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++n) {
         const int buf = n & 1;
@@ -175,17 +94,17 @@ attn_umma_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constan
         mbar_wait(smem_u32(&full[buf]), (n >> 1) & 1);
         STAMP(1);
         tc_fence_after();
-        const uint64_t kdesc = make_desc(base + q_bytes);
+        const uint64_t kdesc = make_sw128_desc(base + q_bytes);
         for (int t = 0; t < tiles; ++t) {
           mbar_wait(smem_u32(&t_free[t]), (n & 1) ^ 1);           // the previous item's epilogue has drained this tile's TMEM region
           tc_fence_after();
-          const uint64_t qdesc = make_desc(base + t * 128 * 128);
+          const uint64_t qdesc = make_sw128_desc(base + t * 128 * 128);
 #pragma unroll
           for (int k = 0; k < HD / 16; ++k) umma_ss(tmem_base + t * 256, qdesc + 2 * k, kdesc + 2 * k, idesc_qk, k != 0);
           umma_commit(smem_u32(&s_ready[t]));
           STAMP(2 + t);
         }
-        const uint64_t vdesc = make_desc(base + q_bytes + kv_bytes);
+        const uint64_t vdesc = make_sw128_desc(base + q_bytes + kv_bytes);
         for (int t = 0; t < tiles; ++t) {
           mbar_wait(smem_u32(&p_ready[t]), n & 1);
           STAMP(4 + t);
@@ -268,7 +187,7 @@ attn_umma_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constan
         }
         float mx = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
         xch[part * 128 + row] = mx;
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + (warp & 3)) : "memory");       // the four warps of this lane quarter: every part of these rows has its scores in registers
+        bar_sync<128>(1 + (warp & 3));       // the four warps of this lane quarter: every part of these rows has its scores in registers
         if (threadIdx.x == 64) STAMP(12 + 8 * t);
         mx = fmaxf(fmaxf(xch[row], xch[128 + row]), fmaxf(xch[256 + row], xch[384 + row]));      // finite: column 0 is a valid key
         const float nms = -mx * scale_log2e;
@@ -279,8 +198,8 @@ attn_umma_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constan
             if (c < nch) {
               float p[4];
 #pragma unroll
-              for (int j = 0; j < 4; ++j) { p[j] = ex2a(fmaf(s[4 * c + j], scale_log2e, nms)); s4[j] += p[j]; }
-              tmem_st2(trow + (part * qc) / 2 + 2 * c, pack_bf16(p[0], p[1]), pack_bf16(p[2], p[3]));
+              for (int j = 0; j < 4; ++j) { p[j] = ex2_approx(fmaf(s[4 * c + j], scale_log2e, nms)); s4[j] += p[j]; }
+              tmem_st2(trow + (part * qc) / 2 + 2 * c, pack_bf16x2(p[0], p[1]), pack_bf16x2(p[2], p[3]));
             }
         }
         const float sum = (s4[0] + s4[1]) + (s4[2] + s4[3]);
@@ -291,7 +210,7 @@ attn_umma_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constan
         if (threadIdx.x == 64) STAMP(14 + 8 * t);
         tc_fence_before();
         mbar_arrive(smem_u32(&p_ready[t]));
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + (warp & 3)) : "memory");       // the maxima in xch are reused by the next tile
+        bar_sync<128>(1 + (warp & 3));       // the maxima in xch are reused by the next tile
       }
       for (int t = 0; t < tiles; ++t) {
         mbar_wait(smem_u32(&o_ready[t]), n & 1);
@@ -311,23 +230,23 @@ attn_umma_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constan
 #pragma unroll
           for (int j = 0; j < 16; j += 8) {
             uint4 v;
-            v.x = pack_bf16(__uint_as_float(o[j]) * inv, __uint_as_float(o[j + 1]) * inv);
-            v.y = pack_bf16(__uint_as_float(o[j + 2]) * inv, __uint_as_float(o[j + 3]) * inv);
-            v.z = pack_bf16(__uint_as_float(o[j + 4]) * inv, __uint_as_float(o[j + 5]) * inv);
-            v.w = pack_bf16(__uint_as_float(o[j + 6]) * inv, __uint_as_float(o[j + 7]) * inv);
+            v.x = pack_bf16x2(__uint_as_float(o[j]) * inv, __uint_as_float(o[j + 1]) * inv);
+            v.y = pack_bf16x2(__uint_as_float(o[j + 2]) * inv, __uint_as_float(o[j + 3]) * inv);
+            v.z = pack_bf16x2(__uint_as_float(o[j + 4]) * inv, __uint_as_float(o[j + 5]) * inv);
+            v.w = pack_bf16x2(__uint_as_float(o[j + 6]) * inv, __uint_as_float(o[j + 7]) * inv);
             *reinterpret_cast<uint4*>(dst + j) = v;
           }
         }
       }
       if (threadIdx.x == 64) STAMP(30);
-      asm volatile("bar.sync %0, 128;" ::"r"(1 + (warp & 3)) : "memory");         // the row sums in xch are reused by the next item
+      bar_sync<128>(1 + (warp & 3));         // the row sums in xch are reused by the next item
     }
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+    tmem_dealloc<1>(tmem_base, 512);
   }
 }
 
@@ -355,7 +274,7 @@ int attn_umma_launch(mdc_ctx* ctx, const void* qkv, int64_t ld, void* out, int64
 #ifdef MDC_DEVTOOLS
   if (const char* e = getenv("MDC_ATTN_TRACE_PTR")) dbg = (long long*)strtoull(e, nullptr, 0);
 #endif
-  attn_umma_kernel<<<grid, THREADS, smem, s>>>(mq, mkv, (bf16*)out, ldo, n_items, S, heads, NK, scale * 1.4426950408889634f, dbg);
+  attn_umma_kernel<<<grid, THREADS, smem, s>>>(mq, mkv, (bf16*)out, ldo, n_items, S, heads, NK, scale * LOG2E, dbg);
   MDC_LAUNCH_CHECK(ctx);
   return 0;
 }

@@ -8,8 +8,11 @@
 #include <stdarg.h>
 #include <math.h>
 #include "../../include/mdc_b200.h"
+#include "ptx.cuh"
 
 typedef __nv_bfloat16 bf16;
+
+constexpr float LOG2E = 1.4426950408889634f;
 
 // ---- error plumbing ------------------------------------------------------------------------
 void mdc_set_error(const char* fmt, ...);
@@ -56,6 +59,12 @@ template <> __device__ __forceinline__ float to_f<bf16>(bf16 v) { return __bfloa
 template <typename T> __device__ __forceinline__ T from_f(float v);
 template <> __device__ __forceinline__ float from_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ bf16 from_f<bf16>(float v) { return __float2bfloat16_rn(v); }
+
+// IEEE half operands and outputs (DESIGN 3.7): clamped to the finite range, then rounded to nearest.  fp16 has 11 significant bits, 8x
+// finer than bf16: tools/error_budget_cpu.py "activations fp16" moves the logit error by < 3e-4, where bf16 activations would cost 1.4e-2
+__device__ __forceinline__ float clamp_f16_range(float v) { return fminf(fmaxf(v, -65504.f), 65504.f); }
+__device__ __forceinline__ __half f16_sat(float v) { return __float2half_rn(clamp_f16_range(v)); }
+__device__ __forceinline__ uint32_t pack_f16x2_sat(float a, float b) { return pack_f16x2(clamp_f16_range(a), clamp_f16_range(b)); }
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

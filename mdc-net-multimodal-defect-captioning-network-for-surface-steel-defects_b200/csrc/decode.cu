@@ -86,11 +86,6 @@ __device__ __forceinline__ void load_x_tile(const XSrc& xs, float* Xs, int b0, i
 //   PLAIN : cp.async 16-byte chunks straight into shared memory
 //   LN    : a warp owns rows (warp, warp+8); both rows' residual+delta slices are loaded as float4 first
 //   EMBED : token ids first (one round trip), then both embedding rows + the positional row
-__device__ __forceinline__ void cp_async16(float* smem_dst, const float* gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory"); }
-
 template <int K>
 __device__ __forceinline__ void load_x_tile_fast(const XSrc& xs, float* Xs, int b0, int B, bool publish) {
   static_assert(K % 128 == 0, "K must be a multiple of 128");
@@ -101,7 +96,7 @@ __device__ __forceinline__ void load_x_tile_fast(const XSrc& xs, float* Xs, int 
 #pragma unroll 8
     for (int i = threadIdx.x; i < BT * CH; i += LIN_THREADS) {
       const int r = i / CH, c4 = i - r * CH, b = b0 + r;
-      if (b < B) cp_async16(Xs + (size_t)r * K + c4 * 4, xs.x + (int64_t)b * xs.ldx + c4 * 4);
+      if (b < B) cp_async16(smem_u32(Xs + (size_t)r * K + c4 * 4), xs.x + (int64_t)b * xs.ldx + c4 * 4);
       else *reinterpret_cast<float4*>(Xs + (size_t)r * K + c4 * 4) = make_float4(0, 0, 0, 0);
     }
     cp_async_wait_all();
@@ -327,14 +322,6 @@ constexpr int MMA_IMGS = 64;       // images per CTA
 constexpr int MMA_KC = 1024;       // operand columns held in shared memory at a time
 constexpr int MMA_PAD = 4;         // halves of row padding: row pitch = 2 words mod 32 (two-way conflicts at worst on the 8-byte loads)
 
-__device__ __forceinline__ void mma16816_f16(float* c, uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint32_t pack_half2(float a, float b) {
-  __half2 h = __floats2half2_rn(fminf(fmaxf(a, -65504.f), 65504.f), fminf(fmaxf(b, -65504.f), 65504.f)); return *reinterpret_cast<uint32_t*>(&h);
-}
-
 // LayerNorm-on-load / embedding operand rows, built ONCE per linear (one warp per image, all images in parallel) as IEEE half in
 // global memory, and published as the next residual (xn_out, f32).  Building them inside every CTA of the linear -- eight rows per
 // warp, one after the other, three dependent memory round trips each -- was 75 % of that kernel's time (ncu, profiles/r2w).
@@ -393,7 +380,7 @@ __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_vec_kernel(XSrc xs, _
   float4* of = xs.xn_out ? reinterpret_cast<float4*>(xs.xn_out + (int64_t)b * K) + lane : nullptr;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
-    oh[32 * i] = make_uint2(pack_half2(v[i].x, v[i].y), pack_half2(v[i].z, v[i].w));
+    oh[32 * i] = make_uint2(pack_f16x2_sat(v[i].x, v[i].y), pack_f16x2_sat(v[i].z, v[i].w));
     if (of) of[32 * i] = v[i];
   }
 }
@@ -425,14 +412,10 @@ __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_kernel(XSrc xs, __hal
   for (int i = 0; i < MMA_KC / 32; ++i) {
     const int c = lane + 32 * i;
     if (c < K) {
-      xh[(int64_t)b * K + c] = __float2half_rn(fminf(fmaxf(v[i], -65504.f), 65504.f));
+      xh[(int64_t)b * K + c] = f16_sat(v[i]);
       if (xs.xn_out) xs.xn_out[(int64_t)b * K + c] = v[i];
     }
   }
-}
-
-__device__ __forceinline__ void cp_async8(void* smem_dst, const void* gsrc) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
 }
 
 // operand rows b0 .. b0+63, columns [k0, k0+kc) -> Xh[64][kc + MMA_PAD] (fp16); rows >= B are zero.
@@ -446,7 +429,7 @@ __device__ __forceinline__ void build_x_half(const XSrc& xs, __half* Xh, int b0,
       const int b = b0 + r;
       __half* dst = Xh + (size_t)r * pitch;
       const __half* src = xs.xh + (int64_t)min(b, B - 1) * K + k0;
-      if (b < B) { for (int c = lane * 4; c < kc; c += 128) cp_async8(dst + c, src + c); }
+      if (b < B) { for (int c = lane * 4; c < kc; c += 128) cp_async8(smem_u32(dst + c), src + c); }
       else { for (int c = lane * 4; c < kc; c += 128) *reinterpret_cast<uint2*>(dst + c) = make_uint2(0u, 0u); }
     }
     cp_async_wait_all();
@@ -469,7 +452,7 @@ __device__ __forceinline__ void build_x_half(const XSrc& xs, __half* Xh, int b0,
       for (int i = 0; i < MMA_KC / 128; ++i) {
         const int c = lane * 4 + 128 * i;
         if (c < kc) {
-          *reinterpret_cast<uint2*>(row + c) = b < B ? make_uint2(pack_half2(v[h][i].x, v[h][i].y), pack_half2(v[h][i].z, v[h][i].w)) : make_uint2(0u, 0u);
+          *reinterpret_cast<uint2*>(row + c) = b < B ? make_uint2(pack_f16x2_sat(v[h][i].x, v[h][i].y), pack_f16x2_sat(v[h][i].z, v[h][i].w)) : make_uint2(0u, 0u);
           if (publish && xs.xn_out && b < B) *reinterpret_cast<float4*>(xs.xn_out + (int64_t)b * K + k0 + c) = v[h][i];
         }
       }
@@ -515,8 +498,9 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_mma_kernel(XSrc xs, co
           for (int nb = 0; nb < 4; ++nb) {
             const uint2 x0 = *reinterpret_cast<const uint2*>(xb + (size_t)(8 * nb) * pitch + 32 * kb);
             const uint2 x1 = *reinterpret_cast<const uint2*>(xb + (size_t)(8 * nb) * pitch + 32 * kb + 4);
-            mma16816_f16(acc[nb], lo.x, hi.x, lo.y, hi.y, x0.x, x0.y);
-            mma16816_f16(acc[nb], lo.z, hi.z, lo.w, hi.w, x1.x, x1.y);
+            const uint32_t a0[4] = {lo.x, hi.x, lo.y, hi.y}, a1[4] = {lo.z, hi.z, lo.w, hi.w};
+            mma_m16n8k16<__half>(acc[nb], a0, x0.x, x0.y);
+            mma_m16n8k16<__half>(acc[nb], a1, x1.x, x1.y);
           }
         }
       }
@@ -563,10 +547,6 @@ constexpr int STREAM_SLOTS = 4;              // 32-column operand blocks in flig
 constexpr int STREAM_SLOT_BYTES = MMA_IMGS * 64;                                   // [64 images][32 halves]
 constexpr int STREAM_SMEM = LIN_WARPS * STREAM_SLOTS * STREAM_SLOT_BYTES;          // 128 KB; the partial tiles alias it afterwards
 
-__device__ __forceinline__ void cp_async16_cg(uint32_t smem_dst, const void* gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gsrc) : "memory");
-}
-
 // MT = 16-row tiles per CTA.  Two tiles share every operand fragment read and halve the CTA count: the same kernel latency for half the SM
 // residency, which is what the batch pipeline (several batches' chains side by side, one such CTA per SM) is bound by.
 template <bool RELU, int MT>
@@ -598,9 +578,9 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_stream_kernel(const __
   // linear and the one or two small kernels behind it run: its weight requests then cost an L2 round trip instead of an HBM one
   if (pf != nullptr && blockIdx.y == 0)
     for (int i = blockIdx.x * LIN_THREADS + threadIdx.x; i < pf_lines; i += gridDim.x * LIN_THREADS)
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(pf + (size_t)i * 128));
+      prefetch_l2(pf + (size_t)i * 128);
   // operand ring of this warp: slot = [64 images][4 x 16 bytes]; lane l copies the 16-byte pieces l, l + 32, ... (piece = 4 image + part)
-  const uint32_t ring = (uint32_t)__cvta_generic_to_shared(stream_smem) + warp * (STREAM_SLOTS * STREAM_SLOT_BYTES);
+  const uint32_t ring = smem_u32(stream_smem) + warp * (STREAM_SLOTS * STREAM_SLOT_BYTES);
   // image slots past the batch are zeroed once and never copied (clamping them to the last row made thousands of L2 requests hit the
   // same two sectors: a B = 16 step was twice as slow as a B = 64 step)
   const __half* xsrc[8];
@@ -613,7 +593,7 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_stream_kernel(const __
     else {
 #pragma unroll
       for (int sl = 0; sl < STREAM_SLOTS; ++sl)
-        asm volatile("st.shared.v4.b32 [%0], {%1,%1,%1,%1};" ::"r"(ring + sl * STREAM_SLOT_BYTES + piece * 16), "r"(0u) : "memory");
+        sts128(ring + sl * STREAM_SLOT_BYTES + piece * 16, 0u, 0u, 0u, 0u);
     }
   }
   auto fetch = [&](int it) {
@@ -621,9 +601,9 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_stream_kernel(const __
       const uint32_t dst = ring + (it % STREAM_SLOTS) * STREAM_SLOT_BYTES + lane * 16;
 #pragma unroll
       for (int j = 0; j < 8; ++j)
-        if (live >> j & 1) cp_async16_cg(dst + 512 * j, xsrc[j] + 256 * it);
+        if (live >> j & 1) cp_async16(dst + 512 * j, xsrc[j] + 256 * it);
     }
-    asm volatile("cp.async.commit_group;" ::: "memory");                    // one group per block, empty past the end
+    cp_async_commit();                                                      // one group per block, empty past the end
   };
 #pragma unroll
   for (int i = 0; i < STREAM_SLOTS; ++i) fetch(i);
@@ -643,17 +623,17 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_stream_kernel(const __
           lo[m] = alo[m][i]; hi[m] = ahi[m][i];
           if (it + PF < nkb) { alo[m][i] = __ldg(reinterpret_cast<const uint4*>(wa[m] + 256 * (it + PF))); ahi[m][i] = __ldg(reinterpret_cast<const uint4*>(wb[m] + 256 * (it + PF))); }
         }
-        asm volatile("cp.async.wait_group %0;" ::"n"(STREAM_SLOTS - 1) : "memory");
+        cp_async_wait<STREAM_SLOTS - 1>();
         __syncwarp();
         const uint32_t src = ring + (it % STREAM_SLOTS) * STREAM_SLOT_BYTES + g * 64 + q * 16;
 #pragma unroll
         for (int nb = 0; nb < 8; ++nb) {
-          uint4 xv;
-          asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(xv.x), "=r"(xv.y), "=r"(xv.z), "=r"(xv.w) : "r"(src + 512 * nb));
+          const uint4 xv = lds128(src + 512 * nb);
 #pragma unroll
           for (int m = 0; m < MT; ++m) {
-            mma16816_f16(acc[m][nb], lo[m].x, hi[m].x, lo[m].y, hi[m].y, xv.x, xv.y);
-            mma16816_f16(acc[m][nb], lo[m].z, hi[m].z, lo[m].w, hi[m].w, xv.z, xv.w);
+            const uint32_t a0[4] = {lo[m].x, hi[m].x, lo[m].y, hi[m].y}, a1[4] = {lo[m].z, hi[m].z, lo[m].w, hi[m].w};
+            mma_m16n8k16<__half>(acc[m][nb], a0, xv.x, xv.y);
+            mma_m16n8k16<__half>(acc[m][nb], a1, xv.z, xv.w);
           }
         }
         __syncwarp();
@@ -661,7 +641,7 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_stream_kernel(const __
       }
     }
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_wait<0>();
   __syncthreads();                                                          // every warp is done with its ring: the partial tiles alias it
   float (*red)[ROWS][STREAM_PITCH] = reinterpret_cast<float (*)[ROWS][STREAM_PITCH]>(stream_smem);
   // acc[m][nb][e]: row 16 m + g + 8 (e >> 1), image 8 nb + 2 q + (e & 1)
@@ -687,7 +667,7 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_stream_kernel(const __
         v += bv;
         if (RELU) v = fmaxf(v, 0.f);
         if (Y) Y[(int64_t)b * ldy + n] = v;
-        if (Yh) Yh[(int64_t)b * ldyh + n] = __float2half_rn(fminf(fmaxf(v, -65504.f), 65504.f));
+        if (Yh) Yh[(int64_t)b * ldyh + n] = f16_sat(v);
       }
     }
   }
@@ -764,7 +744,7 @@ __device__ __forceinline__ void attend_one(const float* q /*smem, HD, pre-scaled
     for (int j = 0; j < 8; ++j) out[sub * 8 + j] = acc[j] * inv;
     if (outh) {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) outh[sub * 8 + j] = __float2half_rn(fminf(fmaxf(acc[j] * inv, -65504.f), 65504.f));
+      for (int j = 0; j < 8; ++j) outh[sub * 8 + j] = f16_sat(acc[j] * inv);
     }
   }
   __syncwarp();
@@ -930,7 +910,7 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_cross_attn_split_kernel(const
     for (int w = 1; w < LIN_WARPS; ++w) v += part[w * HD + c];
     v *= inv;
     if (o) o[(int64_t)b * d + head * HD + c] = v;
-    if (oh) oh[(int64_t)b * d + head * HD + c] = __float2half_rn(fminf(fmaxf(v, -65504.f), 65504.f));
+    if (oh) oh[(int64_t)b * d + head * HD + c] = f16_sat(v);
   }
 }
 

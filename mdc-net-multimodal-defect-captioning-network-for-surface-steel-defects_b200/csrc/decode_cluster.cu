@@ -30,7 +30,7 @@
 #include <stdlib.h>
 #include <string.h>
 
-#define MDC_SEL_SYNC() asm volatile("bar.sync 1, 256;" ::: "memory")
+#define MDC_SEL_SYNC() bar_sync<1, 256>()
 #include "select.cuh"
 using namespace mdcsel;
 
@@ -117,83 +117,7 @@ struct __align__(64) FusedParams {
   float ref_margin;                        // developer build: softmax reference-maximum margin (MDC_DECODE_REF_MARGIN; the product build uses 64)
 };
 
-// ---- PTX helpers ------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_n(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-// bounded wait: a protocol bug traps (reported as a launch failure) instead of hanging the GPU box.  try_wait carries a suspend-time
-// hint: the waiting warp SLEEPS in hardware until the phase completes (or the hint expires) instead of spinning -- a spinning
-// waiter (without the hint try_wait returns after a few hundred cycles: 1.2 G of the 6.5 G instructions of a 256-image launch were
-// this loop, profiles/r2b) takes issue slots from the warps of the same SM sub-partition that have work, in particular from
-// the second CTA that shares the SM in the two-CTAs-per-SM variant.
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (true) {
-    asm volatile("{\n\t.reg .pred P1;\n\tmbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, P1;\n\t}\n"
-                 : "=r"(done) : "r"(bar), "r"(parity), "r"(1000000u) : "memory");      // hint: 1 ms
-    if (done) break;
-    if (++spins > 2000u) __trap();          // ~2 s
-  }
-}
-__device__ __forceinline__ uint32_t mapa(uint32_t addr, uint32_t rank) {
-  uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank)); return r;
-}
-__device__ __forceinline__ void st_async_b32(uint32_t raddr, uint32_t v, uint32_t rbar) {
-  asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(raddr), "r"(v), "r"(rbar) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void cbar() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 consumer warps
-// TMA bulk copy (non-tensor): `bytes` contiguous bytes global -> shared, completion counted on an mbarrier.  The kernel moves
-// EVERYTHING it streams this way (16-32 KB weight stages, 2 KB key/value chunks): tensor-map boxes cost the TMA unit ~4.5 cycles per
-// box ROW whatever its width (64-byte head slices: 14 B/clk/SM, 128-byte weight rows: 28 B/clk/SM -- profiles/r2d), which bounded the
-// previous version of this kernel; contiguous copies of pre-arranged shared-memory images do not pay per row.
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-// L2 prefetch of a contiguous block (no shared memory involved): the producer warp pulls the cross-K/V chunks it will copy a few
-// stages later from HBM into L2, so that the copies themselves meet L2 latency -- the ring holds at most three stages ahead, which
-// at HBM latency is the per-SM streaming rate the cross-attention phase ran at (~40 B/clk)
-__device__ __forceinline__ void bulk_prefetch_l2(const void* src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void ldsm_x4(uint32_t* r, uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void mma16816(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-// projections: fp16 weights (A) x fp16 hi/lo activations (B), fp32 accumulate
-__device__ __forceinline__ void mma16816_h(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint4 lds128(uint32_t addr) {
-  uint4 v; asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr)); return v;
-}
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b); return *reinterpret_cast<uint32_t*>(&h);
-}
-// projection operands are fp16 (11 significant bits, 8x finer than bf16: tools/error_budget_cpu.py "activations fp16" moves the
-// logit error by < 3e-4, where bf16 activations would cost 1.4e-2); |x| is clamped to the fp16 range first
-__device__ __forceinline__ float clamp_h(float x) { return fminf(fmaxf(x, -65504.f), 65504.f); }
-__device__ __forceinline__ void store_h(__half* dst, int idx, float x) { dst[idx] = __float2half_rn(clamp_h(x)); }
-__device__ __forceinline__ uint32_t pack_h2(float a, float b) {
-  __half2 h = __floats2half2_rn(a, b); return *reinterpret_cast<uint32_t*>(&h);
-}
+__device__ __forceinline__ void cbar() { bar_sync<1, NCT>(); }   // the 8 consumer warps
 
 // One 16-row tile of a projection with the weights as the M operand:
 //   acc[nb][0..3] = D[m0+g][img], D[m0+g][img+1], D[m0+g+8][img], D[m0+g+8][img+1], img = 8nb + 2q   (g = lane/4, q = lane%4)
@@ -224,8 +148,8 @@ __device__ __forceinline__ void mma_mtile(uint32_t wblk, int m0, uint32_t bh, fl
   {                                                                                                            \
     constexpr int i_ = (I), buf_ = i_ & 1, par_ = (i_ & 1) * 2;                                                \
     _Pragma("unroll") for (int nb_ = 0; nb_ < NB; ++nb_) {                                                     \
-      mma16816_h(c[nb_][par_], a0[buf_], xb[buf_][nb_][0], xb[buf_][nb_][1]);                                  \
-      mma16816_h(c[nb_][par_ + 1], a1[buf_], xb[buf_][nb_][2], xb[buf_][nb_][3]);                              \
+      mma_m16n8k16<__half>(c[nb_][par_], a0[buf_], xb[buf_][nb_][0], xb[buf_][nb_][1]);                        \
+      mma_m16n8k16<__half>(c[nb_][par_ + 1], a1[buf_], xb[buf_][nb_][2], xb[buf_][nb_][3]);                    \
     }                                                                                                          \
   }
   MDC_MTILE_LOAD(0) MDC_MTILE_LOAD(1)
@@ -251,11 +175,6 @@ __device__ __forceinline__ void mma_mtile(uint32_t wblk, int m0, uint32_t bh, fl
 // tile lands in lanes (g = 0, q) -- exactly where the B fragment of P.V wants column 0: the softmax runs in registers, nothing
 // goes through shared memory.  Lanes of the other row groups compute on zero rows; their values only reach output columns
 // that are never read.  Scores are in log2 units (q is pre-scaled by log2(e)/sqrt(hd)), so p = exp2(s - m).
-constexpr float LOG2E = 1.4426950408889634f;
-
-__device__ __forceinline__ void ldsm_x4_trans(uint32_t* r, uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
 
 // A fragments of q from its bf16 row (32 dims): aq[ks][h] covers dims 16*ks + 8*h + {2q, 2q+1}.  The query fills ALL eight row groups
 // of the M operand (rows 8-15 stay zero): every row group then computes the same scores, so the running maximum, the rescale factor
@@ -266,8 +185,6 @@ __device__ __forceinline__ void build_q_frag(const bf16* qh, uint32_t (&aq)[2][2
 #pragma unroll
   for (int i = 0; i < 4; ++i) aq[i >> 1][i & 1] = *reinterpret_cast<const uint32_t*>(src + (i >> 1) * 16 + (i & 1) * 8);
 }
-
-__device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 // running state of one (image, head) attention job, owned by ONE warp for the whole key range (flash-style online softmax):
 // m: running maximum (log2 units), ls: this lane's share of the softmax denominator (lanes of a quad hold different keys),
@@ -303,8 +220,8 @@ __device__ __forceinline__ void attn_tile(const uint32_t (&kp)[N], const uint32_
 #pragma unroll
     for (int j = 0; j < 2; ++j) {
       float c[4] = {0.f, 0.f, 0.f, 0.f}, d[4] = {0.f, 0.f, 0.f, 0.f};
-      mma16816(c, a_k0, kb[n][j][0], kb[n][j][1]);
-      mma16816(d, a_k1, kb[n][j][2], kb[n][j][3]);
+      mma_m16n8k16<bf16>(c, a_k0, kb[n][j][0], kb[n][j][1]);
+      mma_m16n8k16<bf16>(d, a_k1, kb[n][j][2], kb[n][j][3]);
       sc[n][2 * j] = c[0] + d[0];
       sc[n][2 * j + 1] = c[1] + d[1];
     }
@@ -348,9 +265,9 @@ __device__ __forceinline__ void attn_tile(const uint32_t (&kp)[N], const uint32_
 #pragma unroll
     for (int e = 0; e < 4; ++e) p[e] = ex2_approx(sc[n][e] - st[n].m);
     st[n].ls += (p[0] + p[1]) + (p[2] + p[3]);
-    const uint32_t b0 = pack_bf16(p[0], p[1]), b1 = pack_bf16(p[2], p[3]);
-    mma16816(st[n].o[0], va[n][0], b0, b1);
-    mma16816(st[n].o[1], va[n][1], b0, b1);
+    const uint32_t b0 = pack_bf16x2(p[0], p[1]), b1 = pack_bf16x2(p[2], p[3]);
+    mma_m16n8k16<bf16>(st[n].o[0], va[n][0], b0, b1);
+    mma_m16n8k16<bf16>(st[n].o[1], va[n][1], b0, b1);
   }
 }
 
@@ -386,7 +303,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
   uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);      // pointer arithmetic keeps the shared address space
   const uint32_t sbase = smem_u32(smem);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  uint32_t rank; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+  const uint32_t rank = cluster_rank();
   const int cid = blockIdx.x / CS, n_clusters = gridDim.x / CS;
 
   __half* xh = (__half*)(smem + Y::OFF_XH); __half* fh = (__half*)(smem + Y::OFF_FH);      // projection operands (fp16)
@@ -403,13 +320,13 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
   if (tid == 0) {
     for (int i = 0; i < NS; ++i) { mbar_init(bar(BAR_FULL + i), 1); mbar_init(bar(BAR_EMPTY + i), 8); }
     for (int i = BAR_O; i <= BAR_TOK; ++i) mbar_init(bar(i), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   // zero the ring and the activation operands once: rows >= G of the operands are multiplied by weights and must be finite
   // (ring bytes that a stage does not fill are only ever stale finite fp16 / bf16 data of earlier stages)
   for (int i = tid; i < (NS * STAGE + 3 * Y::ACT_BYTES) / 16; i += NT) reinterpret_cast<uint4*>(smem + Y::OFF_RING)[i] = make_uint4(0u, 0u, 0u, 0u);
   __syncthreads();
-  cluster_sync_all();
+  cluster_sync();
 
   const float scale = rsqrtf((float)HD) * LOG2E;      // scores in log2 units: p = exp2(s - m)
 #ifdef MDC_DEVTOOLS
@@ -447,7 +364,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
       haspad[tid] = any != 0u;
     }
     __syncthreads();
-    cluster_sync_all();          // no peer may push into this CTA before its buffers are set up for the group
+    cluster_sync();          // no peer may push into this CTA before its buffers are set up for the group
 
     if (warp == 8) {
       // =================================== PRODUCER WARP ===================================================
@@ -620,7 +537,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
       auto layer_norm = [&](const float* lnw, const float* lnb, bool fence_appends = false, int l_now = -1, int t_now = -1, int fi = 0) {
         if (warp == 0) FINE(l_now, t_now, fi);
         // this layer's KV append: the generic->async proxy fence (~1200 cycles) of the appending threads overlaps the exchange latency
-        if (fence_appends && tid >= APP0 && tid - APP0 < G * 8) asm volatile("fence.proxy.async;" ::: "memory");
+        if (fence_appends && tid >= APP0 && tid - APP0 < G * 8) fence_proxy_async();
         float gw[8], gb[8];
         if (warp < G) {
 #pragma unroll
@@ -665,7 +582,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
               const int c = lane + 32 * j;
               const float xn = (v[nb][j] - mean[nb]) * rstd[nb] * gw[j] + gb[j];
               xres[img * DM + c] = xn;
-              store_h(xh, img * XP + c, xn);
+              xh[img * XP + c] = f16_sat(xn);
             }
           }
         }
@@ -679,7 +596,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
         const int j = lane & 15;
         const float v0 = __shfl_sync(0xffffffffu, o, 2 * j), v1 = __shfl_sync(0xffffffffu, o, 2 * j + 1);
         if (img < G) {
-          const uint32_t val = pack_h2(clamp_h(v0), clamp_h(v1));
+          const uint32_t val = pack_f16x2_sat(v0, v1);
           const uint32_t off = sbase + Y::OFF_OH + (img * XP + 32 * rank + 2 * j) * 2;
           const int p0 = (lane >> 4) * 4;
 #pragma unroll
@@ -803,7 +720,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
                 const int c = lane + 32 * j;
                 const float x = __ldg(P.emb + (int64_t)tok * DM + c) + pz[j];
                 xres[img * DM + c] = x;
-                store_h(xh, img * XP + c, x);
+                xh[img * XP + c] = f16_sat(x);
               }
             }
           }
@@ -851,7 +768,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
             const int g = at >> 3, which = (at >> 2) & 1, ch = at & 3;
             const float* src = (which ? vnew : knew) + g * 32 + ch * 8;
             const float4 a = *reinterpret_cast<const float4*>(src), b = *reinterpret_cast<const float4*>(src + 4);
-            uint4 o; o.x = pack_bf16(a.x, a.y); o.y = pack_bf16(a.z, a.w); o.z = pack_bf16(b.x, b.y); o.w = pack_bf16(b.z, b.w);
+            uint4 o; o.x = pack_bf16x2(a.x, a.y); o.y = pack_bf16x2(a.z, a.w); o.z = pack_bf16x2(b.x, b.y); o.w = pack_bf16x2(b.z, b.w);
             const int page = pages[g * 32 + t / P.PT];
             const int r = t % P.PT;      // pool: [page][layer][head][k|v][16 tokens][32]; chunk ch of token r at ch ^ ((r >> 1) & 3) (decode.cu kv_chunk)
             bf16* dst = P.kv_pool + ((((int64_t)page * L + l) * CS + rank) * 2 + which) * (int64_t)(P.PT * HD) + r * HD + ((ch ^ ((r >> 1) & 3)) << 3);
@@ -884,7 +801,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
           }
           // this layer's KV append: the generic->async proxy fence (~1200 cycles) of the appending threads runs while they wait for the
           // attention-output gather (it used to sit at the head of LayerNorm 1, which was ~1000 cycles longer than LayerNorm 2)
-          if (tid >= APP0 && tid - APP0 < G * 8) asm volatile("fence.proxy.async;" ::: "memory");
+          if (tid >= APP0 && tid - APP0 < G * 8) fence_proxy_async();
           wait_o();
           TRACE(t);   // 4: o gathered
           // ---- self out-proj slice -> all-gather -> LN1 ------------------------------------------------------------
@@ -947,8 +864,8 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
 #pragma unroll
               for (int nb = 0; nb < NB; ++nb) {
                 const int r = 8 * nb + 2 * fq;
-                store_h(fh, r * XP + h, fmaxf(acc[nb][0] + b0, 0.f)); store_h(fh, (r + 1) * XP + h, fmaxf(acc[nb][1] + b0, 0.f));
-                store_h(fh, r * XP + h + 8, fmaxf(acc[nb][2] + b1, 0.f)); store_h(fh, (r + 1) * XP + h + 8, fmaxf(acc[nb][3] + b1, 0.f));
+                fh[r * XP + h] = f16_sat(fmaxf(acc[nb][0] + b0, 0.f)); fh[(r + 1) * XP + h] = f16_sat(fmaxf(acc[nb][1] + b0, 0.f));
+                fh[r * XP + h + 8] = f16_sat(fmaxf(acc[nb][2] + b1, 0.f)); fh[(r + 1) * XP + h + 8] = f16_sat(fmaxf(acc[nb][3] + b1, 0.f));
               }
             });
           }
@@ -1099,7 +1016,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
   }
   // no CTA may exit while a peer can still push into its shared memory
   __syncthreads();
-  cluster_sync_all();
+  cluster_sync();
 }
 
 // ---- pack kernels: global-memory images of what the kernel wants in shared memory -----------------------------------

@@ -48,117 +48,8 @@ template <int BN, int EW, int CTAS = 1> struct Cfg {
   static constexpr int kSmemBytes = kStages * kStageBytes + kStageOutBytes + 1024 /*align slack*/ + 256 /*barriers*/ + 4 * BN * 4 /*bias+gamma x2 stages*/;
 };
 
-// ---- PTX wrappers --------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}\n" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// bounded wait: a protocol bug traps (reported as a launch failure) instead of hanging the GPU box
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  long long t0 = 0;
-  while (true) {
-    asm volatile("{\n\t.reg .pred P1;\n\tmbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\tselp.u32 %0, 1, 0, P1;\n\t}\n"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (done) break;
-    if ((++spins & 1023u) == 0) {
-      long long now = clock64();
-      if (t0 == 0) t0 = now;
-      else if (now - t0 > 4000000000LL) __trap();   // ~2 s
-    }
-  }
-}
-__device__ __forceinline__ void tma_load_2d(const CUtensorMap* map, uint32_t bar, uint32_t dst, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-               ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1) : "memory");
-}
-// epilogue: shared -> global tile store / reduce-add through the TMA unit (coalesced, OOB rows and columns clipped)
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(map), "r"(src), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* map, uint32_t src, int c0, int c1) {
-  asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];" ::"l"(map), "r"(src), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ uint32_t pack2_bf16(float a, float b) { __nv_bfloat162 h = __floats2bfloat162_rn(a, b); return *reinterpret_cast<uint32_t*>(&h); }
-// IEEE half outputs (the decoder prefill path): clamped to the finite range first
-__device__ __forceinline__ uint32_t pack2_f16(float a, float b) {
-  __half2 h = __floats2half2_rn(fminf(fmaxf(a, -65504.f), 65504.f), fminf(fmaxf(b, -65504.f), 65504.f)); return *reinterpret_cast<uint32_t*>(&h);
-}
-template <bool F16> __device__ __forceinline__ uint32_t pack2_16(float a, float b) { return F16 ? pack2_f16(a, b) : pack2_bf16(a, b); }
-__device__ __forceinline__ void tcgen05_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tcgen05_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-               ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-// ---- cta_group::2 forms (pair of CTAs; CTA rank 0 of the cluster is the leader that issues the MMAs) ----
-__device__ __forceinline__ void tma_load_2d_2sm(const CUtensorMap* map, uint32_t leader_bar, uint32_t dst, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-               ::"r"(dst), "l"(map), "r"(leader_bar), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void umma_f16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-               ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {     // arrives on the barrier at this offset in BOTH CTAs of the pair
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_rank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t local_bar, uint32_t cta) {   // arrive on the same barrier in CTA `cta` of the cluster
-  uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_bar), "r"(cta));
-  // default semantics (release at CTA scope): the arrival orders this warp's TMEM reads (tcgen05.fence::before_thread_sync) before the
-  // leader's next MMAs; .release.cluster would add a cluster-scope memory fence per warp and tile (~1 us per tile measured)
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(r) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t addr, uint32_t* v) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-               "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-               "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                 "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-                 "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-                 "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-               : "r"(addr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// K-major SWIZZLE_128B operand tile: rows of 128 B, 8-row groups 1024 B apart (SBO); LBO unused.
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);          // start address        bits [0,14)
-  d |= (uint64_t)(1024 >> 4) << 32;                // stride byte offset   bits [32,46)
-  d |= (uint64_t)1 << 46;                          // descriptor version 1 (sm_100)
-  d |= (uint64_t)2 << 61;                          // layout type SWIZZLE_128B
-  return d;
-}
-// kind::f16: D=f32 (bits 4-5 =1), A and B formats at bits 7-9 / 10-12 (0 = fp16, 1 = bf16), both K-major, N>>3 at 17, M>>4 at 24
-__host__ __device__ constexpr uint32_t make_idesc(int M, int N, bool f16 = false) {
-  return (1u << 4) | ((f16 ? 0u : 1u) << 7) | ((f16 ? 0u : 1u) << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
+// 16-bit outputs: bf16, or IEEE half (the decoder prefill path) clamped to the finite range first
+template <bool F16> __device__ __forceinline__ uint32_t pack2_16(float a, float b) { return F16 ? pack_f16x2_sat(a, b) : pack_bf16x2(a, b); }
 
 struct EpiArgs {
   void* D; int64_t ldd; const float* bias; const float* aux0; int period; int epilogue;
@@ -169,15 +60,6 @@ struct EpiArgs {
 #else
 #define GEMM_DBG(ep, bit) 0
 #endif
-
-// packed fp32 pairs (sm_100 FFMA2 / FMUL2 / FADD2): the epilogue polynomial runs on two columns per instruction
-__device__ __forceinline__ uint64_t pk2(float a, float b) { uint64_t r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b)); return r; }
-__device__ __forceinline__ void upk2(uint64_t v, float& a, float& b) { asm("mov.b64 {%0, %1}, %2;" : "=f"(a), "=f"(b) : "l"(v)); }
-__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) { uint64_t d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
-__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) { uint64_t d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-
-__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) { uint64_t d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-__device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 // exact-erf GELU of two values, branch-free:  GELU(x) = x Phi(x) = max(x, 0) - a Phi(-a),  a = |x|,  and  Phi(-a) = 2^q(a)  with q a
 // degree-6 polynomial fitted to log2 Phi(-a) on [0, 6] (weighted minimax on the error of a 2^q(a); tools/gelu_fit.py).  |error| of
@@ -231,26 +113,21 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   const int num_kb = (K + BLOCK_K - 1) / BLOCK_K;
 
   if (warp == 0 && elect_one()) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w) : "memory");
-    if (EPI != MDC_EPI_PATCH) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_d) : "memory");
+    prefetch_tmap(&map_a);
+    prefetch_tmap(&map_w);
+    if (EPI != MDC_EPI_PATCH) prefetch_tmap(&map_d);
     for (int i = 0; i < C::kStages; ++i) { mbar_init(smem_u32(&full[i]), 1); mbar_init(smem_u32(&empty[i]), 1); }
     // the accumulator is released by one arrival per epilogue warp of every CTA of the cluster (the leader's barrier is the one waited on)
     for (int i = 0; i < 2; ++i) { mbar_init(smem_u32(&tmem_full[i]), 1); mbar_init(smem_u32(&tmem_empty[i]), EW * CTAS); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   } else if (warp == 1) {
-    if constexpr (CTAS == 2) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr_smem)), "r"(C::kTmemCols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr_smem)), "r"(C::kTmemCols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    tmem_alloc<CTAS>(smem_u32(tmem_ptr_smem), C::kTmemCols);
+    tmem_relinquish<CTAS>();
   }
-  tcgen05_fence_before();
+  tc_fence_before();
   __syncthreads();
   if constexpr (CTAS == 2) cluster_sync();      // the peer's barriers are initialised before anything can signal them
-  tcgen05_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
   if (warp == 0) {
@@ -260,13 +137,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       for (int tile = first_tile; tile < num_tiles; tile += tile_step) {
         const int m0 = (tile / tiles_n) * (BLOCK_M * CTAS) + rank * BLOCK_M, n0 = (tile % tiles_n) * BN + rank * (BN / CTAS);
         for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(smem_u32(&empty[stage]), phase ^ 1);
+          mbar_wait_spin(smem_u32(&empty[stage]), phase ^ 1);
           const uint32_t fb = smem_u32(&full[stage]);
           if (GEMM_DBG(ep, 4)) { if (rank == 0) mbar_arrive(fb); }
           else if constexpr (CTAS == 2) {
             // both CTAs' loads complete on the LEADER's barrier, which expects the bytes of both
             if (rank == 0) mbar_expect_tx(fb, 2 * C::kStageBytes);
-            uint32_t lb; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(lb) : "r"(fb), "r"(0));
+            const uint32_t lb = mapa(fb, 0);
             tma_load_2d_2sm(&map_a, lb, smem_u32(smem_a + stage * C::kABytes), GEMM_DBG(ep, 2) ? 0 : kb * BLOCK_K, GEMM_DBG(ep, 2) ? 0 : m0);
             tma_load_2d_2sm(&map_w, lb, smem_u32(smem_b + stage * C::kBBytes), GEMM_DBG(ep, 2) ? 0 : kb * BLOCK_K, GEMM_DBG(ep, 2) ? 0 : n0);
           } else {
@@ -285,20 +162,20 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     if (rank == 0)                                   // the leader CTA of a pair issues for both
     for (int tile = first_tile; tile < num_tiles; tile += tile_step, ++iter) {
       const int as = iter & 1; const uint32_t aphase = (iter >> 1) & 1;
-      mbar_wait(smem_u32(&tmem_empty[as]), aphase ^ 1);
-      tcgen05_fence_after();
+      mbar_wait_spin(smem_u32(&tmem_empty[as]), aphase ^ 1);
+      tc_fence_after();
       const uint32_t tmem_d = tmem_base + as * BN;
       for (int kb = 0; kb < num_kb; ++kb) {
-        mbar_wait(smem_u32(&full[stage]), phase);
-        tcgen05_fence_after();
+        mbar_wait_spin(smem_u32(&full[stage]), phase);
+        tc_fence_after();
         if (elect_one()) {
-          const uint64_t adesc = make_smem_desc(smem_u32(smem_a + stage * C::kABytes));
-          const uint64_t bdesc = make_smem_desc(smem_u32(smem_b + stage * C::kBBytes));
+          const uint64_t adesc = make_sw128_desc(smem_u32(smem_a + stage * C::kABytes));
+          const uint64_t bdesc = make_sw128_desc(smem_u32(smem_b + stage * C::kBBytes));
           if (!GEMM_DBG(ep, 8))
 #pragma unroll
           for (int k = 0; k < BLOCK_K / UMMA_K; ++k) { // +32 B per UMMA_K inside the swizzle atom -> +2 in the >>4 address field
-            if constexpr (CTAS == 2) umma_f16_2sm(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0);
-            else umma_f16(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0);
+            if constexpr (CTAS == 2) umma_ss_2sm(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0);
+            else umma_ss(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0);
           }
           if constexpr (CTAS == 2) {
             umma_commit_2sm(smem_u32(&empty[stage]));                       // frees the smem slot in both CTAs when these MMAs retire
@@ -334,9 +211,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         s_bias[as * BN + i] = (ok && ep.bias) ? __ldg(ep.bias + n0 + i) : 0.f;
         if (EPI == MDC_EPI_LS_RESIDUAL) s_gamma[as * BN + i] = ok ? __ldg(ep.aux0 + n0 + i) : 0.f;
       }
-      asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
-      mbar_wait(smem_u32(&tmem_full[as]), aphase);
-      tcgen05_fence_after();
+      bar_sync<1, EPI_THREADS>();
+      mbar_wait_spin(smem_u32(&tmem_full[as]), aphase);
+      tc_fence_after();
       const int row0 = m0 + quad * 32, row = row0 + lane;
       const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + as * BN + half * HALF_COLS;
       const float* sb = s_bias + as * BN + half * HALF_COLS;
@@ -368,8 +245,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
           for (int i = 0; i < 8; ++i) {
             const int rl = i * 4 + (lane >> 3), r = row0 + rl;
-            float4 x;
-            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(x.x), "=f"(x.y), "=f"(x.z), "=f"(x.w) : "r"(stage_out + rl * 128 + ((ch ^ (rl & 7)) << 4)));
+            const uint4 xu = lds128(stage_out + rl * 128 + ((ch ^ (rl & 7)) << 4));
+            const float4 x = make_float4(__uint_as_float(xu.x), __uint_as_float(xu.y), __uint_as_float(xu.z), __uint_as_float(xu.w));
             if (r < M && col < N) {
               int img = img0, pr = r - img0 * ep.period;
               if (pr >= ep.period) { pr -= ep.period; ++img; }                     // a 32-row chunk crosses at most one image boundary
@@ -426,7 +303,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
               sts128(row_s + ((c ^ sw) << 4), pack2_16<F16>(o[0], o[1]), pack2_16<F16>(o[2], o[3]), pack2_16<F16>(o[4], o[5]), pack2_16<F16>(o[6], o[7]));
             }
           }
-          fence_async_smem();
+          fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0 && row0 < M && col0 < N && !GEMM_DBG(ep, 16)) {
             const int sc = GEMM_DBG(ep, 64) ? 0 : col0, sr = GEMM_DBG(ep, 64) ? 0 : row0;      // 64: every store to tile (0,0)
@@ -437,7 +314,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           if (C::kOutBufs == 2) obuf ^= 1;
         }
       }
-      tcgen05_fence_before();
+      tc_fence_before();
       __syncwarp();
       if (lane == 0) {                                            // this warp's TMEM reads of the accumulator stage are done
         if constexpr (CTAS == 2) mbar_arrive_cluster(smem_u32(&tmem_empty[as]), 0);
@@ -446,13 +323,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     }
     if (EPI != MDC_EPI_PATCH && lane == 0) bulk_wait_read<0>();   // staging tiles must outlive the last stores' reads
   }
-  tcgen05_fence_before();
+  tc_fence_before();
   __syncthreads();
   if constexpr (CTAS == 2) cluster_sync();      // no CTA leaves while its peer can still signal its barriers or read its operands
   if (warp == 1) {
-    tcgen05_fence_after();
-    if constexpr (CTAS == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::kTmemCols) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::kTmemCols) : "memory");
+    tc_fence_after();
+    tmem_dealloc<CTAS>(tmem_base, C::kTmemCols);
   }
 }
 

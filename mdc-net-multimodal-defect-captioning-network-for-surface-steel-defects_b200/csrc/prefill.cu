@@ -13,8 +13,6 @@
 
 namespace {
 
-constexpr float LOG2E = 1.4426950408889634f;
-
 // ---- embedding + positional table; PAD-key bias -------------------------------------------------------------------------
 __global__ void prefill_embed_kernel(const int32_t* __restrict__ tokens, int tokens_ld, int n, int dim, const float* __restrict__ emb,
                                      const float* __restrict__ pos, int pad_idx, float* __restrict__ x32, __half* __restrict__ x16,
@@ -27,7 +25,7 @@ __global__ void prefill_embed_kernel(const int32_t* __restrict__ tokens, int tok
   for (int c = lane; c < dim; c += 32) {
     const float v = emb[(int64_t)tok * dim + c] + pos[(int64_t)i * dim + c];
     x32[row * dim + c] = v;
-    x16[row * dim + c] = __float2half_rn(fminf(fmaxf(v, -65504.f), 65504.f));
+    x16[row * dim + c] = f16_sat(v);
   }
 }
 
@@ -64,9 +62,9 @@ __global__ void add_layernorm_kernel(float* __restrict__ x32, const __half* __re
 #pragma unroll
     for (int j = 0; j < 8; ++j) o[j] = (v[i][j] - mean) * rstd * __ldg(w + c0 + j) + __ldg(bia + c0 + j);
     store8(x32 + row * DIM + c0, o);
-    uint4 h; __half2* hp = reinterpret_cast<__half2*>(&h);
+    uint4 h; uint32_t* hp = reinterpret_cast<uint32_t*>(&h);
 #pragma unroll
-    for (int j = 0; j < 4; ++j) hp[j] = __floats2half2_rn(fminf(fmaxf(o[2 * j], -65504.f), 65504.f), fminf(fmaxf(o[2 * j + 1], -65504.f), 65504.f));
+    for (int j = 0; j < 4; ++j) hp[j] = pack_f16x2_sat(o[2 * j], o[2 * j + 1]);
     *reinterpret_cast<uint4*>(x16 + row * DIM + c0) = h;
   }
 }
@@ -74,40 +72,18 @@ __global__ void add_layernorm_kernel(float* __restrict__ x32, const __half* __re
 // ---- attention, head width 32 / 64 / 128, on the tensor cores ----------------------------------------------------------------------------
 template <typename T> struct Mma;
 template <> struct Mma<__half> {
-  static __device__ __forceinline__ void mma(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-  }
-  static __device__ __forceinline__ uint32_t pack(float a, float b) { __half2 h = __floats2half2_rn(a, b); return *reinterpret_cast<uint32_t*>(&h); }
+  static __device__ __forceinline__ void mma(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) { mma_m16n8k16<__half>(c, a, b0, b1); }
+  static __device__ __forceinline__ uint32_t pack(float a, float b) { return pack_f16x2(a, b); }
   static __device__ __forceinline__ uint32_t from_half2(uint32_t v) { return v; }
 };
 template <> struct Mma<bf16> {
-  static __device__ __forceinline__ void mma(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-  }
-  static __device__ __forceinline__ uint32_t pack(float a, float b) { __nv_bfloat162 h = __floats2bfloat162_rn(a, b); return *reinterpret_cast<uint32_t*>(&h); }
+  static __device__ __forceinline__ void mma(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) { mma_m16n8k16<bf16>(c, a, b0, b1); }
+  static __device__ __forceinline__ uint32_t pack(float a, float b) { return pack_bf16x2(a, b); }
   static __device__ __forceinline__ uint32_t from_half2(uint32_t v) {      // the fp16 query meets bf16 keys: rounded to the cache precision
     const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&v));
     return pack(f.x, f.y);
   }
 };
-
-__device__ __forceinline__ void ldsm_x4(uint32_t* r, uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_trans(uint32_t* r, uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ float ex2a(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) { asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory"); }
-// [rows][HD * 2 B] panel; 16-byte chunk c of row r is stored at a swizzled chunk so that ldmatrix (eight consecutive rows, one chunk) is
-// conflict-free: 64-byte rows: c ^ ((r >> 1) & 3); 128- and 256-byte rows: c ^ (r & 7)
-template <int HD>
-__device__ __forceinline__ uint32_t swz(int r, int c) {
-  if constexpr (HD == 32) return (uint32_t)(r * 64 + ((c ^ ((r >> 1) & 3)) << 4));
-  else return (uint32_t)(r * (HD * 2) + ((c ^ (r & 7)) << 4));
-}
 
 constexpr int QCH = 128;                 // queries per CTA (8 warps x 16)
 template <int HD> struct AttnCfg { static constexpr int KCH = HD == 128 ? 64 : 128; };    // keys staged per chunk: K and V panels of 8-16 KB each
@@ -122,7 +98,7 @@ __global__ void __launch_bounds__(256) prefill_attn_kernel(const __half* __restr
   __shared__ __align__(128) uint8_t Ks[KCH * HD * 2];
   __shared__ __align__(128) uint8_t Vs[KCH * HD * 2];
   const int head = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, q4 = lane & 3;
-  const uint32_t ks = (uint32_t)__cvta_generic_to_shared(Ks), vs = (uint32_t)__cvta_generic_to_shared(Vs);
+  const uint32_t ks = smem_u32(Ks), vs = smem_u32(Vs);
   const int q0 = blockIdx.z * QCH + warp * 16, r0 = q0 + g, r1 = r0 + 8;
   const bool active = q0 < Lq;
   uint32_t qa[NKS][4];
@@ -152,7 +128,7 @@ __global__ void __launch_bounds__(256) prefill_attn_kernel(const __half* __restr
         *reinterpret_cast<uint4*>(Vs + swz<HD>(r, c)) = make_uint4(0, 0, 0, 0);
       }
     }
-    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
+    cp_async_wait_all();
     __syncthreads();
     int nblk = active ? (min(KCH, Lk - kc0) + 15) / 16 : 0;
     if (CAUSAL && active) nblk = max(0, min(nblk, (q0 + 15 - kc0) / 16 + 1));     // key blocks that hold a key <= the warp's last query
@@ -186,14 +162,14 @@ __global__ void __launch_bounds__(256) prefill_attn_kernel(const __half* __restr
       mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1)); mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
       // a row can be fully masked in a block (causal, row < key0; padded query rows): keep the state untouched then
       const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);
-      const float c0 = mn0 == -INFINITY ? 1.f : ex2a(m0 - mn0), c1 = mn1 == -INFINITY ? 1.f : ex2a(m1 - mn1);
+      const float c0 = mn0 == -INFINITY ? 1.f : ex2_approx(m0 - mn0), c1 = mn1 == -INFINITY ? 1.f : ex2_approx(m1 - mn1);
       const float ms0 = mn0 == -INFINITY ? 0.f : mn0, ms1 = mn1 == -INFINITY ? 0.f : mn1;
       m0 = mn0; m1 = mn1;
       float p[2][4];
 #pragma unroll
       for (int nt = 0; nt < 2; ++nt) {
-        p[nt][0] = ex2a(s[nt][0] - ms0); p[nt][1] = ex2a(s[nt][1] - ms0);
-        p[nt][2] = ex2a(s[nt][2] - ms1); p[nt][3] = ex2a(s[nt][3] - ms1);
+        p[nt][0] = ex2_approx(s[nt][0] - ms0); p[nt][1] = ex2_approx(s[nt][1] - ms0);
+        p[nt][2] = ex2_approx(s[nt][2] - ms1); p[nt][3] = ex2_approx(s[nt][3] - ms1);
       }
       l0 = l0 * c0 + (p[0][0] + p[0][1]) + (p[1][0] + p[1][1]);
       l1 = l1 * c1 + (p[0][2] + p[0][3]) + (p[1][2] + p[1][3]);
