@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MDC_ABI_VERSION 5
+#define MDC_ABI_VERSION 6
 
 /* element types of activations / weights.  MDC_F16 (IEEE half) is only ever the type of the decode-loop weights, see
  * mdc_dims.dec_loop_dtype. */
@@ -222,6 +222,16 @@ typedef struct mdc_decode_state {
   int32_t per_op_kernels;           /* 1 = run every step as per-operation kernels (decode.cu: the path of the fp32 token-exact
                                        mode and of geometries the fused cluster kernel does not cover) even where the fused kernel
                                        applies -- the parity tests compare the two implementations on the same inputs. */
+  int32_t stop_at_eos;              /* 1 = stop at EOS (0, the zero-initialised value, = run every step for every image).  Let e_b be the
+                                       first step at which image b emits `eos_token` (an EOS among the known columns 1..t_begin counts as
+                                       finished from the start).  Token columns 0..e_b+1 and the conf columns of steps <= e_b are bitwise
+                                       what the same call without stopping writes; token columns e_b+2..t_end are pad_idx and the conf
+                                       columns of steps > e_b are 0.0, written by the library whatever the buffers held.  An image that
+                                       never emits EOS gets the no-stop result.  Decoding of a group of images ends once all of them have
+                                       finished (the fused kernel: per cluster group; the per-operation kernels: once the whole batch has
+                                       finished, the remaining launches return at entry).  Results stay batch-invariant.  Requires
+                                       forced == 0 and logits == NULL (steps that do not run have no logits). */
+  int32_t eos_token;                /* the stop token, in [0, vocab) (read only with stop_at_eos) */
 } mdc_decode_state;
 
 size_t mdc_decode_workspace_bytes(const mdc_model* m, int B);

@@ -60,6 +60,7 @@ class DecodeState(C.Structure):
         ("images_per_cluster", C.c_int32),
         ("ctas_per_sm", C.c_int32),
         ("per_op_kernels", C.c_int32),
+        ("stop_at_eos", C.c_int32), ("eos_token", C.c_int32),
     ]
 
 

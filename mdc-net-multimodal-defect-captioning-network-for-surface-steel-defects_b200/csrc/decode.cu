@@ -49,7 +49,11 @@ struct XSrc {
   const __half* xh;                             // HALF: operand rows already built as IEEE half [B][K] (prep_x_half_kernel);
                                                 // PLAIN: optional IEEE-half twin of the f32 rows, written by the producer (row pitch ldxh)
   int64_t ldxh;
+  const int* done;                              // stop at EOS: the batch's all-finished flag (NULL without stopping); set = return at entry
 };
+
+// stop at EOS (per-operation path): every kernel of a step returns at entry once the whole batch has finished
+__device__ __forceinline__ bool batch_done(const int* done) { return done != nullptr && *done != 0; }
 
 // Fill Xs[BT][K] (f32) for batch rows b0..b0+BT-1.
 __device__ __forceinline__ void load_x_tile(const XSrc& xs, float* Xs, int b0, int B, int K, bool publish) {
@@ -214,6 +218,7 @@ template <> struct Raw8<float> {
 template <typename TW, int RW, int KCH, bool RELU>
 __global__ void __launch_bounds__(LIN_THREADS) dec_linear_kernel(XSrc xs, const TW* __restrict__ W, const float* __restrict__ bias,
                                                                   float* __restrict__ Y, int64_t ldy, int B, int N) {
+  if (batch_done(xs.done)) return;
   constexpr int K = KCH * 256;
   extern __shared__ __align__(16) float Xs[];
   const int b0 = blockIdx.y * BT;
@@ -273,6 +278,7 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_kernel(XSrc xs, const 
 template <typename TW, bool RELU>
 __global__ void __launch_bounds__(LIN_THREADS) dec_linear_generic_kernel(XSrc xs, const TW* __restrict__ W, const float* __restrict__ bias,
                                                                           float* __restrict__ Y, int64_t ldy, int B, int N, int K) {
+  if (batch_done(xs.done)) return;
   extern __shared__ __align__(16) float Xs[];
   const int b0 = blockIdx.y * BT;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -330,6 +336,7 @@ constexpr int MMA_PAD = 4;         // halves of row padding: row pitch = 2 words
 // dim-1024 token-step)
 template <int NV>
 __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_vec_kernel(XSrc xs, __half* __restrict__ xh, int B) {
+  if (batch_done(xs.done)) return;
   constexpr int K = NV * 128;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * LIN_WARPS + warp;
@@ -386,6 +393,7 @@ __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_vec_kernel(XSrc xs, _
 }
 
 __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_kernel(XSrc xs, __half* __restrict__ xh, int B, int K) {
+  if (batch_done(xs.done)) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * LIN_WARPS + warp;
   if (b >= B) return;
@@ -463,6 +471,7 @@ __device__ __forceinline__ void build_x_half(const XSrc& xs, __half* Xh, int b0,
 template <bool RELU>
 __global__ void __launch_bounds__(LIN_THREADS) dec_linear_mma_kernel(XSrc xs, const __half* __restrict__ W, const float* __restrict__ bias,
                                                                       float* __restrict__ Y, int64_t ldy, int B, int N, int K) {
+  if (batch_done(xs.done)) return;
   extern __shared__ __align__(16) uint8_t mma_smem[];
   __half* Xh = reinterpret_cast<__half*>(mma_smem);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, q = lane & 3;
@@ -553,7 +562,8 @@ template <bool RELU, int MT>
 __global__ void __launch_bounds__(LIN_THREADS) dec_linear_stream_kernel(const __half* __restrict__ X, int64_t ldx, const __half* __restrict__ W,
                                                                          const float* __restrict__ bias, float* __restrict__ Y, int64_t ldy,
                                                                          __half* __restrict__ Yh, int64_t ldyh, int B, int N, int K,
-                                                                         const uint8_t* __restrict__ pf, int pf_lines) {
+                                                                         const uint8_t* __restrict__ pf, int pf_lines, const int* done) {
+  if (batch_done(done)) return;
   constexpr int ROWS = STREAM_ROWS * MT;
   static_assert(LIN_WARPS * ROWS * STREAM_PITCH * 4 <= STREAM_SMEM, "partial tiles must fit into the operand ring");
   extern __shared__ __align__(128) uint8_t stream_smem[];
@@ -762,7 +772,8 @@ template <typename TKV, int HD>
 __global__ void dec_self_attn_kernel(const float* __restrict__ qkv /*[B,3d]*/, TKV* __restrict__ pool,
                                      const int32_t* __restrict__ page_table, int pages_per_seq, int PT, int n_layers, int layer,
                                      const int32_t* __restrict__ tokens, int tokens_ld, int pad_idx, int t, int d,
-                                     float scale, float* __restrict__ o /*[B,d]*/, __half* __restrict__ oh /*[B,d] or NULL*/) {
+                                     float scale, float* __restrict__ o /*[B,d]*/, __half* __restrict__ oh /*[B,d] or NULL*/, const int* done) {
+  if (batch_done(done)) return;
   constexpr int hd = HD;
   extern __shared__ float sm[];
   const int b = blockIdx.x, head = threadIdx.x >> 5, lane = threadIdx.x & 31, heads = blockDim.x >> 5;
@@ -795,7 +806,8 @@ __global__ void dec_self_attn_kernel(const float* __restrict__ qkv /*[B,3d]*/, T
 // cross-attention over the S memory keys of image b; cross_kv layer plane: [B*S][2d] (K | V)
 template <typename TKV, int HD>
 __global__ void dec_cross_attn_kernel(const float* __restrict__ qc /*[B,d]*/, const TKV* __restrict__ ckv_layer, int S, int d,
-                                      float scale, float* __restrict__ o) {
+                                      float scale, float* __restrict__ o, const int* done) {
+  if (batch_done(done)) return;
   constexpr int hd = HD;
   extern __shared__ float sm[];
   const int b = blockIdx.x, head = threadIdx.x >> 5, lane = threadIdx.x & 31, heads = blockDim.x >> 5;
@@ -817,7 +829,9 @@ __global__ void dec_cross_attn_kernel(const float* __restrict__ qc /*[B,d]*/, co
 // the out-projection (and optionally f32).
 template <typename TKV, int HD>
 __global__ void __launch_bounds__(LIN_THREADS) dec_cross_attn_split_kernel(const float* __restrict__ qc /*[B,d]*/, const TKV* __restrict__ ckv_layer,
-                                                                            int S, int d, float scale, float* __restrict__ o, __half* __restrict__ oh) {
+                                                                            int S, int d, float scale, float* __restrict__ o, __half* __restrict__ oh,
+                                                                            const int* done) {
+  if (batch_done(done)) return;
   constexpr int LPK = HD / 8, KPI = 32 / LPK, UN = 4;
   extern __shared__ float sm[];
   float* qs = sm;                       // HD
@@ -917,17 +931,50 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_cross_attn_split_kernel(const
 using namespace mdcsel;
 
 
+// Stop at EOS on the per-operation path (mdc_decode_state.stop_at_eos), in the decode workspace: fin [B] = image b has finished,
+// state[0] = number of finished images, state[1] = all finished (the `done` flag every kernel of a step tests at entry).  NULL = off.
+struct StopArgs { int* fin; int* state; int eos; };
+
+// Once per mdc_decode_steps call, before the first step (inside a captured graph: at the start of every replay): the token columns
+// t_begin+1..t_end become PAD and the conf columns of steps t_begin..t_end-1 zero -- the values of every position after an image's
+// EOS, which the select of a step that runs overwrites with the selected token -- and the finished flags and count come from the
+// known prefix (an EOS among columns 1..t_begin).  One CTA.
+__global__ void __launch_bounds__(SEL_THREADS) dec_stop_init_kernel(int32_t* __restrict__ tokens, int tokens_ld, float* __restrict__ confs,
+                                                                     int confs_ld, int B, int t_begin, int t_end, int pad, StopArgs stop) {
+  __shared__ int n_fin;
+  if (threadIdx.x == 0) n_fin = 0;
+  __syncthreads();
+  for (int b = threadIdx.x; b < B; b += SEL_THREADS) {
+    int f = 0;
+    for (int c = 1; c <= t_begin; ++c) f |= tokens[(int64_t)b * tokens_ld + c] == stop.eos;
+    stop.fin[b] = f;
+    if (f) atomicAdd(&n_fin, 1);
+  }
+  const int nt = t_end - t_begin;
+  for (int64_t i = threadIdx.x; i < (int64_t)B * nt; i += SEL_THREADS)
+    tokens[(i / nt) * tokens_ld + t_begin + 1 + i % nt] = pad;
+  const int c0 = (t_begin + 3) / 4, nc = (t_end + 3) / 4 - c0;      // conf columns of the steps t % 4 == 0 in [t_begin, t_end)
+  if (confs && nc > 0)
+    for (int64_t i = threadIdx.x; i < (int64_t)B * nc; i += SEL_THREADS) confs[(i / nc) * confs_ld + c0 + i % nc] = 0.f;
+  __syncthreads();
+  if (threadIdx.x == 0) { stop.state[0] = n_fin; stop.state[1] = n_fin == B; }
+}
+
 // select for the decode loop: reads the step's logits [B,V] (written by the head linear), optionally copies them
 // to the caller's logits tensor, then greedy / top-k / top-p select + max-prob.  One CTA per image.
+// With stop at EOS an image that has finished is left alone (its columns hold PAD / 0 from dec_stop_init_kernel); an image that
+// selects EOS is marked finished and counted, and the count reaching B sets the all-finished flag.  (An image not yet finished keeps
+// the count below B during this launch, so the flag cannot change under a CTA that runs.)
 __global__ void __launch_bounds__(SEL_THREADS) dec_select_kernel(const float* __restrict__ step_logits, int V, int Vp2, int t,
                                                                   float* __restrict__ logits_out, int64_t logits_img_stride, int logits_row,
                                                                   int32_t* __restrict__ tokens, int tokens_ld, int forced,
                                                                   float* __restrict__ confs, int confs_ld, const float* __restrict__ uniforms,
-                                                                  int uniforms_ld, int top_k, float top_p) {
+                                                                  int uniforms_ld, int top_k, float top_p, StopArgs stop) {
   extern __shared__ __align__(16) float sm[];
   float* lg = sm;             // V
   float* srt = lg + V;        // Vp2
   const int b = blockIdx.x;
+  if (stop.fin != nullptr && stop.fin[b]) return;
   for (int i = threadIdx.x; i < V; i += SEL_THREADS) {
     float v = step_logits[(int64_t)b * V + i];
     lg[i] = v;
@@ -942,6 +989,10 @@ __global__ void __launch_bounds__(SEL_THREADS) dec_select_kernel(const float* __
   if (threadIdx.x == 0) {
     if (!forced) tokens[(int64_t)b * tokens_ld + t + 1] = token;
     if (confs && (t % 4 == 0)) confs[(int64_t)b * confs_ld + t / 4] = conf;
+    if (stop.fin != nullptr && token == stop.eos) {
+      stop.fin[b] = 1;
+      if (atomicAdd(&stop.state[0], 1) + 1 == (int)gridDim.x) stop.state[1] = 1;
+    }
   }
 }
 
@@ -995,7 +1046,7 @@ int launch_linear(mdc_ctx* ctx, const XSrc& xs, const void* W, const float* bias
   {                                                                                                                                         \
     MDC_ENSURE_SMEM((dec_linear_stream_kernel<RELU_, MT_>), STREAM_SMEM);                                                                   \
     dec_linear_stream_kernel<RELU_, MT_><<<grid, LIN_THREADS, STREAM_SMEM, s>>>(X, ldx, (const __half*)W, bias, Y, ldy, yh, ldyh, B, N, K,   \
-                                                                                (const uint8_t*)next_w, (int)(next_w_bytes / 128));           \
+                                                                                (const uint8_t*)next_w, (int)(next_w_bytes / 128), xs.done); \
   }
       if (relu) { if (mt == 2) MDC_STREAM(true, 2) else MDC_STREAM(true, 1) }
       else { if (mt == 2) MDC_STREAM(false, 2) else MDC_STREAM(false, 1) }
@@ -1009,7 +1060,7 @@ int launch_linear(mdc_ctx* ctx, const XSrc& xs, const void* W, const float* bias
       XSrc src = xs;
       if (!plain) {
         MDC_TRY(launch_prep(ctx, xs, xh_buf, B, K, s));
-        src = XSrc{}; src.mode = XMODE_HALF; src.xh = xh_buf;
+        src = XSrc{}; src.mode = XMODE_HALF; src.xh = xh_buf; src.done = xs.done;
       }
       const size_t sm = (size_t)MMA_IMGS * (size_t)((K < MMA_KC ? K : MMA_KC) + MMA_PAD) * sizeof(__half);
       dim3 grid((N + MMA_ROWS - 1) / MMA_ROWS, (B + MMA_IMGS - 1) / MMA_IMGS);
@@ -1057,13 +1108,14 @@ int launch_linear(mdc_ctx* ctx, const XSrc& xs, const void* W, const float* bias
   MDC_LAUNCH_CHECK(ctx); return 0;
 }
 
-struct Scratch { float *xa, *xb, *xc, *y1, *y2, *y3, *qkv, *qc, *o, *oc, *f1, *lg; __half *xh, *oh, *f1h; };
+struct Scratch { float *xa, *xb, *xc, *y1, *y2, *y3, *qkv, *qc, *o, *oc, *f1, *lg; __half *xh, *oh, *f1h; int *fin, *stop_state; };
 
 size_t scratch_floats(const mdc_dims& d, int B) {
   // + the fp16 operand rows of the tensor-core linears (B x dim halves, behind the step logits, 16-byte aligned)
   // + the IEEE-half twins of the attention output and of the FFN hidden (operands of the weight-streaming linears)
+  // + the stop-at-EOS words (StopArgs: B finished flags, count, all-finished flag; 16-byte aligned)
   return (size_t)B * ((size_t)d.dim * 9 + (size_t)d.dim * 3 + d.dec_ffn + d.vocab) + 4 + ((size_t)B * d.dim + 1) / 2
-         + 8 + ((size_t)B * d.dim + 1) / 2 + ((size_t)B * d.dec_ffn + 1) / 2;
+         + 8 + ((size_t)B * d.dim + 1) / 2 + ((size_t)B * d.dec_ffn + 1) / 2 + 4 + B + 2;
 }
 
 Scratch carve(const mdc_dims& d, int B, void* p) {
@@ -1073,6 +1125,8 @@ Scratch carve(const mdc_dims& d, int B, void* p) {
   s.xh = reinterpret_cast<__half*>((reinterpret_cast<uintptr_t>(f) + 15) & ~(uintptr_t)15);
   s.oh = reinterpret_cast<__half*>((reinterpret_cast<uintptr_t>(s.xh + bd) + 15) & ~(uintptr_t)15);
   s.f1h = reinterpret_cast<__half*>((reinterpret_cast<uintptr_t>(s.oh + bd) + 15) & ~(uintptr_t)15);
+  s.fin = reinterpret_cast<int*>((reinterpret_cast<uintptr_t>(s.f1h + (size_t)B * d.dec_ffn) + 15) & ~(uintptr_t)15);
+  s.stop_state = s.fin + B;
   return s;
 }
 
@@ -1090,7 +1144,10 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
   // the batch pipeline asks for 16 images per cluster = "SM-time over latency": there every linear takes two row tiles per CTA (half the
   // CTAs; same bits -- the tile count does not enter any element's arithmetic).  A/B at B = 64: serial token-step +10 %, pipeline +9 %.
   const int mt2 = st->images_per_cluster >= 16 ? 512 : MDC_STREAM_MT2_MIN_N;
+  const StopArgs stop = st->stop_at_eos ? StopArgs{sc.fin, sc.stop_state, st->eos_token} : StopArgs{nullptr, nullptr, 0};
+  const int* done = st->stop_at_eos ? sc.stop_state + 1 : nullptr;
   XSrc prev{};   // how the next consumer obtains the layer input
+  prev.done = done;
   if (st->x_override) { prev.mode = XMODE_PLAIN; prev.x = st->x_override + (int64_t)t * dim; prev.ldx = (int64_t)st->x_override_ld * dim; }
   else {
     prev.mode = XMODE_EMBED; prev.tokens = st->tokens; prev.tokens_ld = st->tokens_ld; prev.t = t;
@@ -1107,19 +1164,19 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
   {                                                                                                                      \
     MDC_ENSURE_SMEM((dec_self_attn_kernel<T, HD_>), smem);                                                               \
     dec_self_attn_kernel<T, HD_><<<B, d.dec_heads * 32, smem, s>>>(sc.qkv, (T*)st->kv_pool, st->page_table, st->pages_per_seq, \
-        d.page_tokens, d.dec_layers, l, st->tokens, st->tokens_ld, d.pad_idx, t, dim, scale, sc.o, stream ? sc.oh : nullptr); \
+        d.page_tokens, d.dec_layers, l, st->tokens, st->tokens_ld, d.pad_idx, t, dim, scale, sc.o, stream ? sc.oh : nullptr, done); \
   }
       if (hd == 32) MDC_SA(32) else if (hd == 64) MDC_SA(64) else if (hd == 128) MDC_SA(128)
       else MDC_FAIL(-2, "decode: head width %d not in {32,64,128}", hd);
 #undef MDC_SA
       MDC_LAUNCH_CHECK(ctx);
     }
-    XSrc xo{}; xo.mode = XMODE_PLAIN; xo.x = sc.o; xo.ldx = dim;
+    XSrc xo{}; xo.mode = XMODE_PLAIN; xo.x = sc.o; xo.ldx = dim; xo.done = done;
     if (stream) { xo.xh = sc.oh; xo.ldxh = dim; }
     MDC_TRY(launch_linear<TW>(ctx, xo, lw[MDC_SA_OUT_W], (const float*)lw[MDC_SA_OUT_B], sc.y1, dim, B, dim, dim, false, s, sc.xh, nullptr, 0, mt2, lw[MDC_CA_IN_W], (size_t)dim * dim * sizeof(TW)));
     // cross-attention query from LN1(xa + y1); publishes xb
     XSrc x2{}; x2.mode = XMODE_LN; x2.resid = sc.xa; x2.delta = sc.y1; x2.ln_w = (const float*)lw[MDC_LN1_W]; x2.ln_b = (const float*)lw[MDC_LN1_B];
-    x2.eps = 1e-5f; x2.xn_out = sc.xb;
+    x2.eps = 1e-5f; x2.xn_out = sc.xb; x2.done = done;
     MDC_TRY(launch_linear<TW>(ctx, x2, lw[MDC_CA_IN_W], (const float*)lw[MDC_CA_IN_B], sc.qc, dim, B, dim, dim, false, s, sc.xh, nullptr, 0, mt2, lw[MDC_CA_OUT_W], (size_t)dim * dim * sizeof(TW)));
     {
       size_t smem = (size_t)d.dec_heads * (hd + d.n_patches) * sizeof(float);
@@ -1127,13 +1184,13 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
 #define MDC_CA(HD_)                                                                                         \
   {                                                                                                         \
     MDC_ENSURE_SMEM((dec_cross_attn_kernel<T, HD_>), smem);                                                 \
-    dec_cross_attn_kernel<T, HD_><<<B, d.dec_heads * 32, smem, s>>>(sc.qc, ckv, d.n_patches, dim, scale, sc.oc); \
+    dec_cross_attn_kernel<T, HD_><<<B, d.dec_heads * 32, smem, s>>>(sc.qc, ckv, d.n_patches, dim, scale, sc.oc, done); \
   }
 #define MDC_CAS(HD_)                                                                                        \
   {                                                                                                         \
     const size_t smem_s = (size_t)(HD_ + LIN_WARPS * HD_ + 2 * LIN_WARPS + d.n_patches) * sizeof(float);   \
     MDC_ENSURE_SMEM((dec_cross_attn_split_kernel<T, HD_>), smem_s);                                         \
-    dec_cross_attn_split_kernel<T, HD_><<<dim3(d.dec_heads, B), LIN_THREADS, smem_s, s>>>(sc.qc, ckv, d.n_patches, dim, scale, nullptr, sc.oh); \
+    dec_cross_attn_split_kernel<T, HD_><<<dim3(d.dec_heads, B), LIN_THREADS, smem_s, s>>>(sc.qc, ckv, d.n_patches, dim, scale, nullptr, sc.oh, done); \
   }
       if (stream) { if (hd == 32) MDC_CAS(32) else if (hd == 64) MDC_CAS(64) else MDC_CAS(128) }
       else if (hd == 32) MDC_CA(32) else if (hd == 64) MDC_CA(64) else MDC_CA(128)
@@ -1141,22 +1198,22 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
 #undef MDC_CAS
       MDC_LAUNCH_CHECK(ctx);
     }
-    XSrc xco{}; xco.mode = XMODE_PLAIN; xco.x = sc.oc; xco.ldx = dim;
+    XSrc xco{}; xco.mode = XMODE_PLAIN; xco.x = sc.oc; xco.ldx = dim; xco.done = done;
     if (stream) { xco.xh = sc.oh; xco.ldxh = dim; }
     MDC_TRY(launch_linear<TW>(ctx, xco, lw[MDC_CA_OUT_W], (const float*)lw[MDC_CA_OUT_B], sc.y2, dim, B, dim, dim, false, s, sc.xh, nullptr, 0, mt2, lw[MDC_FF1_W], (size_t)d.dec_ffn * dim * sizeof(TW)));
     // FFN
     XSrc x3{}; x3.mode = XMODE_LN; x3.resid = sc.xb; x3.delta = sc.y2; x3.ln_w = (const float*)lw[MDC_LN2_W]; x3.ln_b = (const float*)lw[MDC_LN2_B];
-    x3.eps = 1e-5f; x3.xn_out = sc.xc;
+    x3.eps = 1e-5f; x3.xn_out = sc.xc; x3.done = done;
     if (stream) MDC_TRY(launch_linear<TW>(ctx, x3, lw[MDC_FF1_W], (const float*)lw[MDC_FF1_B], nullptr, 0, B, d.dec_ffn, dim, true, s, sc.xh, sc.f1h, d.dec_ffn, mt2, lw[MDC_FF2_W], (size_t)d.dec_ffn * dim * sizeof(TW)));
     else MDC_TRY(launch_linear<TW>(ctx, x3, lw[MDC_FF1_W], (const float*)lw[MDC_FF1_B], sc.f1, d.dec_ffn, B, d.dec_ffn, dim, true, s, sc.xh, nullptr, 0, mt2));
-    XSrc xf{}; xf.mode = XMODE_PLAIN; xf.x = sc.f1; xf.ldx = d.dec_ffn;
+    XSrc xf{}; xf.mode = XMODE_PLAIN; xf.x = sc.f1; xf.ldx = d.dec_ffn; xf.done = done;
     // what the linear after FFN2 streams: the next layer's in-projection, or the vocabulary head
     const void* next_in_w = l + 1 < d.dec_layers ? (lw + MDC_DEC_LAYER_SLOTS)[MDC_SA_IN_W] : gw[MDC_OUT_W];
     const size_t next_in_bytes = l + 1 < d.dec_layers ? 3 * (size_t)dim * dim * sizeof(TW) : (size_t)d.vocab * dim * sizeof(TW);
     if (stream) { xf.xh = sc.f1h; xf.ldxh = d.dec_ffn; }
     MDC_TRY(launch_linear<TW>(ctx, xf, lw[MDC_FF2_W], (const float*)lw[MDC_FF2_B], sc.y3, dim, B, dim, d.dec_ffn, false, s, sc.xh, nullptr, 0, mt2, next_in_w, next_in_bytes));
     prev = XSrc{}; prev.mode = XMODE_LN; prev.resid = sc.xc; prev.delta = sc.y3; prev.ln_w = (const float*)lw[MDC_LN3_W];
-    prev.ln_b = (const float*)lw[MDC_LN3_B]; prev.eps = 1e-5f;
+    prev.ln_b = (const float*)lw[MDC_LN3_B]; prev.eps = 1e-5f; prev.done = done;
   }
   {
     const int V = d.vocab, Vp2 = next_pow2(V);
@@ -1165,7 +1222,7 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
     MDC_ENSURE_SMEM(dec_select_kernel, smem);
     dec_select_kernel<<<B, SEL_THREADS, smem, s>>>(sc.lg, V, Vp2, t, st->logits, (int64_t)st->logits_ld * V, t + st->logits_row_offset,
                                                   st->tokens, st->tokens_ld, st->forced, st->confs, st->confs_ld, st->uniforms,
-                                                  st->uniforms_ld, st->top_k, st->top_p);
+                                                  st->uniforms_ld, st->top_k, st->top_p, stop);
     MDC_LAUNCH_CHECK(ctx);
   }
   return 0;
@@ -1194,10 +1251,17 @@ extern "C" int mdc_decode_steps(mdc_model* m, const mdc_decode_state* st, int t_
   if (st->logits) MDC_CHECK_ARG(t_end + st->logits_row_offset <= st->logits_ld);
   if (st->confs) MDC_CHECK_ARG((t_end + 3) / 4 <= st->confs_ld);
   if ((st->top_k != 0 || st->top_p != 1.0f) && !st->forced) MDC_CHECK_ARG(st->uniforms && t_end <= st->uniforms_ld);
+  if (st->stop_at_eos) MDC_CHECK_ARG(!st->forced && !st->logits && st->eos_token >= 0 && st->eos_token < m->d.vocab);
   cudaStream_t s = (cudaStream_t)stream;
   if (t_end > t_begin && decode_cluster_supported(m, st, t_end)) {
     Scratch sc = carve(m->d, st->B, st->scratch);      // the cluster kernel only needs the step-logits area
     return decode_cluster_launch(m, st, t_begin, t_end, sc.lg, s);
+  }
+  if (st->stop_at_eos && t_end > t_begin) {
+    Scratch sc = carve(m->d, st->B, st->scratch);
+    dec_stop_init_kernel<<<1, SEL_THREADS, 0, s>>>(st->tokens, st->tokens_ld, st->confs, st->confs_ld, st->B, t_begin, t_end, m->d.pad_idx,
+                                                   StopArgs{sc.fin, sc.stop_state, st->eos_token});
+    MDC_LAUNCH_CHECK(m->ctx);
   }
   for (int t = t_begin; t < t_end; ++t) {
     if (m->d.precision == MDC_F32) MDC_TRY((decode_step_typed<float, float>(m, st, t, s)));

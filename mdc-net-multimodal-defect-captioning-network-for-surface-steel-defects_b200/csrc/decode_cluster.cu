@@ -83,8 +83,10 @@ struct Lay {
   static constexpr int OFF_PAGES = OFF_TOK + 2 * GMX * 4;         // [GMX][32] int32
   static constexpr int OFF_PADF = OFF_PAGES + GMX * 32 * 4;       // [GMX][8] u32: bit u of an image's 256-bit row = token u is PAD
   static constexpr int OFF_HASPAD = OFF_PADF + GMX * 32;          // [GMX] int32: any PAD token among the keys so far
-  static constexpr int OFF_BARS = OFF_HASPAD + GMX * 4;           // mbarriers
-  static constexpr int NBARS = 2 * NS_MAX + 5;
+  static constexpr int OFF_FIN = OFF_HASPAD + GMX * 4;            // stop at EOS: [2] u32 finished masks (by step parity), int all-finished,
+                                                                  // u32 the producer's BAR_STEP phase
+  static constexpr int OFF_BARS = OFF_FIN + 16;                   // mbarriers
+  static constexpr int NBARS = 2 * NS_MAX + 6;
   static constexpr int SMEM_USED = OFF_BARS + NBARS * 8;
   static constexpr int SMEM_BYTES = SMEM_USED + 1024;             // + alignment slack
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
@@ -93,7 +95,8 @@ struct Lay {
   static_assert(GMX * 2048 == STAGE, "a 16-key chunk of all images' K and V head slices fills a stage");
 };
 
-enum { BAR_FULL = 0, BAR_EMPTY = NS_MAX, BAR_O = 2 * NS_MAX, BAR_Y, BAR_F2, BAR_LG, BAR_TOK, BAR_COUNT };
+// BAR_STEP (stop at EOS only): the consumers' decision whether step t runs, handed to the producer before it emits step t's stages
+enum { BAR_FULL = 0, BAR_EMPTY = NS_MAX, BAR_O = 2 * NS_MAX, BAR_Y, BAR_F2, BAR_LG, BAR_TOK, BAR_STEP, BAR_COUNT };
 
 constexpr int BLOCKS_PER_LAYER = 22;   // packed weight blocks per (layer, CTA rank): in-proj q,k,v | self out | cross q | cross out | FFN1 x8 | FFN2 x8
 constexpr int HEAD_PACK_BYTES = BLK_BYTES + 8 * 512;    // per rank: vocabulary rows [0,32) as a 32-row block + rows [32,40) as an 8-row block
@@ -112,6 +115,7 @@ struct __align__(64) FusedParams {
   float* logits_out; int64_t logits_img_stride; int logits_row_offset;
   float* confs; int confs_ld;
   const float* uniforms; int uniforms_ld; int top_k; float top_p; int forced;
+  int eos;                                 // mdc_decode_state.eos_token (read by the kStop instantiations)
   int t_begin, t_end;
   long long* trace; int trace_t;           // developer aid: phase timestamps of CTA 0 at step trace_t (MDC_DECODE_TRACE_PTR)
   float ref_margin;                        // developer build: softmax reference-maximum margin (MDC_DECODE_REF_MARGIN; the product build uses 64)
@@ -291,7 +295,9 @@ __device__ __forceinline__ void warp_greedy_select(const float* lg, int V, int& 
 // instantiation carries no trace instructions.
 // NSTG ring stages; MINB = 2: compact shared-memory layout and a register budget that let two CTAs (of two different clusters,
 // i.e. two independent image groups) share an SM, so that one group's dependent phase chain fills the other's stalls.
-template <bool kTrace, int NB, int NSTG, int MINB>
+// kStop: stop at EOS (mdc_decode_state.stop_at_eos).  A template parameter, so that the instantiations without it compile to the code
+// they had before the option existed (as a run-time flag its few instructions shifted the register allocation: -1.2 % img/s).
+template <bool kTrace, int NB, int NSTG, int MINB, bool kStop>
 __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fused_kernel(const __grid_constant__ FusedParams P) {
   using Y = Lay<NB, NSTG, NB == 2 || MINB == 2>;
   constexpr int GMX = Y::GMX, NS = Y::NS, STAGE = Y::STAGE;
@@ -314,12 +320,15 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
   float* lrecv = (float*)(smem + Y::OFF_LRECV); float* selbuf = (float*)(smem + Y::OFF_SEL);
   int* tokbuf = (int*)(smem + Y::OFF_TOK); int* pages = (int*)(smem + Y::OFF_PAGES); uint32_t* padbits = (uint32_t*)(smem + Y::OFF_PADF);
   int* haspad = (int*)(smem + Y::OFF_HASPAD);
+  uint32_t* finm = (uint32_t*)(smem + Y::OFF_FIN); volatile int* all_fin = (int*)(smem + Y::OFF_FIN + 8);
+  uint32_t* ph_step = (uint32_t*)(smem + Y::OFF_FIN + 12);     // in shared memory: a register live across the group loop costs spills
   const uint32_t bars = sbase + Y::OFF_BARS;
   auto bar = [&](int i) -> uint32_t { return bars + i * 8; };
 
   if (tid == 0) {
     for (int i = 0; i < NS; ++i) { mbar_init(bar(BAR_FULL + i), 1); mbar_init(bar(BAR_EMPTY + i), 8); }
-    for (int i = BAR_O; i <= BAR_TOK; ++i) mbar_init(bar(i), 1);
+    for (int i = BAR_O; i < BAR_COUNT; ++i) mbar_init(bar(i), 1);
+    *ph_step = 0;
     fence_mbarrier_init();
   }
   // zero the ring and the activation operands once: rows >= G of the operands are multiplied by weights and must be finite
@@ -362,6 +371,13 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
       uint32_t any = 0;
       for (int w = 0; w < 8; ++w) any |= padbits[tid * 8 + w];
       haspad[tid] = any != 0u;
+    }
+    if (kStop && warp == 0) {      // images with an EOS among the known columns 1..t_begin are finished from the start
+      bool f = false;
+      if (lane < G)
+        for (int c = 1; c <= P.t_begin; ++c) f |= P.tokens[(int64_t)(img0 + lane) * P.tokens_ld + c] == P.eos;
+      const uint32_t m = __ballot_sync(0xffffffffu, f);
+      if (lane == 0) finm[(P.t_begin + 1) & 1] = m;      // read at step t_begin as "the mask before the previous step"
     }
     __syncthreads();
     cluster_sync();          // no peer may push into this CTA before its buffers are set up for the group
@@ -448,6 +464,27 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
         for (; c < n; ++c) { emit_kv(cross, l, c); if (cross) prefetch_ckv(l, c + PF_AHEAD); }
       };
       for (int t = P.t_begin; t < P.t_end; ++t) {
+        // stop at EOS: no stage of step t before the consumers have decided that it runs (from the tokens of step t - 1), so that the
+        // ring holds nothing the consumers would not take when the group ends here.  This gives up the producer's lookahead across the
+        // step boundary; without stopping the producer never waits here.
+        if (kStop) {
+          const uint32_t ph = *ph_step;
+          mbar_wait(bar(BAR_STEP), ph);
+          __syncwarp();
+          if (lane == 0) *ph_step = ph ^ 1u;
+          if (*all_fin) {
+            // the group ends before step t: token columns t+1..t_end and the conf columns of steps t..t_end-1 of the images this CTA
+            // selects for become PAD / 0 (never left to what the caller's buffers held).  The producer warp is idle from here on and
+            // the consumers wrote only columns <= t; filling here keeps the consumers' register allocation as it was.
+            for (int g = (int)rank; g < G; g += CS) {
+              int32_t* row = P.tokens + (int64_t)(img0 + g) * P.tokens_ld;
+              for (int c = t + 1 + lane; c <= P.t_end; c += 32) row[c] = P.pad_idx;
+              if (P.confs)
+                for (int c = (t + 3) / 4 + lane; c < (P.t_end + 3) / 4; c += 32) P.confs[(int64_t)(img0 + g) * P.confs_ld + c] = 0.f;
+            }
+            break;
+          }
+        }
         const int npg = (t + P.PT - 1) / P.PT;     // pages (= 16-key chunks) holding keys 0..t-1
         for (int l = 0; l < L; ++l) {
           wl = P.wpack + ((size_t)l * CS + rank) * BLOCKS_PER_LAYER * BLK_BYTES;
@@ -704,6 +741,17 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
 
       for (int t = P.t_begin; t < P.t_end; ++t) {
         const int npg = (t + P.PT - 1) / P.PT;
+        // ---- stop at EOS: finished mask before step t (bit g: image g has emitted EOS, or had one among columns 1..t_begin) and the
+        //      decision whether step t runs.  Every CTA of the cluster received the same tokens, so every CTA decides the same. -------
+        if (kStop && warp == 0) {
+          const bool eos_now = t > P.t_begin && lane < G && tokbuf[(t & 1) * GMX + lane] == P.eos;
+          const uint32_t f = finm[(t + 1) & 1] | __ballot_sync(0xffffffffu, eos_now);
+          if (lane == 0) {
+            finm[t & 1] = f;
+            *all_fin = f == (1u << G) - 1u;
+            mbar_arrive(bar(BAR_STEP));
+          }
+        }
         // ---- embedding + positional row (model.py:98-101); PAD flag of the token at position t --------------
         if (warp < G) {
           float pz[8];
@@ -726,6 +774,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
           }
         }
         cbar();
+        if (kStop && *all_fin) break;
         for (int l = 0; l < L; ++l) {
           TRACE(t);   // 0: layer start
           if (kTrace) wait_phase = 0;
@@ -974,6 +1023,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
           mbar_wait(bar(BAR_LG), ph_lg);
           ph_lg ^= 1;
           auto publish = [&](int img, int token, float conf) {     // one thread: token to the caller's buffer and to every peer
+            if (kStop && ((finm[t & 1] >> img) & 1u)) { token = P.pad_idx; conf = 0.f; }    // finished before step t
             if (!P.forced) {
               P.tokens[(int64_t)(img0 + img) * P.tokens_ld + t + 1] = token;
               const uint32_t off = sbase + Y::OFF_TOK + ((((t + 1) & 1) * GMX) + img) * 4;
@@ -1094,18 +1144,19 @@ bool geometry_ok(const mdc_dims& d) {
 // 2: NB = 1, 4-stage ring (64 KB), compact layout, two CTAs per SM (<= 8 images per cluster; two clusters interleave on the same SMs)
 constexpr int N_VARIANTS = 3;
 template <bool kTrace> struct Variants {
-  static const void* fn(int v) {
+  template <bool kStop> static const void* fn_(int v) {
     switch (v) {
-      case 0: return (const void*)decode_fused_kernel<kTrace, 1, 10, 1>;
-      case 1: return (const void*)decode_fused_kernel<kTrace, 2, 4, 1>;
-      default: return (const void*)decode_fused_kernel<kTrace, 1, 4, 2>;
+      case 0: return (const void*)decode_fused_kernel<kTrace, 1, 10, 1, kStop>;
+      case 1: return (const void*)decode_fused_kernel<kTrace, 2, 4, 1, kStop>;
+      default: return (const void*)decode_fused_kernel<kTrace, 1, 4, 2, kStop>;
     }
   }
+  static const void* fn(int v, bool stop) { return stop ? fn_<true>(v) : fn_<false>(v); }
 };
 int variant_smem(int v) { return v == 0 ? Lay<1, 10, false>::SMEM_BYTES : (v == 1 ? Lay<2, 4, true>::SMEM_BYTES : Lay<1, 4, true>::SMEM_BYTES); }
 
 // per-context (= per-device) launch state: the dynamic-smem opt-in and the occupancy query are device properties
-struct ClusterCtxState { int max_clusters[N_VARIANTS]; };
+struct ClusterCtxState { int max_clusters[N_VARIANTS][2]; };      // [variant][stop at EOS]
 
 }  // namespace
 
@@ -1194,6 +1245,7 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
   P.logits_out = st->logits; P.logits_img_stride = (int64_t)st->logits_ld * d.vocab; P.logits_row_offset = st->logits_row_offset;
   P.confs = st->confs; P.confs_ld = st->confs_ld;
   P.uniforms = st->uniforms; P.uniforms_ld = st->uniforms_ld; P.top_k = st->top_k; P.top_p = st->top_p; P.forced = st->forced;
+  P.eos = st->eos_token;
   P.t_begin = t_begin; P.t_end = t_end;
   P.trace = nullptr; P.trace_t = -1; P.ref_margin = 64.0f;
   int ipc = st->images_per_cluster, cps = st->ctas_per_sm;
@@ -1210,11 +1262,12 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
   if (!ctx->decode_state) { ClusterCtxState* cs = new ClusterCtxState(); memset(cs, 0, sizeof(*cs)); ctx->decode_state = cs; }
   ClusterCtxState* cs = (ClusterCtxState*)ctx->decode_state;
   const int smem = variant_smem(variant);
-  if (!cs->max_clusters[variant]) {
-    const void* fn = Variants<false>::fn(variant);
+  const bool stop = st->stop_at_eos != 0;
+  if (!cs->max_clusters[variant][stop]) {
+    const void* fn = Variants<false>::fn(variant, stop);
     MDC_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 #ifdef MDC_DEVTOOLS
-    MDC_CUDA(cudaFuncSetAttribute(Variants<true>::fn(variant), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    MDC_CUDA(cudaFuncSetAttribute(Variants<true>::fn(variant, stop), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 #endif
     cudaLaunchConfig_t q{}; q.gridDim = dim3(CS * 64); q.blockDim = dim3(NT); q.dynamicSmemBytes = smem;
     cudaLaunchAttribute a[1]; a[0].id = cudaLaunchAttributeClusterDimension; a[0].val.clusterDim.x = CS; a[0].val.clusterDim.y = 1; a[0].val.clusterDim.z = 1;
@@ -1222,9 +1275,9 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
     int n = 0;
     cudaError_t e = cudaOccupancyMaxActiveClusters(&n, fn, &q);
     if (e != cudaSuccess || n < 1) { (void)cudaGetLastError(); n = ctx->sm_count / CS / 2; if (n < 1) n = 1; }
-    cs->max_clusters[variant] = n;
+    cs->max_clusters[variant][stop] = n;
   }
-  const int max_clusters = cs->max_clusters[variant];
+  const int max_clusters = cs->max_clusters[variant][stop];
   int G = (P.B + max_clusters - 1) / max_clusters;
   if (ipc > 0 && ipc > G) G = ipc;                                                              // fewer, fuller clusters (batch pipelining)
   if (G > gmx) G = gmx;
@@ -1233,9 +1286,9 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
   P.n_groups = (P.B + G - 1) / G;
   const int n_clusters = P.n_groups < max_clusters ? P.n_groups : max_clusters;
   void* args[1] = {(void*)&P};
-  const void* fn = Variants<false>::fn(variant);
+  const void* fn = Variants<false>::fn(variant, stop);
 #ifdef MDC_DEVTOOLS
-  if (P.trace) fn = Variants<true>::fn(variant);
+  if (P.trace) fn = Variants<true>::fn(variant, stop);
 #endif
   MDC_CUDA(cudaLaunchKernel(fn, dim3(n_clusters * CS), dim3(NT), args, (size_t)smem, s));
   MDC_LAUNCH_CHECK(ctx);

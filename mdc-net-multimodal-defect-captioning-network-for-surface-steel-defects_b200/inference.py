@@ -15,18 +15,22 @@ from .config import CFG
 
 
 @torch.no_grad()
-def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None):
+def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None, stop_at_eos=False):
     """Returns (LongTensor (B, 1+max_len) on CPU, list of ceil(max_len/4) float tensors (B,) on CPU).
 
     `uniforms` (B, max_len) in [0,1) is an optional superset argument: the per-step uniform variates
     of the top-k/top-p sampler (inverse-CDF draw), so that sampling is reproducible; by default they
-    are drawn with torch.rand on the device (the reference uses torch.multinomial, inference_p.py:74)."""
+    are drawn with torch.rand on the device (the reference uses torch.multinomial, inference_p.py:74).
+    `stop_at_eos` (superset argument): stop at tokenizer.EOS_code.  Everything up to and including each
+    image's first EOS is bitwise the default result; after it the tokens are PAD and the confidences 0,
+    and decoding ends once every image has finished -- postprocess() returns the same either way."""
     bos = int(getattr(tokenizer, "BOS_code", CFG.bos_idx))
     if bos != int(CFG.bos_idx):
         raise ValueError("tokenizer.BOS_code must equal CFG.bos_idx (model.py:117 reads the global)")
     if not hasattr(model, "generate_tokens"):
         raise TypeError("generate() needs the B200 EncoderDecoder; there is no PyTorch fallback path")
-    tokens, confs = model.generate_tokens(x, max_len, top_k=top_k, top_p=top_p, uniforms=uniforms)
+    eos = _stop_token(tokenizer) if stop_at_eos else None
+    tokens, confs = model.generate_tokens(x, max_len, top_k=top_k, top_p=top_p, uniforms=uniforms, eos_token=eos)
     host = torch.empty(tokens.shape, dtype=torch.int32, pin_memory=True)
     host_c = torch.empty(confs.shape, dtype=torch.float32, pin_memory=True)
     host.copy_(tokens, non_blocking=True)
@@ -34,6 +38,13 @@ def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None):
     torch.cuda.current_stream(tokens.device).synchronize()      # the ONE sync of the whole call
     n_conf = (max_len + 3) // 4
     return host.long(), [host_c[:, i].clone() for i in range(n_conf)]
+
+
+def _stop_token(tokenizer):
+    """The stop token of `stop_at_eos`; finished rows are filled with CFG.pad_idx, so the tokenizer's PAD must be that token."""
+    if int(getattr(tokenizer, "PAD_code", CFG.pad_idx)) != int(CFG.pad_idx):
+        raise ValueError("stop_at_eos fills finished rows with CFG.pad_idx: tokenizer.PAD_code must equal it")
+    return int(tokenizer.EOS_code)
 
 
 def _preprocess_u8(img_u8, size, out, channels):

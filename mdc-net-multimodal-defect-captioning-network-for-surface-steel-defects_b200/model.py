@@ -297,8 +297,10 @@ class Engine:
 
     def decode(self, cross_kv, tokens, t_begin, t_end, *, max_tokens, forced, logits=None, logits_row_offset=0,
                confs=None, uniforms=None, top_k=0, top_p=1.0, pos_override=None, x_override=None, kv=None, scratch=None,
-               images_per_cluster=None, ctas_per_sm=None, per_op_kernels=None):
-        """Runs decode steps [t_begin, t_end) back to back on the current stream (no host sync)."""
+               images_per_cluster=None, ctas_per_sm=None, per_op_kernels=None, eos_token=None):
+        """Runs decode steps [t_begin, t_end) back to back on the current stream (no host sync).  `eos_token` (free-running only): stop
+        at that token -- after an image's first EOS its token columns are PAD and its confidences 0, and decoding ends once every image
+        has finished (mdc_decode_state.stop_at_eos)."""
         d = self.dims
         B = tokens.shape[0]
         assert tokens.dtype == torch.int32 and tokens.is_contiguous()
@@ -331,6 +333,8 @@ class Engine:
         st.images_per_cluster = int(opt["images_per_cluster"] if images_per_cluster is None else images_per_cluster)
         st.ctas_per_sm = int(opt["ctas_per_sm"] if ctas_per_sm is None else ctas_per_sm)
         st.per_op_kernels = int(opt["per_op_kernels"] if per_op_kernels is None else per_op_kernels)
+        if eos_token is not None:
+            st.stop_at_eos, st.eos_token = 1, int(eos_token)
         with torch.cuda.device(self.device):
             L.check(self.lib.mdc_decode_steps(self.handle, C.byref(st), t_begin, t_end, L.stream_ptr(self.device)))
         return kv, scratch
@@ -525,9 +529,13 @@ class EncoderDecoder(nn.Module, _EngineOwner):
 
     # -- the fast path used by generate(): encode once, cross-K/V once, incremental decode ---------
     @torch.no_grad()
-    def generate_tokens(self, image, max_new_tokens, top_k=0, top_p=1.0, uniforms=None, return_logits=False, use_graph=None):
+    def generate_tokens(self, image, max_new_tokens, top_k=0, top_p=1.0, uniforms=None, return_logits=False, use_graph=None,
+                        eos_token=None):
         """Returns (tokens int32 (B,1+T) on device, confs f32 (B,ceil(T/4)) on device[, logits (B,T,V)]).
-        The whole call (encoder, cross-K/V, T decode steps) is one CUDA graph replay per (B, T, sampler) shape."""
+        The whole call (encoder, cross-K/V, T decode steps) is one CUDA graph replay per (B, T, sampler, stop token) shape.
+        `eos_token`: stop at that token (superset argument).  Up to and including an image's first EOS the result is bitwise the
+        no-stop result; after it the tokens are PAD and the confidences 0, and decoding ends once every image has finished.  Not
+        with `return_logits` (steps that do not run have no logits; predict()/forward() serve that use)."""
         eng = self._engine(image.device if image.is_cuda else None)
         d = eng.dims
         T = int(max_new_tokens)
@@ -535,15 +543,21 @@ class EncoderDecoder(nn.Module, _EngineOwner):
             raise RuntimeError(f"max_len {T} exceeds CFG.max_len-1 = {d.max_pos}: the positional table has no more rows "
                                "(reference fails at model.py:93, Q6)")
         sampling = (top_k != 0 or top_p != 1)
+        if eos_token is not None:
+            if return_logits:
+                raise ValueError("return_logits=True cannot be combined with eos_token: steps that do not run have no logits")
+            eos_token = int(eos_token)
+            if not 0 <= eos_token < d.vocab:
+                raise ValueError(f"eos_token {eos_token} is outside the vocabulary [0, {d.vocab})")
         if use_graph is None:
             use_graph = os.environ.get("MDC_NO_GRAPH", "0") != "1"
-        key = (id(eng), image.shape[0], T, int(top_k), float(top_p), bool(return_logits), bool(use_graph), _decode_options_key())
+        key = (id(eng), image.shape[0], T, int(top_k), float(top_p), bool(return_logits), bool(use_graph), eos_token, _decode_options_key())
         plans = self.__dict__.setdefault("_plans", {})
         if plans.get("eng") is not eng:
             plans.clear(); plans["eng"] = eng
         plan = plans.get(key)
         if plan is None:
-            plan = GenerationPlan(eng, image.shape[0], T, top_k, top_p, sampling, return_logits, use_graph)
+            plan = GenerationPlan(eng, image.shape[0], T, top_k, top_p, sampling, return_logits, use_graph, eos_token=eos_token)
             plans[key] = plan
         if sampling and uniforms is None:
             uniforms = torch.rand((image.shape[0], T), dtype=torch.float32, device=eng.device)
@@ -557,17 +571,19 @@ class GenerationPlan:
     """Static buffers + (optionally) a captured CUDA graph for one (batch, new tokens, sampler) shape:
     encoder -> memory -> cross-K/V -> T decode steps, no host synchronisation anywhere inside."""
 
-    def __init__(self, eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split=False, images_per_cluster=None, ctas_per_sm=None):
+    def __init__(self, eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split=False, images_per_cluster=None, ctas_per_sm=None,
+                 eos_token=None):
         # everything below (allocations, warm-up launches, graph capture) on the ENGINE's device: torch.cuda.graph captures the current
         # device's stream, so with another device current the capture came back empty and replays did nothing (two-device test)
         with torch.cuda.device(eng.device):
-            self._build(eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split, images_per_cluster, ctas_per_sm)
+            self._build(eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split, images_per_cluster, ctas_per_sm, eos_token)
 
-    def _build(self, eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split, images_per_cluster, ctas_per_sm):
+    def _build(self, eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split, images_per_cluster, ctas_per_sm, eos_token):
         d = eng.dims
         dev = eng.device
         self.eng, self.B, self.T = eng, B, T
         self.top_k, self.top_p = int(top_k), float(top_p)
+        self.eos_token = eos_token
         self.images_per_cluster = _DECODE_OPTIONS["images_per_cluster"] if images_per_cluster is None else int(images_per_cluster)
         self.ctas_per_sm = _DECODE_OPTIONS["ctas_per_sm"] if ctas_per_sm is None else int(ctas_per_sm)
         self.per_op_kernels = bool(_DECODE_OPTIONS["per_op_kernels"])
@@ -635,7 +651,8 @@ class GenerationPlan:
         self.tokens[:, 0].fill_(int(CFG.bos_idx))
         eng.decode(self.ckv, self.tokens, 0, self.T, max_tokens=self.T, forced=False, logits=self.logits, logits_row_offset=0,
                    confs=self.confs, uniforms=self.uniforms, top_k=self.top_k, top_p=self.top_p, kv=self.kv, scratch=self.scratch,
-                   images_per_cluster=self.images_per_cluster, ctas_per_sm=self.ctas_per_sm, per_op_kernels=self.per_op_kernels)
+                   images_per_cluster=self.images_per_cluster, ctas_per_sm=self.ctas_per_sm, per_op_kernels=self.per_op_kernels,
+                   eos_token=self.eos_token)
 
     def run(self, image, uniforms=None):
         d = self.eng.dims

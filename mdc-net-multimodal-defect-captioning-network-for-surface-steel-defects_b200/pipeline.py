@@ -38,7 +38,8 @@ class Ticket:
 
 class GenerationPipeline:
     def __init__(self, model, batch, max_new_tokens, top_k=0, top_p=1.0, depth=None, decode_streams=None, images_per_cluster=16,
-                 ctas_per_sm=0, to_host=False, device=None):
+                 ctas_per_sm=0, to_host=False, device=None, eos_token=None):
+        """`eos_token`: stop at that token, as EncoderDecoder.generate_tokens(..., eos_token=...) does."""
         from .model import GenerationPlan
         if not hasattr(model, "_engine"):
             raise TypeError("GenerationPipeline needs the B200 EncoderDecoder; there is no PyTorch fallback path")
@@ -60,7 +61,8 @@ class GenerationPipeline:
         dev = eng.device
         with torch.cuda.device(dev):
             self.plans = [GenerationPlan(eng, self.B, T, top_k, top_p, self.sampling, False, True, split=True,
-                                         images_per_cluster=images_per_cluster, ctas_per_sm=ctas_per_sm) for _ in range(self.depth)]
+                                         images_per_cluster=images_per_cluster, ctas_per_sm=ctas_per_sm, eos_token=eos_token)
+                          for _ in range(self.depth)]
             self.s_enc = torch.cuda.Stream(device=dev, priority=0)      # encoder / cross-K/V: fills whatever the decodes leave idle
             self.s_copy = torch.cuda.Stream(device=dev, priority=0)     # host->device copy (+ the u8 transform) of the NEXT batch: on the
             # encoder stream the 38.5 MB f32 copy of a batch (~0.8 ms on PCIe) sat between two encoder passes (e2e 4 % below the device-resident rate)
@@ -133,14 +135,16 @@ class GenerationPipeline:
 
 
 @torch.no_grad()
-def generate_stream(model, batches, tokenizer, max_len=50, top_k=0, top_p=1, depth=None):
+def generate_stream(model, batches, tokenizer, max_len=50, top_k=0, top_p=1, depth=None, stop_at_eos=False):
     """The reference's inference loop as ONE pipelined call: yields, per batch and in order, what `generate(model, x, tokenizer,
     max_len, top_k, top_p)` returns -- (LongTensor (B,1+max_len) on CPU, list of ceil(max_len/4) float tensors (B,) on CPU).
     `batches` is any iterable of f32 (B,3,H,W) tensors (host, ideally pinned, or device) -- or of raw grayscale u8 (B,h,w)
-    tensors, normalised on the device (preprocess_gray)."""
+    tensors, normalised on the device (preprocess_gray).  `stop_at_eos`: as in generate()."""
     bos = int(getattr(tokenizer, "BOS_code", CFG.bos_idx))
     if bos != int(CFG.bos_idx):
         raise ValueError("tokenizer.BOS_code must equal CFG.bos_idx (model.py:117 reads the global)")
+    from .inference import _stop_token
+    eos = _stop_token(tokenizer) if stop_at_eos else None
     pipes, pipe, pending = model.__dict__.setdefault("_stream_pipes", {}), None, []     # plans + graphs are reused across calls
     n_conf = (max_len + 3) // 4
 
@@ -150,9 +154,10 @@ def generate_stream(model, batches, tokenizer, max_len=50, top_k=0, top_p=1, dep
 
     for x in batches:
         dev = x.device if x.is_cuda else None
-        key = ((x.shape[0], x.dim(), str(x.dtype)) if x.dtype == torch.uint8 else tuple(x.shape), int(max_len), int(top_k), float(top_p), depth, str(dev))
+        key = ((x.shape[0], x.dim(), str(x.dtype)) if x.dtype == torch.uint8 else tuple(x.shape), int(max_len), int(top_k), float(top_p), depth, str(dev), eos)
         if key not in pipes or pipes[key].eng is not model._engine(dev):      # new shape (e.g. the ragged last batch) / new weights
-            pipes[key] = GenerationPipeline(model, x.shape[0], max_len, top_k=top_k, top_p=top_p, depth=depth, to_host=True, device=dev)
+            pipes[key] = GenerationPipeline(model, x.shape[0], max_len, top_k=top_k, top_p=top_p, depth=depth, to_host=True, device=dev,
+                                            eos_token=eos)
         if pipes[key] is not pipe:
             while pending:                       # different plans share no events: drain before switching
                 yield finish(pending.pop(0))
