@@ -29,10 +29,10 @@
 extern "C" {
 #endif
 
-#define MDC_ABI_VERSION 6
+#define MDC_ABI_VERSION 7
 
-/* element types of activations / weights.  MDC_F16 (IEEE half) is only ever the type of the decode-loop weights, see
- * mdc_dims.dec_loop_dtype. */
+/* element types of activations / weights.  MDC_F16 (IEEE half) is the type of the decode-loop weights under precision MDC_BF16
+ * (see the weight table) and of mdc_gemm's fp16 mode. */
 enum { MDC_F32 = 0, MDC_BF16 = 1, MDC_F16 = 2 };
 
 /* GEMM epilogues: D = epi(A[M,K] . W[N,K]^T) */
@@ -127,18 +127,17 @@ typedef struct mdc_dims {
   int32_t pad_idx, bos_idx;
   int32_t has_axial;     /* axial_model.Decoder.axial_attention present */
   int32_t page_tokens;   /* self-attention KV page size in tokens (16) */
-  int32_t dec_loop_dtype;/* element type of the weights the autoregressive loop re-reads every step: MDC_SA_IN_W, MDC_SA_OUT_W,
-                            rows [0,dim) of MDC_CA_IN_W (the cross-attention query projection), MDC_CA_OUT_W, MDC_FF1_W, MDC_FF2_W
-                            and MDC_OUT_W.  MDC_F32 with precision MDC_F32; with precision MDC_BF16 either MDC_BF16 or MDC_F16.
-                            fp16 has the same footprint and tensor-core rate as bf16 but 3 more mantissa bits: rounding these
-                            weights to bf16 alone costs 1.4e-2 of the 2e-2 max-abs logit budget (tools/error_budget_cpu.py),
-                            to fp16 2e-3.  Rows [dim,3dim) of MDC_CA_IN_W (cross K/V in-projection, a tcgen05 GEMM against the
-                            bf16 memory) and every other GEMM weight stay `precision` typed; KV caches stay `precision` typed. */
 } mdc_dims;
 
 /* Weight table: device pointers in the order of enum mdc_weight_slot, per-layer slots repeated.
- * GEMM weights are `precision` typed [N,K] (decode-loop weights: `dec_loop_dtype`, see mdc_dims); everything else
- * (biases, norms, gammas, positional tables, embedding, cls token) is f32.  The library keeps the pointers, never copies. */
+ * GEMM weights are `precision` typed [N,K]; everything else (biases, norms, gammas, positional tables, embedding, cls token) is
+ * f32.  The library keeps the pointers, never copies.
+ * Decode-loop weights, the ones the autoregressive loop re-reads every step: MDC_SA_IN_W, MDC_SA_OUT_W, rows [0,dim) of
+ * MDC_CA_IN_W (the cross-attention query projection), MDC_CA_OUT_W, MDC_FF1_W, MDC_FF2_W and MDC_OUT_W.  They are f32 under
+ * precision MDC_F32 and IEEE half (MDC_F16) under MDC_BF16: fp16 has the same footprint and tensor-core rate as bf16 but 3 more
+ * mantissa bits, and rounding these weights to bf16 alone costs 1.4e-2 of the 2e-2 max-abs logit budget (tools/error_budget_cpu.py),
+ * to fp16 2e-3.  Rows [dim,3dim) of MDC_CA_IN_W (cross K/V in-projection, a tcgen05 GEMM against the bf16 memory) stay `precision`
+ * typed, like every other GEMM weight and the KV caches. */
 enum mdc_enc_slot {  /* encoder globals */
   MDC_W_PATCH = 0, MDC_B_PATCH, MDC_CLS, MDC_POS, MDC_NORM_W, MDC_NORM_B, MDC_ENC_GLOBAL_SLOTS
 };
@@ -156,6 +155,8 @@ enum mdc_dec_layer_slot {  /* per decoder layer, after the decoder globals */
   MDC_FF1_W, MDC_FF1_B, MDC_FF2_W, MDC_FF2_B, MDC_LN3_W, MDC_LN3_B, MDC_DEC_LAYER_SLOTS
 };
 
+/* With decoder layers, the decoder's head width (dim / dec_heads) must be 32, 64 or 128 and dim at most 1024: the widths the
+ * decode kernels cover.  Any other geometry is rejected here, before anything runs. */
 int mdc_model_create(mdc_ctx* ctx, const mdc_dims* dims, const void* const* weights, int n_weights,
                      mdc_model** out);
 int mdc_model_destroy(mdc_model* m);
@@ -235,7 +236,7 @@ typedef struct mdc_decode_state {
 } mdc_decode_state;
 
 size_t mdc_decode_workspace_bytes(const mdc_model* m, int B);
-/* Decode-loop weights (mdc_dims.dec_loop_dtype slots) pre-arranged for the fused decode kernel: per (layer, cluster rank) the
+/* Decode-loop weights (see the weight table) pre-arranged for the fused decode kernel: per (layer, cluster rank) the
  * 32-row blocks the kernel consumes, in consumption order, each stored as the exact shared-memory image its tensor-core
  * fragment loads expect -- one contiguous bulk copy per pipeline stage instead of per-row tensor-map traffic.
  * mdc_decode_pack_bytes() is 0 when the fused kernel does not cover the model's geometry (the per-operation kernels then

@@ -32,7 +32,7 @@ class Dims(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "precision", "img_size", "patch", "in_chans", "enc_dim", "enc_depth", "enc_heads", "enc_mlp",
         "n_patches", "dim", "dec_heads", "dec_layers", "dec_ffn", "vocab", "max_pos", "pad_idx", "bos_idx",
-        "has_axial", "page_tokens", "dec_loop_dtype")]
+        "has_axial", "page_tokens")]
 
 
 class TokenGrammar(C.Structure):

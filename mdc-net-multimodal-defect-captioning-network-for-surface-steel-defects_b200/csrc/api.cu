@@ -51,10 +51,17 @@ extern "C" int mdc_model_create(mdc_ctx* ctx, const mdc_dims* d, const void* con
   MDC_CHECK_ARG(ctx && d && weights && out);
   MDC_CHECK_ARG(d->precision == MDC_F32 || d->precision == MDC_BF16);
   MDC_CHECK_ARG(n_weights == mdc_model_num_weights(d));
-  MDC_CHECK_ARG(d->precision == MDC_F32 ? d->dec_loop_dtype == MDC_F32 : (d->dec_loop_dtype == MDC_BF16 || d->dec_loop_dtype == MDC_F16));
   MDC_CHECK_ARG(d->enc_dim % d->enc_heads == 0 && d->dim % d->dec_heads == 0);
   MDC_CHECK_ARG(d->enc_dim % 8 == 0 && d->dim % 32 == 0 && d->dec_ffn % 8 == 0);
   MDC_CHECK_ARG((d->dim / d->dec_heads) % 8 == 0 && (d->dim / d->dec_heads) <= 128);
+  if (d->dec_layers > 0) {
+    const int hd = d->dim / d->dec_heads;
+    if (hd != 32 && hd != 64 && hd != 128)
+      MDC_FAIL(-2, "mdc_model_create: decoder head width %d (dim %d / %d heads) is not supported: the decode kernels cover 32, 64 and 128",
+               hd, d->dim, d->dec_heads);
+    if (d->dim > MDC_MAX_DEC_DIM)
+      MDC_FAIL(-2, "mdc_model_create: decoder dim %d is not supported: the decode kernels cover at most %d", d->dim, MDC_MAX_DEC_DIM);
+  }
   MDC_CHECK_ARG(d->enc_depth == 0 || d->n_patches == (d->img_size / d->patch) * (d->img_size / d->patch));
   MDC_CHECK_ARG(d->page_tokens > 0 && d->vocab > 0 && d->vocab <= 4096 && d->max_pos > 0);
   mdc_model* m = (mdc_model*)calloc(1, sizeof(mdc_model));

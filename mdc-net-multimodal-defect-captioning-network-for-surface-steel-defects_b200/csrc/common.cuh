@@ -14,6 +14,9 @@ typedef __nv_bfloat16 bf16;
 
 constexpr float LOG2E = 1.4426950408889634f;
 
+// widest decoder model row the decode kernels build (LayerNorm-on-load / embedding operands); mdc_model_create rejects wider decoders
+constexpr int MDC_MAX_DEC_DIM = 1024;
+
 // ---- error plumbing ------------------------------------------------------------------------
 void mdc_set_error(const char* fmt, ...);
 #define MDC_FAIL(code, ...) do { mdc_set_error(__VA_ARGS__); return (code); } while (0)

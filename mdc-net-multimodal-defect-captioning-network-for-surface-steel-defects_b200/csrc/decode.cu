@@ -55,6 +55,98 @@ struct XSrc {
 // stop at EOS (per-operation path): every kernel of a step returns at entry once the whole batch has finished
 __device__ __forceinline__ bool batch_done(const int* done) { return done != nullptr && *done != 0; }
 
+// ---- operand rows: LayerNorm-on-load LN(resid + delta) or embedding emb[tokens[b, t]] + pos[t], K <= MDC_MAX_DEC_DIM columns ----
+// One builder per form, shared by the kernel that builds a linear's operand tile in shared memory and the one that builds the rows
+// as IEEE half in global memory, so a row has the same bits whichever kernel built it.
+
+// Scalar form, any K: lane handles the columns c = lane + 32 i < K of row b.
+//   REGS : v is a register array, v[i] = column c; the loops run a constant 32 times, unroll fully, and every load is in flight at once
+//   else : v is the row itself (shared memory), v[c] = column c; the loops stop at K
+template <bool REGS>
+__device__ __forceinline__ void operand_row(const XSrc& xs, int b, int K, float* v) {
+  const int lane = threadIdx.x & 31, cend = REGS ? lane + MDC_MAX_DEC_DIM : K;
+  auto at = [&](int i, int c) -> float& { return v[REGS ? i : c]; };
+  if (xs.mode == XMODE_EMBED) {
+    const int tok = xs.tokens[(int64_t)b * xs.tokens_ld + xs.t];
+    const float* e = xs.emb + (int64_t)tok * K; const float* pz = xs.pos + (int64_t)xs.t * K;
+    for (int c = lane, i = 0; c < cend; c += 32, ++i) { if (c < K) at(i, c) = e[c] + pz[c]; }
+  } else {
+    const float* a = xs.resid + (int64_t)b * K; const float* d = xs.delta + (int64_t)b * K;
+    float sum = 0.f;
+    for (int c = lane, i = 0; c < cend; c += 32, ++i) { if (c < K) { const float x = a[c] + d[c]; at(i, c) = x; sum += x; } }
+    const float mean = warp_sum(sum) / (float)K;
+    float q = 0.f;
+    for (int c = lane, i = 0; c < cend; c += 32, ++i) { if (c < K) { const float t = at(i, c) - mean; q += t * t; } }
+    const float rstd = 1.0f / sqrtf(warp_sum(q) / (float)K + xs.eps);
+    for (int c = lane, i = 0; c < cend; c += 32, ++i) { if (c < K) at(i, c) = (at(i, c) - mean) * rstd * xs.ln_w[c] + xs.ln_b[c]; }
+  }
+}
+
+// Vector form, K = NV * 128: lane holds the float4 at columns 128 i + 4 lane of the R rows b + 8 h, built in lockstep; rows past the
+// batch (>= B) are built from a valid row and must not be stored.  Every load of all R rows, the LayerNorm weights included, is issued
+// before the first reduction: one memory round trip instead of two.
+template <int NV, int R>
+__device__ __forceinline__ void operand_rows_vec(const XSrc& xs, int b, int B, float4 (&v)[R][NV]) {
+  static_assert(NV * 128 <= MDC_MAX_DEC_DIM, "operand rows are model rows");
+  constexpr int K = NV * 128;
+  const int lane = threadIdx.x & 31;
+  if (xs.mode == XMODE_EMBED) {
+    int tok[R];
+#pragma unroll
+    for (int h = 0; h < R; ++h) { const int bh = b + 8 * h; tok[h] = (bh < B) ? xs.tokens[(int64_t)bh * xs.tokens_ld + xs.t] : 0; }
+    float4 pz[NV];
+#pragma unroll
+    for (int i = 0; i < NV; ++i) pz[i] = __ldg(reinterpret_cast<const float4*>(xs.pos + (int64_t)xs.t * K + (i * 32 + lane) * 4));
+#pragma unroll
+    for (int h = 0; h < R; ++h)
+#pragma unroll
+      for (int i = 0; i < NV; ++i) v[h][i] = __ldg(reinterpret_cast<const float4*>(xs.emb + (int64_t)tok[h] * K + (i * 32 + lane) * 4));
+#pragma unroll
+    for (int h = 0; h < R; ++h)
+#pragma unroll
+      for (int i = 0; i < NV; ++i) { v[h][i].x += pz[i].x; v[h][i].y += pz[i].y; v[h][i].z += pz[i].z; v[h][i].w += pz[i].w; }
+  } else {  // XMODE_LN
+    float4 dl[R][NV];
+#pragma unroll
+    for (int h = 0; h < R; ++h) {
+      const int bh = min(b + 8 * h, B - 1);
+#pragma unroll
+      for (int i = 0; i < NV; ++i) {
+        v[h][i] = *reinterpret_cast<const float4*>(xs.resid + (int64_t)bh * K + (i * 32 + lane) * 4);
+        dl[h][i] = *reinterpret_cast<const float4*>(xs.delta + (int64_t)bh * K + (i * 32 + lane) * 4);
+      }
+    }
+    float4 g[NV], be[NV];
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+      g[i] = __ldg(reinterpret_cast<const float4*>(xs.ln_w + (i * 32 + lane) * 4));
+      be[i] = __ldg(reinterpret_cast<const float4*>(xs.ln_b + (i * 32 + lane) * 4));
+    }
+#pragma unroll
+    for (int h = 0; h < R; ++h) {
+      float sum = 0.f;
+#pragma unroll
+      for (int i = 0; i < NV; ++i) {
+        v[h][i].x += dl[h][i].x; v[h][i].y += dl[h][i].y; v[h][i].z += dl[h][i].z; v[h][i].w += dl[h][i].w;
+        sum += (v[h][i].x + v[h][i].y) + (v[h][i].z + v[h][i].w);
+      }
+      const float mean = warp_sum(sum) / (float)K;
+      float q = 0.f;
+#pragma unroll
+      for (int i = 0; i < NV; ++i) {
+        float a0 = v[h][i].x - mean, a1 = v[h][i].y - mean, a2 = v[h][i].z - mean, a3 = v[h][i].w - mean;
+        q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
+      }
+      const float rstd = 1.0f / sqrtf(warp_sum(q) / (float)K + xs.eps);
+#pragma unroll
+      for (int i = 0; i < NV; ++i) {
+        v[h][i].x = (v[h][i].x - mean) * rstd * g[i].x + be[i].x; v[h][i].y = (v[h][i].y - mean) * rstd * g[i].y + be[i].y;
+        v[h][i].z = (v[h][i].z - mean) * rstd * g[i].z + be[i].z; v[h][i].w = (v[h][i].w - mean) * rstd * g[i].w + be[i].w;
+      }
+    }
+  }
+}
+
 // Fill Xs[BT][K] (f32) for batch rows b0..b0+BT-1.
 __device__ __forceinline__ void load_x_tile(const XSrc& xs, float* Xs, int b0, int B, int K, bool publish) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -65,19 +157,8 @@ __device__ __forceinline__ void load_x_tile(const XSrc& xs, float* Xs, int b0, i
     if (xs.mode == XMODE_PLAIN) {
       const float* src = xs.x + (int64_t)b * xs.ldx;
       for (int c = lane * 4; c < K; c += 128) *reinterpret_cast<float4*>(row + c) = *reinterpret_cast<const float4*>(src + c);
-    } else if (xs.mode == XMODE_EMBED) {
-      const int tok = xs.tokens[(int64_t)b * xs.tokens_ld + xs.t];
-      const float* e = xs.emb + (int64_t)tok * K; const float* p = xs.pos + (int64_t)xs.t * K;
-      for (int c = lane; c < K; c += 32) row[c] = e[c] + p[c];
     } else {
-      const float* a = xs.resid + (int64_t)b * K; const float* d = xs.delta + (int64_t)b * K;
-      float s = 0.f;
-      for (int c = lane; c < K; c += 32) { float v = a[c] + d[c]; row[c] = v; s += v; }
-      float mean = warp_sum(s) / (float)K;
-      float q = 0.f;
-      for (int c = lane; c < K; c += 32) { float v = row[c] - mean; q += v * v; }
-      float rstd = 1.0f / sqrtf(warp_sum(q) / (float)K + xs.eps);
-      for (int c = lane; c < K; c += 32) row[c] = (row[c] - mean) * rstd * xs.ln_w[c] + xs.ln_b[c];
+      operand_row<false>(xs, b, K, row);
     }
     if (publish && xs.xn_out) {
       __syncwarp();
@@ -87,15 +168,14 @@ __device__ __forceinline__ void load_x_tile(const XSrc& xs, float* Xs, int b0, i
 }
 
 // Compile-time-K operand tile: every global load of the tile is in flight before the first use.
-//   PLAIN : cp.async 16-byte chunks straight into shared memory
-//   LN    : a warp owns rows (warp, warp+8); both rows' residual+delta slices are loaded as float4 first
-//   EMBED : token ids first (one round trip), then both embedding rows + the positional row
+//   PLAIN      : cp.async 16-byte chunks straight into shared memory; the only form of an operand wider than a model row
+//                (FFN2, K = 2048: mdc_model_create caps the model width at MDC_MAX_DEC_DIM)
+//   LN / EMBED : a warp owns rows (warp, warp+8), built in lockstep (operand_rows_vec)
 template <int K>
 __device__ __forceinline__ void load_x_tile_fast(const XSrc& xs, float* Xs, int b0, int B, bool publish) {
   static_assert(K % 128 == 0, "K must be a multiple of 128");
-  constexpr int V4 = K / 128;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (xs.mode == XMODE_PLAIN) {
+  if (K > MDC_MAX_DEC_DIM || xs.mode == XMODE_PLAIN) {
     constexpr int CH = K / 4;   // 16-byte chunks per row
 #pragma unroll 8
     for (int i = threadIdx.x; i < BT * CH; i += LIN_THREADS) {
@@ -113,72 +193,19 @@ __device__ __forceinline__ void load_x_tile_fast(const XSrc& xs, float* Xs, int 
     }
     return;
   }
-  if constexpr (K > 1024) { return; } else {   // LN / EMBED rows are model-width (<= 1024); wider K is only ever a PLAIN operand
-  float4 v[2][V4];
-  if (xs.mode == XMODE_EMBED) {
-    int tok[2];
-#pragma unroll
-    for (int h = 0; h < 2; ++h) { const int b = b0 + warp + 8 * h; tok[h] = (b < B) ? xs.tokens[(int64_t)b * xs.tokens_ld + xs.t] : 0; }
-    float4 pz[V4];
-#pragma unroll
-    for (int i = 0; i < V4; ++i) pz[i] = __ldg(reinterpret_cast<const float4*>(xs.pos + (int64_t)xs.t * K + (i * 32 + lane) * 4));
-#pragma unroll
-    for (int h = 0; h < 2; ++h)
-#pragma unroll
-      for (int i = 0; i < V4; ++i) v[h][i] = __ldg(reinterpret_cast<const float4*>(xs.emb + (int64_t)tok[h] * K + (i * 32 + lane) * 4));
-#pragma unroll
-    for (int h = 0; h < 2; ++h)
-#pragma unroll
-      for (int i = 0; i < V4; ++i) { v[h][i].x += pz[i].x; v[h][i].y += pz[i].y; v[h][i].z += pz[i].z; v[h][i].w += pz[i].w; }
-  } else {  // XMODE_LN
-    float4 dl[2][V4];
+  if constexpr (K <= MDC_MAX_DEC_DIM) {
+    constexpr int NV = K / 128;
+    float4 v[2][NV];
+    operand_rows_vec<NV, 2>(xs, b0 + warp, B, v);
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
-      const int b = min(b0 + warp + 8 * h, B - 1);
+      const int r = warp + 8 * h, b = b0 + r;
 #pragma unroll
-      for (int i = 0; i < V4; ++i) {
-        v[h][i] = *reinterpret_cast<const float4*>(xs.resid + (int64_t)b * K + (i * 32 + lane) * 4);
-        dl[h][i] = *reinterpret_cast<const float4*>(xs.delta + (int64_t)b * K + (i * 32 + lane) * 4);
+      for (int i = 0; i < NV; ++i) {
+        *reinterpret_cast<float4*>(Xs + (size_t)r * K + (i * 32 + lane) * 4) = (b < B) ? v[h][i] : make_float4(0, 0, 0, 0);
+        if (publish && xs.xn_out && b < B) *reinterpret_cast<float4*>(xs.xn_out + (int64_t)b * K + (i * 32 + lane) * 4) = v[h][i];
       }
     }
-    float4 g[V4], be[V4];
-#pragma unroll
-    for (int i = 0; i < V4; ++i) {
-      g[i] = __ldg(reinterpret_cast<const float4*>(xs.ln_w + (i * 32 + lane) * 4));
-      be[i] = __ldg(reinterpret_cast<const float4*>(xs.ln_b + (i * 32 + lane) * 4));
-    }
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      float sum = 0.f;
-#pragma unroll
-      for (int i = 0; i < V4; ++i) {
-        v[h][i].x += dl[h][i].x; v[h][i].y += dl[h][i].y; v[h][i].z += dl[h][i].z; v[h][i].w += dl[h][i].w;
-        sum += (v[h][i].x + v[h][i].y) + (v[h][i].z + v[h][i].w);
-      }
-      const float mean = warp_sum(sum) / (float)K;
-      float q = 0.f;
-#pragma unroll
-      for (int i = 0; i < V4; ++i) {
-        float a0 = v[h][i].x - mean, a1 = v[h][i].y - mean, a2 = v[h][i].z - mean, a3 = v[h][i].w - mean;
-        q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
-      }
-      const float rstd = 1.0f / sqrtf(warp_sum(q) / (float)K + xs.eps);
-#pragma unroll
-      for (int i = 0; i < V4; ++i) {
-        v[h][i].x = (v[h][i].x - mean) * rstd * g[i].x + be[i].x; v[h][i].y = (v[h][i].y - mean) * rstd * g[i].y + be[i].y;
-        v[h][i].z = (v[h][i].z - mean) * rstd * g[i].z + be[i].z; v[h][i].w = (v[h][i].w - mean) * rstd * g[i].w + be[i].w;
-      }
-    }
-  }
-#pragma unroll
-  for (int h = 0; h < 2; ++h) {
-    const int r = warp + 8 * h, b = b0 + r;
-#pragma unroll
-    for (int i = 0; i < V4; ++i) {
-      *reinterpret_cast<float4*>(Xs + (size_t)r * K + (i * 32 + lane) * 4) = (b < B) ? v[h][i] : make_float4(0, 0, 0, 0);
-      if (publish && xs.xn_out && b < B) *reinterpret_cast<float4*>(xs.xn_out + (int64_t)b * K + (i * 32 + lane) * 4) = v[h][i];
-    }
-  }
   }
 }
 
@@ -194,7 +221,7 @@ template <> struct Raw8<bf16> {
     for (int i = 0; i < 4; ++i) { float2 t = __bfloat1622float2(h[i]); f[2 * i] = t.x; f[2 * i + 1] = t.y; }
   }
 };
-template <> struct Raw8<__half> {      // decode-loop weights on the bf16 path (mdc_dims.dec_loop_dtype == MDC_F16)
+template <> struct Raw8<__half> {      // decode-loop weights under bf16 precision
   uint4 v;
   __device__ __forceinline__ void load(const __half* p) { v = __ldg(reinterpret_cast<const uint4*>(p)); }
   __device__ __forceinline__ void zero() { v = make_uint4(0, 0, 0, 0); }
@@ -331,9 +358,8 @@ constexpr int MMA_PAD = 4;         // halves of row padding: row pitch = 2 words
 // LayerNorm-on-load / embedding operand rows, built ONCE per linear (one warp per image, all images in parallel) as IEEE half in
 // global memory, and published as the next residual (xn_out, f32).  Building them inside every CTA of the linear -- eight rows per
 // warp, one after the other, three dependent memory round trips each -- was 75 % of that kernel's time (ncu, profiles/r2w).
-// K % 128 == 0 (every model width on the path): 128-bit loads and stores, lane holds columns 128 i + 4 lane .. +4 -- the scalar form below
-// issues 128 loads and 64 stores per lane for a 1024-wide row and was LSU-latency bound (7.9 us per launch at B = 64, a quarter of a
-// dim-1024 token-step)
+// K % 128 == 0 (every model width on the path): 128-bit loads and stores -- the scalar form below issues 128 loads and 64 stores per
+// lane for a 1024-wide row and was LSU-latency bound (7.9 us per launch at B = 64, a quarter of a dim-1024 token-step)
 template <int NV>
 __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_vec_kernel(XSrc xs, __half* __restrict__ xh, int B) {
   if (batch_done(xs.done)) return;
@@ -341,54 +367,14 @@ __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_vec_kernel(XSrc xs, _
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * LIN_WARPS + warp;
   if (b >= B) return;
-  float4 v[NV];
-  if (xs.mode == XMODE_EMBED) {
-    const int tok = xs.tokens[(int64_t)b * xs.tokens_ld + xs.t];
-    const float4* e = reinterpret_cast<const float4*>(xs.emb + (int64_t)tok * K) + lane;
-    const float4* pz = reinterpret_cast<const float4*>(xs.pos + (int64_t)xs.t * K) + lane;
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-      const float4 a = __ldg(e + 32 * i), c = __ldg(pz + 32 * i);
-      v[i] = make_float4(a.x + c.x, a.y + c.y, a.z + c.z, a.w + c.w);
-    }
-  } else {
-    const float4* a = reinterpret_cast<const float4*>(xs.resid + (int64_t)b * K) + lane;
-    const float4* d = reinterpret_cast<const float4*>(xs.delta + (int64_t)b * K) + lane;
-    float4 dl[NV];
-#pragma unroll
-    for (int i = 0; i < NV; ++i) { v[i] = a[32 * i]; dl[i] = d[32 * i]; }
-    float sum = 0.f;
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-      v[i].x += dl[i].x; v[i].y += dl[i].y; v[i].z += dl[i].z; v[i].w += dl[i].w;
-      sum += (v[i].x + v[i].y) + (v[i].z + v[i].w);
-    }
-    const float4* gw = reinterpret_cast<const float4*>(xs.ln_w) + lane;
-    const float4* gb = reinterpret_cast<const float4*>(xs.ln_b) + lane;
-    float4 gq[NV], bq[NV];             // requested before the two reductions: one memory round trip for the whole kernel instead of two
-#pragma unroll                        // (token-step at dim 1024, B = 64: 860 -> 777 us)
-    for (int i = 0; i < NV; ++i) { gq[i] = __ldg(gw + 32 * i); bq[i] = __ldg(gb + 32 * i); }
-    const float mean = warp_sum(sum) / (float)K;
-    float q = 0.f;
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-      const float a0 = v[i].x - mean, a1 = v[i].y - mean, a2 = v[i].z - mean, a3 = v[i].w - mean;
-      q += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
-    }
-    const float rstd = 1.0f / sqrtf(warp_sum(q) / (float)K + xs.eps);
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-      const float4 g = gq[i], be = bq[i];
-      v[i].x = (v[i].x - mean) * rstd * g.x + be.x; v[i].y = (v[i].y - mean) * rstd * g.y + be.y;
-      v[i].z = (v[i].z - mean) * rstd * g.z + be.z; v[i].w = (v[i].w - mean) * rstd * g.w + be.w;
-    }
-  }
+  float4 v[1][NV];
+  operand_rows_vec<NV, 1>(xs, b, B, v);
   uint2* oh = reinterpret_cast<uint2*>(xh + (int64_t)b * K) + lane;
   float4* of = xs.xn_out ? reinterpret_cast<float4*>(xs.xn_out + (int64_t)b * K) + lane : nullptr;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
-    oh[32 * i] = make_uint2(pack_f16x2_sat(v[i].x, v[i].y), pack_f16x2_sat(v[i].z, v[i].w));
-    if (of) of[32 * i] = v[i];
+    oh[32 * i] = make_uint2(pack_f16x2_sat(v[0][i].x, v[0][i].y), pack_f16x2_sat(v[0][i].z, v[0][i].w));
+    if (of) of[32 * i] = v[0][i];
   }
 }
 
@@ -397,27 +383,10 @@ __global__ void __launch_bounds__(LIN_THREADS) prep_x_half_kernel(XSrc xs, __hal
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * LIN_WARPS + warp;
   if (b >= B) return;
-  float v[MMA_KC / 32];                       // lane holds columns lane + 32 i
-  if (xs.mode == XMODE_EMBED) {
-    const int tok = xs.tokens[(int64_t)b * xs.tokens_ld + xs.t];
-    const float* e = xs.emb + (int64_t)tok * K; const float* pz = xs.pos + (int64_t)xs.t * K;
+  float v[MDC_MAX_DEC_DIM / 32];
+  operand_row<true>(xs, b, K, v);
 #pragma unroll
-    for (int i = 0; i < MMA_KC / 32; ++i) { const int c = lane + 32 * i; v[i] = c < K ? __ldg(e + c) + __ldg(pz + c) : 0.f; }
-  } else {
-    const float* a = xs.resid + (int64_t)b * K; const float* d = xs.delta + (int64_t)b * K;
-    float sum = 0.f;
-#pragma unroll
-    for (int i = 0; i < MMA_KC / 32; ++i) { const int c = lane + 32 * i; v[i] = c < K ? a[c] + d[c] : 0.f; sum += v[i]; }
-    const float mean = warp_sum(sum) / (float)K;
-    float q = 0.f;
-#pragma unroll
-    for (int i = 0; i < MMA_KC / 32; ++i) { const int c = lane + 32 * i; const float t = c < K ? v[i] - mean : 0.f; q += t * t; }
-    const float rstd = 1.0f / sqrtf(warp_sum(q) / (float)K + xs.eps);
-#pragma unroll
-    for (int i = 0; i < MMA_KC / 32; ++i) { const int c = lane + 32 * i; if (c < K) v[i] = (v[i] - mean) * rstd * __ldg(xs.ln_w + c) + __ldg(xs.ln_b + c); }
-  }
-#pragma unroll
-  for (int i = 0; i < MMA_KC / 32; ++i) {
+  for (int i = 0; i < MDC_MAX_DEC_DIM / 32; ++i) {
     const int c = lane + 32 * i;
     if (c < K) {
       xh[(int64_t)b * K + c] = f16_sat(v[i]);
@@ -547,10 +516,8 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_linear_mma_kernel(XSrc xs, co
 // lane (g, q) reads the 16 bytes X[image 8 nb + g][32 kb + 8 q .. +8) = both k-steps of the block under the same k permutation as
 // above.  The eight K-partials of the 16 x 64 tile are summed through shared memory in warp order (deterministic, batch-invariant).
 constexpr int STREAM_ROWS = 16;
-#ifndef MDC_STREAM_MT2_MIN_N
-#define MDC_STREAM_MT2_MIN_N 2048          // linears at least this wide take two 16-row tiles per CTA (A/B on B200, B = 64: every linear: serial
-                                           // token-step +10 %, pipeline +9 %; N >= 2048 only: serial -0.5 %, pipeline +5 %)
-#endif
+constexpr int STREAM_MT2_MIN_N = 2048;       // linears at least this wide take two 16-row tiles per CTA (A/B on B200, B = 64: every linear:
+                                             // serial token-step +10 %, pipeline +9 %; N >= 2048 only: serial -0.5 %, pipeline +5 %)
 constexpr int STREAM_PITCH = MMA_IMGS + 8;   // floats per row of a warp's partial tile
 constexpr int STREAM_SLOTS = 4;              // 32-column operand blocks in flight per warp (K = 1024: the warp's whole share)
 constexpr int STREAM_SLOT_BYTES = MMA_IMGS * 64;                                   // [64 images][32 halves]
@@ -826,11 +793,10 @@ __global__ void dec_cross_attn_kernel(const float* __restrict__ qc /*[B,d]*/, co
 // trips of 2 KB each for S = 196 (45 us per layer at B = 64, 1.1 TB/s).  Here warp w takes the passes w, w + 8, ..., all 512 CTAs of
 // a B = 64 launch are resident and every K (then V) byte of the layer is requested within four rounds.  Scores go through shared
 // memory; max / sum / the eight partial outputs are combined in warp order (deterministic).  Output as IEEE half = the operand of
-// the out-projection (and optionally f32).
+// the out-projection.
 template <typename TKV, int HD>
 __global__ void __launch_bounds__(LIN_THREADS) dec_cross_attn_split_kernel(const float* __restrict__ qc /*[B,d]*/, const TKV* __restrict__ ckv_layer,
-                                                                            int S, int d, float scale, float* __restrict__ o, __half* __restrict__ oh,
-                                                                            const int* done) {
+                                                                            int S, int d, float scale, __half* __restrict__ oh, const int* done) {
   if (batch_done(done)) return;
   constexpr int LPK = HD / 8, KPI = 32 / LPK, UN = 4;
   extern __shared__ float sm[];
@@ -923,8 +889,7 @@ __global__ void __launch_bounds__(LIN_THREADS) dec_cross_attn_split_kernel(const
 #pragma unroll
     for (int w = 1; w < LIN_WARPS; ++w) v += part[w * HD + c];
     v *= inv;
-    if (o) o[(int64_t)b * d + head * HD + c] = v;
-    if (oh) oh[(int64_t)b * d + head * HD + c] = f16_sat(v);
+    oh[(int64_t)b * d + head * HD + c] = f16_sat(v);
   }
 }
 
@@ -1029,7 +994,7 @@ inline bool stream_linears(int B, int K) { return B >= 16 && K % 256 == 0; }
 
 template <typename TW>
 int launch_linear(mdc_ctx* ctx, const XSrc& xs, const void* W, const float* bias, float* Y, int64_t ldy, int B, int N, int K,
-                  bool relu, cudaStream_t s, __half* xh_buf = nullptr, __half* yh = nullptr, int64_t ldyh = 0, int mt2_min_n = MDC_STREAM_MT2_MIN_N,
+                  bool relu, cudaStream_t s, __half* xh_buf = nullptr, __half* yh = nullptr, int64_t ldyh = 0, int mt2_min_n = STREAM_MT2_MIN_N,
                   const void* next_w = nullptr, size_t next_w_bytes = 0) {
   MDC_CHECK_ARG(K % 8 == 0);
   if constexpr (std::is_same<TW, __half>::value) {
@@ -1130,9 +1095,11 @@ Scratch carve(const mdc_dims& d, int B, void* p) {
   return s;
 }
 
-// TW: element type of the decode-loop weights (mdc_dims.dec_loop_dtype), T: element type of the KV caches (`precision`)
-template <typename TW, typename T>
+// T: element type of the KV caches (`precision`); TW: element type of the decode-loop weights, f32 under fp32 and IEEE half under bf16
+template <typename T>
 int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStream_t s) {
+  using TW = typename std::conditional<std::is_same<T, float>::value, float, __half>::type;
+  constexpr bool HALF = std::is_same<TW, __half>::value;
   mdc_ctx* ctx = m->ctx; const mdc_dims& d = m->d;
   const int B = st->B, dim = d.dim, hd = dim / d.dec_heads;
   const void** gw = m->w + MDC_ENC_GLOBAL_SLOTS + d.enc_depth * MDC_ENC_BLOCK_SLOTS;
@@ -1140,10 +1107,10 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
   Scratch sc = carve(d, B, st->scratch);
   const float scale = 1.0f / sqrtf((float)hd);
   // wide batches on fp16 decode-loop weights: weight-streaming linears fed with IEEE-half operands by their producers
-  const bool stream = std::is_same<TW, __half>::value && stream_linears(B, dim) && stream_linears(B, d.dec_ffn) && dim % 8 == 0;
+  const bool stream = HALF && stream_linears(B, dim) && stream_linears(B, d.dec_ffn) && dim % 8 == 0;
   // the batch pipeline asks for 16 images per cluster = "SM-time over latency": there every linear takes two row tiles per CTA (half the
   // CTAs; same bits -- the tile count does not enter any element's arithmetic).  A/B at B = 64: serial token-step +10 %, pipeline +9 %.
-  const int mt2 = st->images_per_cluster >= 16 ? 512 : MDC_STREAM_MT2_MIN_N;
+  const int mt2 = st->images_per_cluster >= 16 ? 512 : STREAM_MT2_MIN_N;
   const StopArgs stop = st->stop_at_eos ? StopArgs{sc.fin, sc.stop_state, st->eos_token} : StopArgs{nullptr, nullptr, 0};
   const int* done = st->stop_at_eos ? sc.stop_state + 1 : nullptr;
   XSrc prev{};   // how the next consumer obtains the layer input
@@ -1166,8 +1133,7 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
     dec_self_attn_kernel<T, HD_><<<B, d.dec_heads * 32, smem, s>>>(sc.qkv, (T*)st->kv_pool, st->page_table, st->pages_per_seq, \
         d.page_tokens, d.dec_layers, l, st->tokens, st->tokens_ld, d.pad_idx, t, dim, scale, sc.o, stream ? sc.oh : nullptr, done); \
   }
-      if (hd == 32) MDC_SA(32) else if (hd == 64) MDC_SA(64) else if (hd == 128) MDC_SA(128)
-      else MDC_FAIL(-2, "decode: head width %d not in {32,64,128}", hd);
+      if (hd == 32) MDC_SA(32) else if (hd == 64) MDC_SA(64) else MDC_SA(128)      // the head widths mdc_model_create accepts
 #undef MDC_SA
       MDC_LAUNCH_CHECK(ctx);
     }
@@ -1190,9 +1156,9 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
   {                                                                                                         \
     const size_t smem_s = (size_t)(HD_ + LIN_WARPS * HD_ + 2 * LIN_WARPS + d.n_patches) * sizeof(float);   \
     MDC_ENSURE_SMEM((dec_cross_attn_split_kernel<T, HD_>), smem_s);                                         \
-    dec_cross_attn_split_kernel<T, HD_><<<dim3(d.dec_heads, B), LIN_THREADS, smem_s, s>>>(sc.qc, ckv, d.n_patches, dim, scale, nullptr, sc.oh, done); \
+    dec_cross_attn_split_kernel<T, HD_><<<dim3(d.dec_heads, B), LIN_THREADS, smem_s, s>>>(sc.qc, ckv, d.n_patches, dim, scale, sc.oh, done); \
   }
-      if (stream) { if (hd == 32) MDC_CAS(32) else if (hd == 64) MDC_CAS(64) else MDC_CAS(128) }
+      if (stream) { if constexpr (HALF) { if (hd == 32) MDC_CAS(32) else if (hd == 64) MDC_CAS(64) else MDC_CAS(128) } }
       else if (hd == 32) MDC_CA(32) else if (hd == 64) MDC_CA(64) else MDC_CA(128)
 #undef MDC_CA
 #undef MDC_CAS
@@ -1264,9 +1230,8 @@ extern "C" int mdc_decode_steps(mdc_model* m, const mdc_decode_state* st, int t_
     MDC_LAUNCH_CHECK(m->ctx);
   }
   for (int t = t_begin; t < t_end; ++t) {
-    if (m->d.precision == MDC_F32) MDC_TRY((decode_step_typed<float, float>(m, st, t, s)));
-    else if (m->d.dec_loop_dtype == MDC_F16) MDC_TRY((decode_step_typed<__half, bf16>(m, st, t, s)));
-    else MDC_TRY((decode_step_typed<bf16, bf16>(m, st, t, s)));
+    if (m->d.precision == MDC_F32) MDC_TRY(decode_step_typed<float>(m, st, t, s));
+    else MDC_TRY(decode_step_typed<bf16>(m, st, t, s));
   }
   return 0;
 }

@@ -15,7 +15,7 @@
 //     ahead of the 8 consumer warps across phase, layer and step boundaries.
 //   * projections run on the tensor cores with the roles swapped: the WEIGHT rows are the MMA M dimension
 //     (mma.sync m16n8k16, A fragments by ldmatrix from the swizzled TMA tile), the images are the N = 8
-//     dimension (one or two column blocks per weight fragment), so no MMA lane is wasted on padding.  The decode-loop weights are IEEE fp16 (mdc_dims.dec_loop_dtype: same
+//     dimension (one or two column blocks per weight fragment), so no MMA lane is wasted on padding.  The decode-loop weights are IEEE fp16 (the weight table of mdc_b200.h: same
 //     bytes as bf16, 8x smaller rounding) and so are the projection operands (activations rounded to fp16: 11 significant bits).
 //     Attention keeps bf16 K/V (the caches) with bf16 queries and probabilities.
 //   * activations (a few KB) are exchanged through DISTRIBUTED SHARED MEMORY, push style: the producer of a slice
@@ -1132,7 +1132,7 @@ struct FusedCache {
 };
 
 bool geometry_ok(const mdc_dims& d) {
-  if (d.precision != MDC_BF16 || d.dec_loop_dtype != MDC_F16 || d.dim != DM || d.dec_heads != CS || d.dec_ffn != FFN) return false;
+  if (d.precision != MDC_BF16 || d.dim != DM || d.dec_heads != CS || d.dec_ffn != FFN) return false;
   if (d.dec_layers < 1 || d.dec_layers > 8 || d.vocab > CS * VSL || d.vocab < 8) return false;
   if (d.n_patches < 1 || d.page_tokens != 16) return false;
   return true;

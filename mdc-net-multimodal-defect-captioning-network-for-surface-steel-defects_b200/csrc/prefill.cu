@@ -246,7 +246,7 @@ size_t ws_bytes(const mdc_dims& d, int B, int n) {
 
 bool geometry_ok(const mdc_dims& d) {
   const int hd = d.dec_heads > 0 ? d.dim / d.dec_heads : 0;
-  return d.precision == MDC_BF16 && d.dec_loop_dtype == MDC_F16 && (d.dim == 256 || d.dim == 512 || d.dim == 1024) && hd * d.dec_heads == d.dim &&
+  return d.precision == MDC_BF16 && (d.dim == 256 || d.dim == 512 || d.dim == 1024) && hd * d.dec_heads == d.dim &&
          (hd == 32 || hd == 64 || hd == 128) && d.dec_ffn % 8 == 0 && d.dec_layers >= 1;
 }
 

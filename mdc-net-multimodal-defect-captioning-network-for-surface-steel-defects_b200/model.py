@@ -186,7 +186,6 @@ class Engine:
 
         d = L.Dims()
         d.precision = self.code
-        d.dec_loop_dtype = L.MDC_F16 if self.dtype == torch.bfloat16 else L.MDC_F32
         d.page_tokens = int(getattr(CFG, "kv_page_tokens", 16))
         d.pad_idx, d.bos_idx = int(CFG.pad_idx), int(CFG.bos_idx)
         if encoder is not None:
