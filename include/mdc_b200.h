@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MDC_ABI_VERSION 7
+#define MDC_ABI_VERSION 8
 
 /* element types of activations / weights.  MDC_F16 (IEEE half) is the type of the decode-loop weights under precision MDC_BF16
  * (see the weight table) and of mdc_gemm's fp16 mode. */
@@ -261,6 +261,50 @@ int mdc_decode_steps(mdc_model* m, const mdc_decode_state* st, int t_begin, int 
 size_t mdc_decoder_prefill_workspace_bytes(const mdc_model* m, int B, int n);
 int mdc_decoder_prefill(mdc_model* m, const int32_t* tokens, int tokens_ld, int B, int n, const float* pos, const void* cross_kv,
                         float* logits, int logits_ld, int row_offset, int n_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- beam search over the paged KV cache ---------------------------------------------------------------------------------
+ * B images, K beams (1 <= K <= 16).  Row r = b*K + k of every [B*K, ...] buffer is beam k of image b; each row keeps a score s_r and a
+ * finish step f_r (-1 while running).  Start: every token row [BOS, PAD, ...], s = 0 for k = 0 and -inf otherwise, f = -1; the page
+ * table equals own_pages.  Step t (t = 0 .. T-1): mdc_decode_steps(t, t+1) teacher-forced (forced = 1) over the B*K rows writes the
+ * step-t logits l, then mdc_beam_step(t):
+ *   lp_r[v] = (l_v - m) - log sum_u exp(l_u - m) in f32 (m = row max; accurate expf/logf, a fixed reduction order);
+ *   candidates: every (r, v) of a running row with s_r > -inf, scored s_r + lp_r[v]; exactly (r, PAD) at s_r for a finished row;
+ *   per image the K best are kept (ties: lower beam index k, then lower token id); new beam j (0 = best) takes the parent's token row
+ *   with column t+1 = v, the parent's KV of positions 0..t, the new score, f = f_parent if the parent had finished, t if v == eos_token,
+ *   else -1, and the parent's per-token histories plus this step's entries: log-prob lp (0 for a finished parent's PAD) at column t,
+ *   confidence exp(lp) (0 for a finished parent) at column t/4 when t % 4 == 0.
+ * A row's score is therefore, bit for bit, the f32 sum of its per-token log-probs in step order.  No early exit, no sampling.
+ * KV pages: row r writes only its own page own_pages[r][t / page_tokens] at step t.  At the reorder after step t (jc = t / page_tokens)
+ * entries i < jc of a new beam's live row are its parent's (full pages, never written again, shared); entry jc is the parent's too when
+ * step t filled that page, and otherwise the beam's own page jc, into which the parent's valid token slots 0 .. t % page_tokens are
+ * copied (every layer, head, K and V; only when the parent is another row).  Parents' rows and pages are staged through the workspace
+ * first, because a destination can be another child's source.  Buffers never move, so a whole beam search captures as one CUDA graph.
+ *   tokens       int32 [B*K, tokens_ld]            the decode state's token rows (t + 1 < tokens_ld)
+ *   kv_pool      the decode state's pool; page_table the live int32 [B*K, pages_per_seq] table mdc_decode_steps reads (rewritten here);
+ *   own_pages    int32 [B*K, pages_per_seq] the rows' initial, distinct pages (never written)
+ *   scores f32 [B*K], finish_step int32 [B*K]; token_logprobs f32 [B*K, token_logprobs_ld] and confs f32 [B*K, confs_ld], either NULL
+ *   workspace    mdc_beam_workspace_bytes() (0 for K outside 1..16)
+ * mdc_beam_finalize: normalised score s / len^length_penalty, len = f + 1 for a finished beam and T otherwise; order_out int32 [B, K]
+ * lists each image's beam indices by normalised score, descending (ties: lower index first), norm_scores_out f32 [B, K] in that order.
+ * Rejected with a message: K outside 1..16 or above the vocabulary, vocab > 4096, eos_token outside the vocabulary, a t past the
+ * positional table, the token columns or the pages, a short workspace. */
+typedef struct mdc_beam_state {
+  int32_t B, K;
+  int32_t* tokens; int32_t tokens_ld;
+  void* kv_pool; int32_t* page_table; const int32_t* own_pages; int32_t pages_per_seq;
+  float* scores; int32_t* finish_step;
+  float* token_logprobs; int32_t token_logprobs_ld;
+  float* confs; int32_t confs_ld;
+  int32_t eos_token;
+  void* workspace; size_t workspace_bytes;
+} mdc_beam_state;
+
+size_t mdc_beam_workspace_bytes(const mdc_model* m, int B, int K);
+/* selection, reorder and partial-page copy after step t: logits f32, row r's step-t logits at logits + r * logits_ld.  At most three
+ * launches, no host synchronisation. */
+int mdc_beam_step(mdc_model* m, const mdc_beam_state* st, const float* logits, int64_t logits_ld, int t, void* stream);
+int mdc_beam_finalize(mdc_model* m, const mdc_beam_state* st, int T, float length_penalty, int32_t* order_out /*[B,K]*/,
+                      float* norm_scores_out /*[B,K]*/, void* stream);
 
 /* (d) head + select as a stand-alone op: logits f32 [B,V] -> token, max prob, probability of the selected token.
  * greedy: argmax(softmax(logits)) = first max index (inference_p.py:77);

@@ -9,7 +9,7 @@ from .tokenizer import Tokenizer, top_k_sampling, top_k_sampling_with_scores_2d
 from .model import Encoder, Decoder, EncoderDecoder, Engine, decode_options
 from .axial_model import AxialAttention
 from . import axial_model
-from .inference import generate, postprocess, postprocess_with_captions, preprocess_gray, preprocess_bgr
+from .inference import generate, generate_beam, postprocess, postprocess_with_captions, preprocess_gray, preprocess_bgr
 from .pipeline import GenerationPipeline, generate_stream
 from .iou import (bbox_iou, calculate_batch_iou, calculate_batch_max_iou, calculate_batch_max_iou_torchvision,
                   calculate_batch_max_iou_masked, giou_pairwise, giou_loss_with_scores, calculate_iou, iou_loss)
@@ -20,6 +20,6 @@ from .metrics import MeanAveragePrecision, calculate_bleu_scores
 from . import _lib
 
 __all__ = ["CFG", "Tokenizer", "top_k_sampling", "top_k_sampling_with_scores_2d", "Encoder", "Decoder", "EncoderDecoder", "Engine", "decode_options", "AxialAttention", "axial_model",
-           "generate", "postprocess", "postprocess_with_captions", "preprocess_gray", "preprocess_bgr", "GenerationPipeline", "generate_stream", "bbox_iou", "calculate_batch_iou", "calculate_batch_max_iou",
+           "generate", "generate_beam", "postprocess", "postprocess_with_captions", "preprocess_gray", "preprocess_bgr", "GenerationPipeline", "generate_stream", "bbox_iou", "calculate_batch_iou", "calculate_batch_max_iou",
            "calculate_batch_max_iou_torchvision", "calculate_batch_max_iou_masked", "giou_pairwise",
            "giou_loss_with_scores", "calculate_iou", "iou_loss", "PagedKVCache", "PageAllocator", "parallel", "metrics", "MeanAveragePrecision", "calculate_bleu_scores"]

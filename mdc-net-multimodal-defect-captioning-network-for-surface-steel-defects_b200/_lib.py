@@ -64,6 +64,19 @@ class DecodeState(C.Structure):
     ]
 
 
+class BeamState(C.Structure):
+    _fields_ = [
+        ("B", C.c_int32), ("K", C.c_int32),
+        ("tokens", C.c_void_p), ("tokens_ld", C.c_int32),
+        ("kv_pool", C.c_void_p), ("page_table", C.c_void_p), ("own_pages", C.c_void_p), ("pages_per_seq", C.c_int32),
+        ("scores", C.c_void_p), ("finish_step", C.c_void_p),
+        ("token_logprobs", C.c_void_p), ("token_logprobs_ld", C.c_int32),
+        ("confs", C.c_void_p), ("confs_ld", C.c_int32),
+        ("eos_token", C.c_int32),
+        ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t),
+    ]
+
+
 _P, _I, _L, _F, _SZ = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_size_t
 
 # name -> (restype, argtypes); the complete export list of include/mdc_b200.h
@@ -94,6 +107,9 @@ SIGNATURES = {
     "mdc_decode_steps": (_I, [_P, C.POINTER(DecodeState), _I, _I, _P]),
     "mdc_decoder_prefill_workspace_bytes": (_SZ, [_P, _I, _I]),
     "mdc_decoder_prefill": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _I, _I, _I, _P, _SZ, _P]),
+    "mdc_beam_workspace_bytes": (_SZ, [_P, _I, _I]),
+    "mdc_beam_step": (_I, [_P, C.POINTER(BeamState), _P, _L, _I, _P]),
+    "mdc_beam_finalize": (_I, [_P, C.POINTER(BeamState), _I, _F, _P, _P, _P]),
     "mdc_select": (_I, [_P, _P, _L, _I, _I, _I, _F, _P, _P, _P, _P, _P]),
     "mdc_axial_workspace_bytes": (_SZ, [_P, _I, _I]),
     "mdc_axial_attention": (_I, [_P, _P, _I, _I, _I, _P, _P, _SZ, _P]),

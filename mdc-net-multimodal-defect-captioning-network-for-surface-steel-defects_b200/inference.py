@@ -40,6 +40,34 @@ def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None, s
     return host.long(), [host_c[:, i].clone() for i in range(n_conf)]
 
 
+@torch.no_grad()
+def generate_beam(model, x, tokenizer, max_len=50, num_beams=4, length_penalty=1.0):
+    """Beam search (superset function): returns exactly what generate() returns -- LongTensor (B, 1+max_len) and a list of
+    ceil(max_len/4) (B,) confidence tensors, on CPU -- for each image's best beam by score / len^length_penalty, so that postprocess()
+    and postprocess_with_captions() read it unchanged.  Beams end at tokenizer.EOS_code (the tokens after it are PAD, the confidences 0);
+    there is no early exit once every beam has ended, and no sampling inside beams.  Semantics: DESIGN.md §3.4c."""
+    bos = int(getattr(tokenizer, "BOS_code", CFG.bos_idx))
+    if bos != int(CFG.bos_idx):
+        raise ValueError("tokenizer.BOS_code must equal CFG.bos_idx (model.py:117 reads the global)")
+    if not hasattr(model, "generate_beam_tokens"):
+        raise TypeError("generate_beam() needs the B200 EncoderDecoder; there is no PyTorch fallback path")
+    if not 1 <= int(num_beams) <= 16:
+        raise ValueError(f"num_beams {num_beams} is outside 1..16")
+    if int(max_len) > int(CFG.max_len) - 1:
+        raise ValueError(f"max_len {max_len} exceeds CFG.max_len-1 = {int(CFG.max_len) - 1} (model.py:93, Q6)")
+    if not x.is_cuda:
+        raise ValueError("generate_beam() takes the images on a CUDA device; there is no CPU fallback")
+    eos = _stop_token(tokenizer)
+    tokens, _, _, confs = model.generate_beam_tokens(x, max_len, num_beams, length_penalty, eos_token=eos)
+    host = torch.empty(tokens[:, 0].shape, dtype=torch.int32, pin_memory=True)
+    host_c = torch.empty(confs[:, 0].shape, dtype=torch.float32, pin_memory=True)
+    host.copy_(tokens[:, 0], non_blocking=True)
+    host_c.copy_(confs[:, 0], non_blocking=True)
+    torch.cuda.current_stream(tokens.device).synchronize()
+    n_conf = (max_len + 3) // 4
+    return host.long(), [host_c[:, i].clone() for i in range(n_conf)]
+
+
 def _stop_token(tokenizer):
     """The stop token of `stop_at_eos`; finished rows are filled with CFG.pad_idx, so the tokenizer's PAD must be that token."""
     if int(getattr(tokenizer, "PAD_code", CFG.pad_idx)) != int(CFG.pad_idx):

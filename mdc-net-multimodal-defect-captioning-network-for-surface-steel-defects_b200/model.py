@@ -565,6 +565,36 @@ class EncoderDecoder(nn.Module, _EngineOwner):
             return tokens.clone(), confs.clone(), logits.clone()
         return tokens.clone(), confs.clone()
 
+    @torch.no_grad()
+    def generate_beam_tokens(self, image, max_new_tokens, num_beams, length_penalty=1.0, *, eos_token, use_graph=None):
+        """Beam search (superset method; semantics in include/mdc_b200.h and DESIGN.md §3.4c).  Returns, on the device, each image's
+        beams best first by length-normalised score: tokens int32 (B,K,1+T), normalised scores f32 (B,K), per-token log-probs f32
+        (B,K,T) and confidences f32 (B,K,ceil(T/4)).  Tokens after a beam's EOS are PAD, with log-prob and confidence 0.  The whole
+        call (encoder, cross-K/V for the B*K rows, T x (one teacher-forced decode step + one beam step), the final ordering) is one
+        CUDA graph replay per (B, T, K, length penalty, stop token) shape."""
+        eng = self._engine(image.device if image.is_cuda else None)
+        d = eng.dims
+        T, K = int(max_new_tokens), int(num_beams)
+        if not 1 <= K <= 16:
+            raise ValueError(f"num_beams {K} is outside 1..16")
+        if not 1 <= T <= d.max_pos:
+            raise RuntimeError(f"max_len {T} is outside 1..CFG.max_len-1 = {d.max_pos}: the positional table has no more rows "
+                               "(reference fails at model.py:93, Q6)")
+        eos_token = int(eos_token)
+        if not 0 <= eos_token < d.vocab:
+            raise ValueError(f"eos_token {eos_token} is outside the vocabulary [0, {d.vocab})")
+        if use_graph is None:
+            use_graph = os.environ.get("MDC_NO_GRAPH", "0") != "1"
+        key = ("beam", id(eng), image.shape[0], T, K, float(length_penalty), eos_token, bool(use_graph), _decode_options_key())
+        plans = self.__dict__.setdefault("_plans", {})
+        if plans.get("eng") is not eng:
+            plans.clear(); plans["eng"] = eng
+        plan = plans.get(key)
+        if plan is None:
+            plan = BeamPlan(eng, image.shape[0], T, K, float(length_penalty), eos_token, use_graph)
+            plans[key] = plan
+        return tuple(o.clone() for o in plan.run(image))
+
 
 class GenerationPlan:
     """Static buffers + (optionally) a captured CUDA graph for one (batch, new tokens, sampler) shape:
@@ -667,3 +697,103 @@ class GenerationPlan:
             else:
                 self._launch()
         return self.tokens, self.confs, self.logits
+
+
+class BeamPlan:
+    """Static buffers + (optionally) a captured CUDA graph for one beam-search shape (B images, T new tokens, K beams): encoder ->
+    memory repeated K times -> cross-K/V of the B*K rows -> T x (teacher-forced decode step t, mdc_beam_step t) -> mdc_beam_finalize.
+    The KV pool holds B*K rows of distinct pages (`own`, never rewritten); `kv.page_table` is the live table the decode kernels read,
+    reset to `own` at the start of every run."""
+
+    def __init__(self, eng, B, T, K, length_penalty, eos_token, use_graph):
+        with torch.cuda.device(eng.device):
+            self._build(eng, B, T, K, length_penalty, eos_token, use_graph)
+
+    def _build(self, eng, B, T, K, length_penalty, eos_token, use_graph):
+        d = eng.dims
+        dev = eng.device
+        BK = B * K
+        self.eng, self.B, self.T, self.K = eng, B, T, K
+        self.length_penalty, self.eos_token = float(length_penalty), int(eos_token)
+        self.x = torch.zeros((B, d.in_chans, d.img_size, d.img_size), dtype=torch.float32, device=dev)
+        self.ws_bytes = eng.lib.mdc_encode_workspace_bytes(eng.handle, B)
+        self.ws = torch.empty(self.ws_bytes, dtype=torch.uint8, device=dev)
+        self.memory = torch.empty((B, d.n_patches, d.dim), dtype=eng.dtype, device=dev)
+        self.memory_k = torch.empty((B, K, d.n_patches, d.dim), dtype=eng.dtype, device=dev)
+        self.ckv = torch.empty(eng.lib.mdc_cross_kv_bytes(eng.handle, BK), dtype=torch.uint8, device=dev)
+        self.tokens = torch.empty((BK, T + 1), dtype=torch.int32, device=dev)
+        self.logits = torch.empty((BK, T, d.vocab), dtype=torch.float32, device=dev)
+        self.kv = PagedKVCache(BK, T, d.dec_layers, d.dim, d.page_tokens, eng.dtype, dev)
+        self.own = self.kv.page_table.clone()
+        self.scratch = torch.empty(eng.lib.mdc_decode_workspace_bytes(eng.handle, BK), dtype=torch.uint8, device=dev)
+        self.scores = torch.empty(BK, dtype=torch.float32, device=dev)
+        self.score0 = torch.full((B, K), -float("inf"), dtype=torch.float32, device=dev)
+        self.score0[:, 0] = 0.0
+        self.finish = torch.empty(BK, dtype=torch.int32, device=dev)
+        self.lps = torch.zeros((BK, T), dtype=torch.float32, device=dev)
+        self.confs = torch.zeros((BK, (T + 3) // 4), dtype=torch.float32, device=dev)
+        self.beam_ws = torch.empty(eng.lib.mdc_beam_workspace_bytes(eng.handle, B, K), dtype=torch.uint8, device=dev)
+        self.order = torch.empty((B, K), dtype=torch.int32, device=dev)
+        self.norm = torch.empty((B, K), dtype=torch.float32, device=dev)
+        self.rows = torch.arange(B, device=dev, dtype=torch.int64)[:, None] * K
+        st = L.BeamState()
+        st.B, st.K = B, K
+        st.tokens, st.tokens_ld = self.tokens.data_ptr(), self.tokens.shape[1]
+        st.kv_pool, st.page_table, st.own_pages = self.kv.pool.data_ptr(), self.kv.page_table.data_ptr(), self.own.data_ptr()
+        st.pages_per_seq = self.kv.pages_per_seq
+        st.scores, st.finish_step = self.scores.data_ptr(), self.finish.data_ptr()
+        st.token_logprobs, st.token_logprobs_ld = self.lps.data_ptr(), T
+        st.confs, st.confs_ld = self.confs.data_ptr(), self.confs.shape[1]
+        st.eos_token = self.eos_token
+        st.workspace, st.workspace_bytes = self.beam_ws.data_ptr(), self.beam_ws.numel()
+        self.state = st
+        self.graph = None
+        if use_graph:
+            side = torch.cuda.Stream(device=dev)
+            side.wait_stream(torch.cuda.current_stream(dev))
+            with torch.cuda.stream(side):
+                self._launch()                      # warm-up: tensor maps, smem attributes, lazy module load
+            torch.cuda.current_stream(dev).wait_stream(side)
+            torch.cuda.synchronize(dev)
+            g = torch.cuda.CUDAGraph()
+            n0 = L.launch_count(dev)
+            with torch.cuda.graph(g, stream=side):
+                self._launch()
+            self.graph_kernels = L.launch_count(dev) - n0
+            self.graph = g
+
+    def _launch(self):
+        eng, B, K, T = self.eng, self.B, self.K, self.T
+        d = eng.dims
+        s = L.stream_ptr(eng.device)
+        with torch.cuda.device(eng.device):
+            L.check(eng.lib.mdc_encode(eng.handle, L.ptr(self.x), B, None, L.ptr(self.memory), L.ptr(self.ws), self.ws_bytes, s))
+            self.memory_k.copy_(self.memory[:, None].expand_as(self.memory_k))
+            L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory_k), B * K, L.ptr(self.ckv), s))
+            self.tokens.fill_(int(CFG.pad_idx))
+            self.tokens[:, 0].fill_(int(CFG.bos_idx))
+            self.kv.page_table.copy_(self.own)
+            self.scores.copy_(self.score0.view(-1))
+            self.finish.fill_(-1)
+            row_bytes = d.vocab * self.logits.element_size()
+            for t in range(T):
+                eng.decode(self.ckv, self.tokens, t, t + 1, max_tokens=T, forced=True, logits=self.logits, logits_row_offset=0,
+                           kv=self.kv, scratch=self.scratch)
+                L.check(eng.lib.mdc_beam_step(eng.handle, C.byref(self.state), C.c_void_p(self.logits.data_ptr() + t * row_bytes),
+                                              T * d.vocab, t, s))
+            L.check(eng.lib.mdc_beam_finalize(eng.handle, C.byref(self.state), T, self.length_penalty, L.ptr(self.order),
+                                              L.ptr(self.norm), s))
+
+    def run(self, image):
+        if tuple(image.shape) != tuple(self.x.shape):
+            raise AssertionError("Input size doesn't match model")
+        with torch.cuda.device(self.eng.device):
+            self.x.copy_(image, non_blocking=True)
+            if self.graph is not None:
+                self.graph.replay()
+                L.note_graph_replay(self.eng.device, self.graph_kernels)
+            else:
+                self._launch()
+            rows = (self.rows + self.order.long()).view(-1)          # best-first gather of each image's rows
+            B, K = self.B, self.K
+            return (self.tokens[rows].view(B, K, -1), self.norm, self.lps[rows].view(B, K, -1), self.confs[rows].view(B, K, -1))
