@@ -12,6 +12,7 @@ from __future__ import annotations
 import torch
 
 from .config import CFG
+from .model import check_max_len
 
 
 @torch.no_grad()
@@ -24,20 +25,14 @@ def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None, s
     `stop_at_eos` (superset argument): stop at tokenizer.EOS_code.  Everything up to and including each
     image's first EOS is bitwise the default result; after it the tokens are PAD and the confidences 0,
     and decoding ends once every image has finished -- postprocess() returns the same either way."""
-    bos = int(getattr(tokenizer, "BOS_code", CFG.bos_idx))
-    if bos != int(CFG.bos_idx):
-        raise ValueError("tokenizer.BOS_code must equal CFG.bos_idx (model.py:117 reads the global)")
+    _check_bos(tokenizer)
     if not hasattr(model, "generate_tokens"):
         raise TypeError("generate() needs the B200 EncoderDecoder; there is no PyTorch fallback path")
     eos = _stop_token(tokenizer) if stop_at_eos else None
     tokens, confs = model.generate_tokens(x, max_len, top_k=top_k, top_p=top_p, uniforms=uniforms, eos_token=eos)
-    host = torch.empty(tokens.shape, dtype=torch.int32, pin_memory=True)
-    host_c = torch.empty(confs.shape, dtype=torch.float32, pin_memory=True)
-    host.copy_(tokens, non_blocking=True)
-    host_c.copy_(confs, non_blocking=True)
+    host = _to_pinned(tokens, confs)
     torch.cuda.current_stream(tokens.device).synchronize()      # the ONE sync of the whole call
-    n_conf = (max_len + 3) // 4
-    return host.long(), [host_c[:, i].clone() for i in range(n_conf)]
+    return _host_result(*host)
 
 
 @torch.no_grad()
@@ -46,26 +41,37 @@ def generate_beam(model, x, tokenizer, max_len=50, num_beams=4, length_penalty=1
     ceil(max_len/4) (B,) confidence tensors, on CPU -- for each image's best beam by score / len^length_penalty, so that postprocess()
     and postprocess_with_captions() read it unchanged.  Beams end at tokenizer.EOS_code (the tokens after it are PAD, the confidences 0);
     there is no early exit once every beam has ended, and no sampling inside beams.  Semantics: DESIGN.md §3.4c."""
-    bos = int(getattr(tokenizer, "BOS_code", CFG.bos_idx))
-    if bos != int(CFG.bos_idx):
-        raise ValueError("tokenizer.BOS_code must equal CFG.bos_idx (model.py:117 reads the global)")
+    _check_bos(tokenizer)
     if not hasattr(model, "generate_beam_tokens"):
         raise TypeError("generate_beam() needs the B200 EncoderDecoder; there is no PyTorch fallback path")
-    if not 1 <= int(num_beams) <= 16:
-        raise ValueError(f"num_beams {num_beams} is outside 1..16")
-    if int(max_len) > int(CFG.max_len) - 1:
-        raise ValueError(f"max_len {max_len} exceeds CFG.max_len-1 = {int(CFG.max_len) - 1} (model.py:93, Q6)")
+    check_max_len(int(max_len), int(CFG.max_len) - 1, ValueError)      # generate_beam_tokens raises RuntimeError
     if not x.is_cuda:
         raise ValueError("generate_beam() takes the images on a CUDA device; there is no CPU fallback")
     eos = _stop_token(tokenizer)
     tokens, _, _, confs = model.generate_beam_tokens(x, max_len, num_beams, length_penalty, eos_token=eos)
-    host = torch.empty(tokens[:, 0].shape, dtype=torch.int32, pin_memory=True)
-    host_c = torch.empty(confs[:, 0].shape, dtype=torch.float32, pin_memory=True)
-    host.copy_(tokens[:, 0], non_blocking=True)
-    host_c.copy_(confs[:, 0], non_blocking=True)
+    host = _to_pinned(tokens[:, 0], confs[:, 0])
     torch.cuda.current_stream(tokens.device).synchronize()
-    n_conf = (max_len + 3) // 4
-    return host.long(), [host_c[:, i].clone() for i in range(n_conf)]
+    return _host_result(*host)
+
+
+def _to_pinned(tokens, confs):
+    """Pinned host copies of a call's device tokens and confidences, enqueued on the current stream: valid once the call has
+    synchronised."""
+    host = torch.empty(tokens.shape, dtype=torch.int32, pin_memory=True)
+    host_c = torch.empty(confs.shape, dtype=torch.float32, pin_memory=True)
+    host.copy_(tokens, non_blocking=True)
+    host_c.copy_(confs, non_blocking=True)
+    return host, host_c
+
+
+def _host_result(host, host_c):
+    """generate()'s result from the host copies: LongTensor (B, 1+max_len) and the list of the ceil(max_len/4) (B,) confidence columns."""
+    return host.long(), [host_c[:, i].clone() for i in range(host_c.shape[1])]
+
+
+def _check_bos(tokenizer):
+    if int(getattr(tokenizer, "BOS_code", CFG.bos_idx)) != int(CFG.bos_idx):
+        raise ValueError("tokenizer.BOS_code must equal CFG.bos_idx (model.py:117 reads the global)")
 
 
 def _stop_token(tokenizer):

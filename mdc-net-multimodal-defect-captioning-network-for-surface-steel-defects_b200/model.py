@@ -527,6 +527,19 @@ class EncoderDecoder(nn.Module, _EngineOwner):
         return self.decoder._predict_with(eng, memory, tgt)
 
     # -- the fast path used by generate(): encode once, cross-K/V once, incremental decode ---------
+    def _plan(self, eng, key, use_graph, make):
+        """The cached plan of one call shape; `make(use_graph)` builds it on first use.  Every plan is dropped when the engine changes
+        (new weights, precision or device).  `use_graph` None: capture CUDA graphs unless MDC_NO_GRAPH=1."""
+        if use_graph is None:
+            use_graph = os.environ.get("MDC_NO_GRAPH", "0") != "1"
+        key = (*key, bool(use_graph), _decode_options_key())
+        plans = self.__dict__.setdefault("_plans", {})
+        if plans.get("eng") is not eng:
+            plans.clear(); plans["eng"] = eng
+        if key not in plans:
+            plans[key] = make(use_graph)
+        return plans[key]
+
     @torch.no_grad()
     def generate_tokens(self, image, max_new_tokens, top_k=0, top_p=1.0, uniforms=None, return_logits=False, use_graph=None,
                         eos_token=None):
@@ -536,30 +549,16 @@ class EncoderDecoder(nn.Module, _EngineOwner):
         no-stop result; after it the tokens are PAD and the confidences 0, and decoding ends once every image has finished.  Not
         with `return_logits` (steps that do not run have no logits; predict()/forward() serve that use)."""
         eng = self._engine(image.device if image.is_cuda else None)
-        d = eng.dims
-        T = int(max_new_tokens)
-        if T > d.max_pos:
-            raise RuntimeError(f"max_len {T} exceeds CFG.max_len-1 = {d.max_pos}: the positional table has no more rows "
-                               "(reference fails at model.py:93, Q6)")
-        sampling = (top_k != 0 or top_p != 1)
+        B, T = image.shape[0], int(max_new_tokens)
+        check_max_len(T, eng.dims.max_pos)
         if eos_token is not None:
             if return_logits:
                 raise ValueError("return_logits=True cannot be combined with eos_token: steps that do not run have no logits")
-            eos_token = int(eos_token)
-            if not 0 <= eos_token < d.vocab:
-                raise ValueError(f"eos_token {eos_token} is outside the vocabulary [0, {d.vocab})")
-        if use_graph is None:
-            use_graph = os.environ.get("MDC_NO_GRAPH", "0") != "1"
-        key = (id(eng), image.shape[0], T, int(top_k), float(top_p), bool(return_logits), bool(use_graph), eos_token, _decode_options_key())
-        plans = self.__dict__.setdefault("_plans", {})
-        if plans.get("eng") is not eng:
-            plans.clear(); plans["eng"] = eng
-        plan = plans.get(key)
-        if plan is None:
-            plan = GenerationPlan(eng, image.shape[0], T, top_k, top_p, sampling, return_logits, use_graph, eos_token=eos_token)
-            plans[key] = plan
-        if sampling and uniforms is None:
-            uniforms = torch.rand((image.shape[0], T), dtype=torch.float32, device=eng.device)
+            eos_token = check_eos_token(eos_token, eng.dims.vocab)
+        plan = self._plan(eng, (id(eng), B, T, int(top_k), float(top_p), bool(return_logits), eos_token), use_graph,
+                          lambda graph: GenerationPlan(eng, B, T, top_k, top_p, return_logits, graph, eos_token=eos_token))
+        if plan.uniforms is not None and uniforms is None:
+            uniforms = torch.rand((B, T), dtype=torch.float32, device=eng.device)
         tokens, confs, logits = plan.run(image, uniforms)
         if return_logits:
             return tokens.clone(), confs.clone(), logits.clone()
@@ -573,96 +572,128 @@ class EncoderDecoder(nn.Module, _EngineOwner):
         call (encoder, cross-K/V for the B*K rows, T x (one teacher-forced decode step + one beam step), the final ordering) is one
         CUDA graph replay per (B, T, K, length penalty, stop token) shape."""
         eng = self._engine(image.device if image.is_cuda else None)
-        d = eng.dims
-        T, K = int(max_new_tokens), int(num_beams)
+        B, T, K = image.shape[0], int(max_new_tokens), int(num_beams)
         if not 1 <= K <= 16:
             raise ValueError(f"num_beams {K} is outside 1..16")
-        if not 1 <= T <= d.max_pos:
-            raise RuntimeError(f"max_len {T} is outside 1..CFG.max_len-1 = {d.max_pos}: the positional table has no more rows "
-                               "(reference fails at model.py:93, Q6)")
-        eos_token = int(eos_token)
-        if not 0 <= eos_token < d.vocab:
-            raise ValueError(f"eos_token {eos_token} is outside the vocabulary [0, {d.vocab})")
-        if use_graph is None:
-            use_graph = os.environ.get("MDC_NO_GRAPH", "0") != "1"
-        key = ("beam", id(eng), image.shape[0], T, K, float(length_penalty), eos_token, bool(use_graph), _decode_options_key())
-        plans = self.__dict__.setdefault("_plans", {})
-        if plans.get("eng") is not eng:
-            plans.clear(); plans["eng"] = eng
-        plan = plans.get(key)
-        if plan is None:
-            plan = BeamPlan(eng, image.shape[0], T, K, float(length_penalty), eos_token, use_graph)
-            plans[key] = plan
+        if T < 1:
+            raise RuntimeError(f"max_len {T}: beam search needs at least one new token")
+        check_max_len(T, eng.dims.max_pos)
+        eos_token = check_eos_token(eos_token, eng.dims.vocab)
+        plan = self._plan(eng, ("beam", id(eng), B, T, K, float(length_penalty), eos_token), use_graph,
+                          lambda graph: BeamPlan(eng, B, T, K, length_penalty, eos_token, graph))
         return tuple(o.clone() for o in plan.run(image))
 
 
-class GenerationPlan:
-    """Static buffers + (optionally) a captured CUDA graph for one (batch, new tokens, sampler) shape:
-    encoder -> memory -> cross-K/V -> T decode steps, no host synchronisation anywhere inside."""
+def check_max_len(T, max_pos, error=RuntimeError):
+    """Generation reads one row of the decoder's positional table per new token, and the table has max_pos = CFG.max_len-1 rows."""
+    if T > max_pos:
+        raise error(f"max_len {T} exceeds CFG.max_len-1 = {max_pos}: the positional table has no more rows "
+                    "(reference fails at model.py:93, Q6)")
 
-    def __init__(self, eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split=False, images_per_cluster=None, ctas_per_sm=None,
-                 eos_token=None):
-        # everything below (allocations, warm-up launches, graph capture) on the ENGINE's device: torch.cuda.graph captures the current
-        # device's stream, so with another device current the capture came back empty and replays did nothing (two-device test)
-        with torch.cuda.device(eng.device):
-            self._build(eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split, images_per_cluster, ctas_per_sm, eos_token)
 
-    def _build(self, eng, B, T, top_k, top_p, sampling, want_logits, use_graph, split, images_per_cluster, ctas_per_sm, eos_token):
-        d = eng.dims
-        dev = eng.device
+def check_eos_token(eos_token, vocab):
+    eos_token = int(eos_token)
+    if not 0 <= eos_token < vocab:
+        raise ValueError(f"eos_token {eos_token} is outside the vocabulary [0, {vocab})")
+    return eos_token
+
+
+def capture_graphs(device, *launches):
+    """Captures each of `launches` (functions that enqueue work on the current stream) into its own CUDA graph and returns, in the same
+    order, (graph, kernels of libmdc_b200.so in one replay) pairs for replay().  All of them run once first as a warm-up (tensor maps,
+    shared-memory attributes, lazy module load), then the device is synchronised.  Warm-up and capture run under `device`, on one side
+    stream of it given explicitly: torch's default capture stream is a process-wide singleton on whichever device captured first, and a
+    graph of another device captured there replays nothing."""
+    with torch.cuda.device(device):
+        side = torch.cuda.Stream(device=device)
+        side.wait_stream(torch.cuda.current_stream(device))
+        with torch.cuda.stream(side):
+            for launch in launches:
+                launch()
+        torch.cuda.current_stream(device).wait_stream(side)
+        torch.cuda.synchronize(device)
+        graphs = []
+        for launch in launches:
+            graph, n0 = torch.cuda.CUDAGraph(), L.launch_count(device)
+            with torch.cuda.graph(graph, stream=side):
+                launch()
+            graphs.append((graph, L.launch_count(device) - n0))
+        return graphs
+
+
+def replay(device, captured):
+    """Replays one (graph, kernel count) pair of capture_graphs() on the current stream and counts its kernels in L.launch_count."""
+    graph, n_kernels = captured
+    graph.replay()
+    L.note_graph_replay(device, n_kernels)
+
+
+class _Plan:
+    """Static buffers of one generation call shape on the engine's device: the B input images `x`, the encoder workspace and `memory`,
+    and for the `rows` decoded sequences (B, or B*K beams) the cross-K/V, tokens, confidences, KV cache and decode scratch.  A plan
+    launches its whole call in `_launch` (no host synchronisation inside) and returns `_outputs()`; `run` replays `graph` instead
+    where the plan captured one.  `uniforms`: the sampler's variates, for plans that sample."""
+
+    graph = uniforms = None
+
+    def __init__(self, eng, B, T, rows):
+        d, dev = eng.dims, eng.device
         self.eng, self.B, self.T = eng, B, T
-        self.top_k, self.top_p = int(top_k), float(top_p)
-        self.eos_token = eos_token
-        self.images_per_cluster = _DECODE_OPTIONS["images_per_cluster"] if images_per_cluster is None else int(images_per_cluster)
-        self.ctas_per_sm = _DECODE_OPTIONS["ctas_per_sm"] if ctas_per_sm is None else int(ctas_per_sm)
-        self.per_op_kernels = bool(_DECODE_OPTIONS["per_op_kernels"])
         self.x = torch.zeros((B, d.in_chans, d.img_size, d.img_size), dtype=torch.float32, device=dev)
         self.ws_bytes = eng.lib.mdc_encode_workspace_bytes(eng.handle, B)
         self.ws = torch.empty(self.ws_bytes, dtype=torch.uint8, device=dev)
         self.memory = torch.empty((B, d.n_patches, d.dim), dtype=eng.dtype, device=dev)
-        self.ckv = torch.empty(eng.lib.mdc_cross_kv_bytes(eng.handle, B), dtype=torch.uint8, device=dev)
-        self.tokens = torch.empty((B, T + 1), dtype=torch.int32, device=dev)
-        self.confs = torch.zeros((B, (T + 3) // 4), dtype=torch.float32, device=dev)
-        self.logits = torch.empty((B, T, d.vocab), dtype=torch.float32, device=dev) if want_logits else None
-        self.uniforms = torch.zeros((B, T), dtype=torch.float32, device=dev) if sampling else None
-        self.kv = PagedKVCache(B, T, d.dec_layers, d.dim, d.page_tokens, eng.dtype, dev)
-        self.scratch = torch.empty(eng.lib.mdc_decode_workspace_bytes(eng.handle, B), dtype=torch.uint8, device=dev)
-        self.graph = None
-        self.split = bool(split)
-        if split:
-            # two graphs (encoder + cross-K/V | decode loop) so that a GenerationPipeline can run them on different streams
-            assert use_graph, "split plans are graph plans"
-            side = torch.cuda.Stream(device=dev)
-            side.wait_stream(torch.cuda.current_stream(dev))
-            with torch.cuda.stream(side):
-                self._launch_encode(); self._launch_decode()
-            torch.cuda.current_stream(dev).wait_stream(side)
-            torch.cuda.synchronize(dev)
-            self.enc_graph, self.dec_graph = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-            n0 = L.launch_count(dev)
-            with torch.cuda.graph(self.enc_graph, stream=side):     # an explicit capture stream of THIS device (torch's default one is a
-                                                                    # process-wide singleton on whichever device captured first)
-                self._launch_encode()
-            n1 = L.launch_count(dev)
-            with torch.cuda.graph(self.dec_graph, stream=side):
-                self._launch_decode()
-            self.enc_kernels, self.dec_kernels = n1 - n0, L.launch_count(dev) - n1
-            self.enc_done, self.dec_done = torch.cuda.Event(), torch.cuda.Event()
-            self.busy = False
-            return
-        if use_graph:
-            side = torch.cuda.Stream(device=dev)
-            side.wait_stream(torch.cuda.current_stream(dev))
-            with torch.cuda.stream(side):
-                self._launch()                      # warm-up: tensor maps, smem attributes, lazy module load
-            torch.cuda.current_stream(dev).wait_stream(side)
-            torch.cuda.synchronize(dev)
-            g = torch.cuda.CUDAGraph()
-            n0 = L.launch_count(dev)
-            with torch.cuda.graph(g, stream=side):
+        self.ckv = torch.empty(eng.lib.mdc_cross_kv_bytes(eng.handle, rows), dtype=torch.uint8, device=dev)
+        self.tokens = torch.empty((rows, T + 1), dtype=torch.int32, device=dev)
+        self.confs = torch.zeros((rows, (T + 3) // 4), dtype=torch.float32, device=dev)
+        self.kv = PagedKVCache(rows, T, d.dec_layers, d.dim, d.page_tokens, eng.dtype, dev)
+        self.scratch = torch.empty(eng.lib.mdc_decode_workspace_bytes(eng.handle, rows), dtype=torch.uint8, device=dev)
+
+    def check_input(self, image):
+        if tuple(image.shape) != tuple(self.x.shape):
+            raise AssertionError("Input size doesn't match model")
+
+    def run(self, image, uniforms=None):
+        self.check_input(image)
+        with torch.cuda.device(self.eng.device):
+            self.x.copy_(image, non_blocking=True)               # H2D from (pinned) host memory or D2D
+            if self.uniforms is not None:
+                self.uniforms.copy_(uniforms.to(torch.float32), non_blocking=True)
+            if self.graph is None:
                 self._launch()
-            self.graph_kernels = L.launch_count(dev) - n0      # kernels of libmdc_b200.so inside one replay
-            self.graph = g
+            else:
+                replay(self.eng.device, self.graph)
+            return self._outputs()
+
+    def _encode(self):
+        eng = self.eng
+        L.check(eng.lib.mdc_encode(eng.handle, L.ptr(self.x), self.B, None, L.ptr(self.memory), L.ptr(self.ws), self.ws_bytes,
+                                   L.stream_ptr(eng.device)))
+
+    def _reset_tokens(self):
+        self.tokens.fill_(int(CFG.pad_idx))
+        self.tokens[:, 0].fill_(int(CFG.bos_idx))
+
+
+class GenerationPlan(_Plan):
+    """One (batch, new tokens, sampler, stop token) shape: encoder -> memory -> cross-K/V -> T decode steps.  With `use_graph` the
+    whole call is one CUDA graph; with `split` it is two (encoder + cross-K/V | decode loop), `enc_graph` and `dec_graph`, so that a
+    GenerationPipeline can run them on different streams.  `images_per_cluster` / `ctas_per_sm` override the decode launch options;
+    the others come from decode_options."""
+
+    def __init__(self, eng, B, T, top_k=0, top_p=1.0, want_logits=False, use_graph=True, split=False, eos_token=None,
+                 images_per_cluster=None, ctas_per_sm=None):
+        super().__init__(eng, B, T, B)
+        d, dev = eng.dims, eng.device
+        self.top_k, self.top_p, self.eos_token = int(top_k), float(top_p), eos_token
+        self.images_per_cluster, self.ctas_per_sm = images_per_cluster, ctas_per_sm
+        self.logits = torch.empty((B, T, d.vocab), dtype=torch.float32, device=dev) if want_logits else None
+        if top_k != 0 or top_p != 1:
+            self.uniforms = torch.zeros((B, T), dtype=torch.float32, device=dev)
+        if split:
+            self.enc_graph, self.dec_graph = capture_graphs(dev, self._launch_encode, self._launch_decode)
+        elif use_graph:
+            [self.graph] = capture_graphs(dev, self._launch)
 
     def _launch(self):
         self._launch_encode()
@@ -670,68 +701,37 @@ class GenerationPlan:
 
     def _launch_encode(self):
         eng = self.eng
-        with torch.cuda.device(eng.device):
-            L.check(eng.lib.mdc_encode(eng.handle, L.ptr(self.x), self.B, None, L.ptr(self.memory), L.ptr(self.ws), self.ws_bytes, L.stream_ptr(eng.device)))
-            L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory), self.B, L.ptr(self.ckv), L.stream_ptr(eng.device)))
+        self._encode()
+        L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory), self.B, L.ptr(self.ckv), L.stream_ptr(eng.device)))
 
     def _launch_decode(self):
-        eng = self.eng
-        self.tokens.fill_(int(CFG.pad_idx))
-        self.tokens[:, 0].fill_(int(CFG.bos_idx))
-        eng.decode(self.ckv, self.tokens, 0, self.T, max_tokens=self.T, forced=False, logits=self.logits, logits_row_offset=0,
-                   confs=self.confs, uniforms=self.uniforms, top_k=self.top_k, top_p=self.top_p, kv=self.kv, scratch=self.scratch,
-                   images_per_cluster=self.images_per_cluster, ctas_per_sm=self.ctas_per_sm, per_op_kernels=self.per_op_kernels,
-                   eos_token=self.eos_token)
+        self._reset_tokens()
+        self.eng.decode(self.ckv, self.tokens, 0, self.T, max_tokens=self.T, forced=False, logits=self.logits, logits_row_offset=0,
+                        confs=self.confs, uniforms=self.uniforms, top_k=self.top_k, top_p=self.top_p, kv=self.kv, scratch=self.scratch,
+                        images_per_cluster=self.images_per_cluster, ctas_per_sm=self.ctas_per_sm, eos_token=self.eos_token)
 
-    def run(self, image, uniforms=None):
-        d = self.eng.dims
-        if tuple(image.shape) != tuple(self.x.shape):
-            raise AssertionError("Input size doesn't match model")
-        with torch.cuda.device(self.eng.device):
-            self.x.copy_(image, non_blocking=True)               # H2D from (pinned) host memory or D2D
-            if self.uniforms is not None:
-                self.uniforms.copy_(uniforms.to(torch.float32), non_blocking=True)
-            if self.graph is not None:
-                self.graph.replay()
-                L.note_graph_replay(self.eng.device, self.graph_kernels)
-            else:
-                self._launch()
+    def _outputs(self):
         return self.tokens, self.confs, self.logits
 
 
-class BeamPlan:
-    """Static buffers + (optionally) a captured CUDA graph for one beam-search shape (B images, T new tokens, K beams): encoder ->
-    memory repeated K times -> cross-K/V of the B*K rows -> T x (teacher-forced decode step t, mdc_beam_step t) -> mdc_beam_finalize.
+class BeamPlan(_Plan):
+    """One beam-search shape (B images, T new tokens, K beams): encoder -> memory repeated K times -> cross-K/V of the B*K rows ->
+    T x (teacher-forced decode step t, mdc_beam_step t) -> mdc_beam_finalize, captured as one CUDA graph with `use_graph`.
     The KV pool holds B*K rows of distinct pages (`own`, never rewritten); `kv.page_table` is the live table the decode kernels read,
     reset to `own` at the start of every run."""
 
     def __init__(self, eng, B, T, K, length_penalty, eos_token, use_graph):
-        with torch.cuda.device(eng.device):
-            self._build(eng, B, T, K, length_penalty, eos_token, use_graph)
-
-    def _build(self, eng, B, T, K, length_penalty, eos_token, use_graph):
-        d = eng.dims
-        dev = eng.device
-        BK = B * K
-        self.eng, self.B, self.T, self.K = eng, B, T, K
-        self.length_penalty, self.eos_token = float(length_penalty), int(eos_token)
-        self.x = torch.zeros((B, d.in_chans, d.img_size, d.img_size), dtype=torch.float32, device=dev)
-        self.ws_bytes = eng.lib.mdc_encode_workspace_bytes(eng.handle, B)
-        self.ws = torch.empty(self.ws_bytes, dtype=torch.uint8, device=dev)
-        self.memory = torch.empty((B, d.n_patches, d.dim), dtype=eng.dtype, device=dev)
+        super().__init__(eng, B, T, B * K)
+        d, dev, BK = eng.dims, eng.device, B * K
+        self.K, self.length_penalty, self.eos_token = K, float(length_penalty), int(eos_token)
         self.memory_k = torch.empty((B, K, d.n_patches, d.dim), dtype=eng.dtype, device=dev)
-        self.ckv = torch.empty(eng.lib.mdc_cross_kv_bytes(eng.handle, BK), dtype=torch.uint8, device=dev)
-        self.tokens = torch.empty((BK, T + 1), dtype=torch.int32, device=dev)
         self.logits = torch.empty((BK, T, d.vocab), dtype=torch.float32, device=dev)
-        self.kv = PagedKVCache(BK, T, d.dec_layers, d.dim, d.page_tokens, eng.dtype, dev)
         self.own = self.kv.page_table.clone()
-        self.scratch = torch.empty(eng.lib.mdc_decode_workspace_bytes(eng.handle, BK), dtype=torch.uint8, device=dev)
         self.scores = torch.empty(BK, dtype=torch.float32, device=dev)
         self.score0 = torch.full((B, K), -float("inf"), dtype=torch.float32, device=dev)
         self.score0[:, 0] = 0.0
         self.finish = torch.empty(BK, dtype=torch.int32, device=dev)
         self.lps = torch.zeros((BK, T), dtype=torch.float32, device=dev)
-        self.confs = torch.zeros((BK, (T + 3) // 4), dtype=torch.float32, device=dev)
         self.beam_ws = torch.empty(eng.lib.mdc_beam_workspace_bytes(eng.handle, B, K), dtype=torch.uint8, device=dev)
         self.order = torch.empty((B, K), dtype=torch.int32, device=dev)
         self.norm = torch.empty((B, K), dtype=torch.float32, device=dev)
@@ -747,53 +747,30 @@ class BeamPlan:
         st.eos_token = self.eos_token
         st.workspace, st.workspace_bytes = self.beam_ws.data_ptr(), self.beam_ws.numel()
         self.state = st
-        self.graph = None
         if use_graph:
-            side = torch.cuda.Stream(device=dev)
-            side.wait_stream(torch.cuda.current_stream(dev))
-            with torch.cuda.stream(side):
-                self._launch()                      # warm-up: tensor maps, smem attributes, lazy module load
-            torch.cuda.current_stream(dev).wait_stream(side)
-            torch.cuda.synchronize(dev)
-            g = torch.cuda.CUDAGraph()
-            n0 = L.launch_count(dev)
-            with torch.cuda.graph(g, stream=side):
-                self._launch()
-            self.graph_kernels = L.launch_count(dev) - n0
-            self.graph = g
+            [self.graph] = capture_graphs(dev, self._launch)
 
     def _launch(self):
         eng, B, K, T = self.eng, self.B, self.K, self.T
         d = eng.dims
         s = L.stream_ptr(eng.device)
-        with torch.cuda.device(eng.device):
-            L.check(eng.lib.mdc_encode(eng.handle, L.ptr(self.x), B, None, L.ptr(self.memory), L.ptr(self.ws), self.ws_bytes, s))
-            self.memory_k.copy_(self.memory[:, None].expand_as(self.memory_k))
-            L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory_k), B * K, L.ptr(self.ckv), s))
-            self.tokens.fill_(int(CFG.pad_idx))
-            self.tokens[:, 0].fill_(int(CFG.bos_idx))
-            self.kv.page_table.copy_(self.own)
-            self.scores.copy_(self.score0.view(-1))
-            self.finish.fill_(-1)
-            row_bytes = d.vocab * self.logits.element_size()
-            for t in range(T):
-                eng.decode(self.ckv, self.tokens, t, t + 1, max_tokens=T, forced=True, logits=self.logits, logits_row_offset=0,
-                           kv=self.kv, scratch=self.scratch)
-                L.check(eng.lib.mdc_beam_step(eng.handle, C.byref(self.state), C.c_void_p(self.logits.data_ptr() + t * row_bytes),
-                                              T * d.vocab, t, s))
-            L.check(eng.lib.mdc_beam_finalize(eng.handle, C.byref(self.state), T, self.length_penalty, L.ptr(self.order),
-                                              L.ptr(self.norm), s))
+        self._encode()
+        self.memory_k.copy_(self.memory[:, None].expand_as(self.memory_k))
+        L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory_k), B * K, L.ptr(self.ckv), s))
+        self._reset_tokens()
+        self.kv.page_table.copy_(self.own)
+        self.scores.copy_(self.score0.view(-1))
+        self.finish.fill_(-1)
+        row_bytes = d.vocab * self.logits.element_size()
+        for t in range(T):
+            eng.decode(self.ckv, self.tokens, t, t + 1, max_tokens=T, forced=True, logits=self.logits, logits_row_offset=0,
+                       kv=self.kv, scratch=self.scratch)
+            L.check(eng.lib.mdc_beam_step(eng.handle, C.byref(self.state), C.c_void_p(self.logits.data_ptr() + t * row_bytes),
+                                          T * d.vocab, t, s))
+        L.check(eng.lib.mdc_beam_finalize(eng.handle, C.byref(self.state), T, self.length_penalty, L.ptr(self.order),
+                                          L.ptr(self.norm), s))
 
-    def run(self, image):
-        if tuple(image.shape) != tuple(self.x.shape):
-            raise AssertionError("Input size doesn't match model")
-        with torch.cuda.device(self.eng.device):
-            self.x.copy_(image, non_blocking=True)
-            if self.graph is not None:
-                self.graph.replay()
-                L.note_graph_replay(self.eng.device, self.graph_kernels)
-            else:
-                self._launch()
-            rows = (self.rows + self.order.long()).view(-1)          # best-first gather of each image's rows
-            B, K = self.B, self.K
-            return (self.tokens[rows].view(B, K, -1), self.norm, self.lps[rows].view(B, K, -1), self.confs[rows].view(B, K, -1))
+    def _outputs(self):
+        rows = (self.rows + self.order.long()).view(-1)          # best-first gather of each image's rows
+        B, K = self.B, self.K
+        return (self.tokens[rows].view(B, K, -1), self.norm, self.lps[rows].view(B, K, -1), self.confs[rows].view(B, K, -1))

@@ -17,8 +17,8 @@ from __future__ import annotations
 
 import torch
 
-from . import _lib as L
-from .config import CFG
+from .inference import _check_bos, _host_result, _stop_token, _to_pinned, preprocess_bgr, preprocess_gray
+from .model import GenerationPlan, check_max_len, replay
 
 
 class Ticket:
@@ -40,14 +40,11 @@ class GenerationPipeline:
     def __init__(self, model, batch, max_new_tokens, top_k=0, top_p=1.0, depth=None, decode_streams=None, images_per_cluster=16,
                  ctas_per_sm=0, to_host=False, device=None, eos_token=None):
         """`eos_token`: stop at that token, as EncoderDecoder.generate_tokens(..., eos_token=...) does."""
-        from .model import GenerationPlan
         if not hasattr(model, "_engine"):
             raise TypeError("GenerationPipeline needs the B200 EncoderDecoder; there is no PyTorch fallback path")
         eng = model._engine(device)
-        d = eng.dims
         T = int(max_new_tokens)
-        if T > d.max_pos:
-            raise RuntimeError(f"max_len {T} exceeds CFG.max_len-1 = {d.max_pos} (model.py:93, Q6)")
+        check_max_len(T, eng.dims.max_pos)
         # operating point: the fused decode kernel holds 32 SMs for ~12 ms per batch -> 4 decode streams, 6 plans; geometries it does not
         # cover (dim 1024 of trail_01.py:158-160) decode as a chain of ~100 few-microsecond kernels per token on at most 64-192 CTAs,
         # which leaves most of the GPU idle per batch -> 8 decode streams, 10 plans (tools/config_t_probe.py: 720 -> 1 900 img/s)
@@ -57,16 +54,16 @@ class GenerationPipeline:
         if depth is None:
             depth = 6 if fused else int(decode_streams) + 2
         self.eng, self.B, self.T, self.depth, self.to_host = eng, int(batch), T, int(depth), bool(to_host)
-        self.sampling = (top_k != 0 or top_p != 1)
         dev = eng.device
         with torch.cuda.device(dev):
-            self.plans = [GenerationPlan(eng, self.B, T, top_k, top_p, self.sampling, False, True, split=True,
-                                         images_per_cluster=images_per_cluster, ctas_per_sm=ctas_per_sm, eos_token=eos_token)
-                          for _ in range(self.depth)]
+            self.plans = [GenerationPlan(eng, self.B, T, top_k, top_p, split=True, eos_token=eos_token,
+                                         images_per_cluster=images_per_cluster, ctas_per_sm=ctas_per_sm) for _ in range(self.depth)]
             self.s_enc = torch.cuda.Stream(device=dev, priority=0)      # encoder / cross-K/V: fills whatever the decodes leave idle
             self.s_copy = torch.cuda.Stream(device=dev, priority=0)     # host->device copy (+ the u8 transform) of the NEXT batch: on the
             # encoder stream the 38.5 MB f32 copy of a batch (~0.8 ms on PCIe) sat between two encoder passes (e2e 4 % below the device-resident rate)
             self.copy_done = [torch.cuda.Event() for _ in range(self.depth)]
+            self.enc_done = [torch.cuda.Event() for _ in range(self.depth)]
+            self.dec_done = [torch.cuda.Event() for _ in range(self.depth)]
             self.s_decs = [torch.cuda.Stream(device=dev, priority=-1) for _ in range(max(1, int(decode_streams)))]   # clusters first
         self.n = 0
 
@@ -75,7 +72,8 @@ class GenerationPipeline:
         cv2.imread returns them, which the fused preprocessing kernel (inference.preprocess_gray / preprocess_bgr: the reference's
         cv2-resize + normalise transform, bit-exact in its uint8 part) turns into the plan's input buffer on the device.
         Returns a Ticket."""
-        p = self.plans[self.n % self.depth]
+        i = self.n % self.depth
+        p, busy = self.plans[i], self.n >= self.depth                   # busy: plan i has run before
         s_dec = self.s_decs[self.n % len(self.s_decs)]
         self.n += 1
         dev = self.eng.device
@@ -83,44 +81,35 @@ class GenerationPipeline:
         if gray:
             if image.dim() not in (3, 4) or image.shape[0] != self.B or (image.dim() == 4 and image.shape[-1] != 3):
                 raise AssertionError("raw input must be uint8 (B,h,w) gray or (B,h,w,3) BGR")
-        elif tuple(image.shape) != tuple(p.x.shape):
-            raise AssertionError("Input size doesn't match model")
+        else:
+            p.check_input(image)
         cur = torch.cuda.current_stream(dev)
-        cdone = self.copy_done[(self.n - 1) % self.depth]
         self.s_copy.wait_stream(cur)                                    # the caller's prior work on `image`
         with torch.cuda.stream(self.s_copy):
-            if p.busy:
-                self.s_copy.wait_event(p.enc_done)                      # the plan's previous encoder pass has read its input buffer
+            if busy:
+                self.s_copy.wait_event(self.enc_done[i])                # the plan's previous encoder pass has read its input buffer
             if gray:
-                from .inference import preprocess_gray, preprocess_bgr
                 (preprocess_gray if image.dim() == 3 else preprocess_bgr)(image, size=p.x.shape[-1], out=p.x)
             else:
                 p.x.copy_(image, non_blocking=True)
-            cdone.record(self.s_copy)
+            self.copy_done[i].record(self.s_copy)
         self.s_enc.wait_stream(cur)
         with torch.cuda.stream(self.s_enc):
-            if p.busy:
-                self.s_enc.wait_event(p.dec_done)                       # plan buffers are free again
-            self.s_enc.wait_event(cdone)
+            if busy:
+                self.s_enc.wait_event(self.dec_done[i])                 # plan buffers are free again
+            self.s_enc.wait_event(self.copy_done[i])
             if p.uniforms is not None:
                 if uniforms is None:
                     uniforms = torch.rand((self.B, self.T), dtype=torch.float32, device=dev)
                 p.uniforms.copy_(uniforms.to(torch.float32), non_blocking=True)
-            p.enc_graph.replay()
-            L.note_graph_replay(dev, p.enc_kernels)
-            p.enc_done.record(self.s_enc)
+            replay(dev, p.enc_graph)
+            self.enc_done[i].record(self.s_enc)
         with torch.cuda.stream(s_dec):
-            s_dec.wait_event(p.enc_done)
-            p.dec_graph.replay()
-            L.note_graph_replay(dev, p.dec_kernels)
+            s_dec.wait_event(self.enc_done[i])
+            replay(dev, p.dec_graph)
             tokens, confs = p.tokens.clone(), p.confs.clone()
-            ht = hc = None
-            if self.to_host:
-                ht = torch.empty(tokens.shape, dtype=torch.int32, pin_memory=True)
-                hc = torch.empty(confs.shape, dtype=torch.float32, pin_memory=True)
-                ht.copy_(tokens, non_blocking=True); hc.copy_(confs, non_blocking=True)
-            p.dec_done.record(s_dec)
-            p.busy = True
+            ht, hc = _to_pinned(tokens, confs) if self.to_host else (None, None)
+            self.dec_done[i].record(s_dec)
             done = torch.cuda.Event()
             done.record(s_dec)
         return Ticket(tokens, confs, ht, hc, done, s_dec)
@@ -140,17 +129,12 @@ def generate_stream(model, batches, tokenizer, max_len=50, top_k=0, top_p=1, dep
     max_len, top_k, top_p)` returns -- (LongTensor (B,1+max_len) on CPU, list of ceil(max_len/4) float tensors (B,) on CPU).
     `batches` is any iterable of f32 (B,3,H,W) tensors (host, ideally pinned, or device) -- or of raw grayscale u8 (B,h,w)
     tensors, normalised on the device (preprocess_gray).  `stop_at_eos`: as in generate()."""
-    bos = int(getattr(tokenizer, "BOS_code", CFG.bos_idx))
-    if bos != int(CFG.bos_idx):
-        raise ValueError("tokenizer.BOS_code must equal CFG.bos_idx (model.py:117 reads the global)")
-    from .inference import _stop_token
+    _check_bos(tokenizer)
     eos = _stop_token(tokenizer) if stop_at_eos else None
     pipes, pipe, pending = model.__dict__.setdefault("_stream_pipes", {}), None, []     # plans + graphs are reused across calls
-    n_conf = (max_len + 3) // 4
 
     def finish(t):
-        host, host_c = t.result()
-        return host.long(), [host_c[:, i].clone() for i in range(n_conf)]
+        return _host_result(*t.result())
 
     for x in batches:
         dev = x.device if x.is_cuda else None

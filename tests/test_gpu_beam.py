@@ -5,7 +5,6 @@ checks that premise: one-step windows give the same logits, bit for bit, as one 
 oracle's beam search (fp32), against greedy generate_tokens (K = 1, bf16), against a teacher-forced rescoring of every returned beam
 (which needs no KV reorder), and check the EOS / length-penalty contract with EOS raised to arrive at spread-out steps (the eos_bias /
 choose_delta technique of the stop-at-EOS tests)."""
-import contextlib
 import ctypes as C
 
 import pytest
@@ -16,10 +15,11 @@ pytestmark = pytest.mark.gpu
 import mdcnet_b200 as M  # noqa: E402
 from oracle import cases, mdc_oracle as O  # noqa: E402
 from tests.beam_oracle import generate_beam  # noqa: E402
+from tests.eos_helpers import EOS, choose_delta, eos_bias  # noqa: E402
 
 L = M._lib
 DEV = "cuda"
-EOS, PAD, BOS = 301, 302, 300
+PAD, BOS = 302, 300
 
 
 @pytest.fixture(scope="module")
@@ -35,46 +35,6 @@ def model_s():
 @pytest.fixture(scope="module")
 def model_t():
     return cases.build_product_model("T", seed=0, gamma_seed=5).to(DEV)
-
-
-@contextlib.contextmanager
-def eos_bias(model, delta):
-    b = model.decoder.output.bias
-    with torch.no_grad():
-        saved = b[EOS].clone()
-        b[EOS] += delta
-    try:
-        yield model
-    finally:
-        with torch.no_grad():
-            b[EOS] = saved
-
-
-def choose_delta(model, x, T, **kw):
-    """delta for which some but not all images emit EOS within T steps (greedy), at as many different steps as possible, with no
-    margin within 1e-3 of delta."""
-    _, _, lg = model.generate_tokens(x, T, return_logits=True, use_graph=False, **kw)
-    others = lg.clone()
-    others[..., EOS] = -float("inf")
-    margin = (others.max(-1).values - lg[..., EOS]).double().cpu()          # (B, T)
-    vals = margin.flatten().unique()                                          # sorted
-    mids = (vals[:-1] + vals[1:]) / 2
-    cands = mids[(vals[1:] - vals[:-1]) > 2e-3]
-    cands = cands[torch.linspace(0, len(cands) - 1, min(len(cands), 600)).long()]
-    best, best_key = None, None
-    B = margin.shape[0]
-    for d in cands.tolist():
-        hit = margin < d
-        done = hit.any(1)
-        n = int(done.sum())
-        if not 0 < n < B:
-            continue
-        key = (len(set(hit.float().argmax(1)[done].tolist())), -abs(n / B - 0.6))
-        if best_key is None or key > best_key:
-            best, best_key = d, key
-    if best is None:
-        pytest.fail("no delta leaves some images finished and some not")
-    return best
 
 
 def _seq_sum(lp):

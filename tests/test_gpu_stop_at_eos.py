@@ -5,7 +5,6 @@ image and step, the margin max_{v != eos} logit_v - logit_eos; adding a constant
 first step whose margin is below delta (the trajectory before that step is unchanged).  delta is chosen so that some images finish
 at spread-out steps and some never do, and so that no margin lies within 1e-3 of it (no near-ties).  The contract is then checked
 between the stop and the no-stop runs of the modified model."""
-import contextlib
 
 import pytest
 import torch
@@ -14,9 +13,10 @@ pytestmark = pytest.mark.gpu
 
 import mdcnet_b200 as M  # noqa: E402
 from oracle import cases  # noqa: E402
+from tests.eos_helpers import EOS, choose_delta, eos_bias  # noqa: E402
 
 DEV = "cuda"
-EOS, PAD, BOS = 301, 302, 300
+PAD, BOS = 302, 300
 
 
 @pytest.fixture(scope="module")
@@ -36,46 +36,6 @@ def _model_t():
             if k.endswith("gamma"):
                 p.copy_(torch.rand(p.shape, generator=g) + 0.5)
     return model.to(DEV)
-
-
-@contextlib.contextmanager
-def eos_bias(model, delta):
-    b = model.decoder.output.bias
-    with torch.no_grad():
-        saved = b[EOS].clone()
-        b[EOS] += delta
-    try:
-        yield model
-    finally:
-        with torch.no_grad():
-            b[EOS] = saved
-
-
-def choose_delta(model, x, T, **kw):
-    """delta for which some but not all images emit EOS within T steps, at as many different steps as possible, with no margin within
-    1e-3 of delta."""
-    _, _, lg = model.generate_tokens(x, T, return_logits=True, use_graph=False, **kw)
-    others = lg.clone()
-    others[..., EOS] = -float("inf")
-    margin = (others.max(-1).values - lg[..., EOS]).double().cpu()          # (B, T)
-    vals = margin.flatten().unique()                                          # sorted
-    mids = (vals[:-1] + vals[1:]) / 2
-    cands = mids[(vals[1:] - vals[:-1]) > 2e-3]
-    cands = cands[torch.linspace(0, len(cands) - 1, min(len(cands), 600)).long()]
-    best, best_key = None, None
-    B = margin.shape[0]
-    for d in cands.tolist():
-        hit = margin < d
-        done = hit.any(1)
-        n = int(done.sum())
-        if not 0 < n < B:
-            continue
-        key = (len(set(hit.float().argmax(1)[done].tolist())), -abs(n / B - 0.6))
-        if best_key is None or key > best_key:
-            best, best_key = d, key
-    if best is None:
-        pytest.fail("no delta leaves some images finished and some not")
-    return best
 
 
 def check_contract(tok_ns, conf_ns, tok_s, conf_s, T):
