@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MDC_ABI_VERSION 8
+#define MDC_ABI_VERSION 9
 
 /* element types of activations / weights.  MDC_F16 (IEEE half) is the type of the decode-loop weights under precision MDC_BF16
  * (see the weight table) and of mdc_gemm's fp16 mode. */
@@ -233,6 +233,15 @@ typedef struct mdc_decode_state {
                                        finished, the remaining launches return at entry).  Results stay batch-invariant.  Requires
                                        forced == 0 and logits == NULL (steps that do not run have no logits). */
   int32_t eos_token;                /* the stop token, in [0, vocab) (read only with stop_at_eos) */
+  const int32_t* prompt_len;        /* int32 [B] or NULL (= no prompt).  Prompted decoding: row b knows columns 0..l_b (l_b = prompt_len[b]),
+                                       column 0 BOS and columns 1..l_b the caller's prompt, written into `tokens` before the call.  Step t
+                                       with t + 1 <= l_b is a prompt step: its input is column t and it writes KV position t as any step;
+                                       its output column t+1 keeps the prompt token (never written) and that token is what later steps
+                                       read; it is never counted as an EOS; its conf column (t % 4 == 0) receives the max probability of
+                                       the (filtered) distribution at that step, as a teacher-forced step writes it.  Steps t >= l_b run
+                                       as without a prompt.  With a prompt equal to the first l_b tokens an unprompted call generates,
+                                       tokens and confs are bitwise that call's.  With stop_at_eos the PAD / 0 pre-fill leaves the prompt
+                                       columns alone.  The prompt must hold no EOS (the host layer rejects one).  Requires forced == 0. */
 } mdc_decode_state;
 
 size_t mdc_decode_workspace_bytes(const mdc_model* m, int B);
@@ -261,6 +270,19 @@ int mdc_decode_steps(mdc_model* m, const mdc_decode_state* st, int t_begin, int 
 size_t mdc_decoder_prefill_workspace_bytes(const mdc_model* m, int B, int n);
 int mdc_decoder_prefill(mdc_model* m, const int32_t* tokens, int tokens_ld, int B, int n, const float* pos, const void* cross_kv,
                         float* logits, int logits_ld, int row_offset, int n_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- prompt prefill: steps [0, n) of a decode state as one all-positions pass ------------------------------------------------------
+ * Equivalent, up to rounding, to mdc_decode_steps(st, 0, n) when every row knows columns 1..n (prompt_len[b] >= n, or the columns are
+ * otherwise known): the same layer chain as mdc_decoder_prefill over columns 0..n-1 of st->tokens, and in addition it writes KV positions
+ * 0..n-1 of every layer into the rows' pages through st->page_table (in st->precision, the pool layout mdc_decode_steps reads), the
+ * logits rows t + logits_row_offset of steps t < n when st->logits is set, and the conf columns t / 4 (t % 4 == 0, t < n) when st->confs
+ * is set -- the max probability of the distribution filtered by st->top_k / st->top_p, as the decode select computes it.  It never writes
+ * tokens.  Afterwards mdc_decode_steps(st, n, T) continues.  Not with forced, x_override or per-step stop state (stop_at_eos is honoured by
+ * the continuing mdc_decode_steps call, whose known prefix then covers columns 1..n).
+ * mdc_decode_prefill_workspace_bytes() is 0 where the prefill does not cover the geometry (fp32 precision, widths other than
+ * 256 / 512 / 1024, head widths other than 32 / 64 / 128): callers then run the prompt steps with mdc_decode_steps. */
+size_t mdc_decode_prefill_workspace_bytes(const mdc_model* m, int B, int n);
+int mdc_decode_prefill_steps(mdc_model* m, const mdc_decode_state* st, int n, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- beam search over the paged KV cache ---------------------------------------------------------------------------------
  * B images, K beams (1 <= K <= 16).  Row r = b*K + k of every [B*K, ...] buffer is beam k of image b; each row keeps a score s_r and a

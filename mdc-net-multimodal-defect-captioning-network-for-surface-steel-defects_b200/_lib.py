@@ -61,6 +61,7 @@ class DecodeState(C.Structure):
         ("ctas_per_sm", C.c_int32),
         ("per_op_kernels", C.c_int32),
         ("stop_at_eos", C.c_int32), ("eos_token", C.c_int32),
+        ("prompt_len", C.c_void_p),
     ]
 
 
@@ -107,6 +108,8 @@ SIGNATURES = {
     "mdc_decode_steps": (_I, [_P, C.POINTER(DecodeState), _I, _I, _P]),
     "mdc_decoder_prefill_workspace_bytes": (_SZ, [_P, _I, _I]),
     "mdc_decoder_prefill": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _I, _I, _I, _P, _SZ, _P]),
+    "mdc_decode_prefill_workspace_bytes": (_SZ, [_P, _I, _I]),
+    "mdc_decode_prefill_steps": (_I, [_P, C.POINTER(DecodeState), _I, _P, _SZ, _P]),
     "mdc_beam_workspace_bytes": (_SZ, [_P, _I, _I]),
     "mdc_beam_step": (_I, [_P, C.POINTER(BeamState), _P, _L, _I, _P]),
     "mdc_beam_finalize": (_I, [_P, C.POINTER(BeamState), _I, _F, _P, _P, _P]),

@@ -123,6 +123,13 @@ __device__ __forceinline__ void store8(bf16* p, const float* v) {
     }                                                                                                           \
   } while (0)
 
+// Paged self-attention KV pool (mdc_decode_state.kv_pool): [page][layer][head][k|v][page_tokens][hd] -- the K and V rows of one (page,
+// layer, head) are one contiguous 2 * page_tokens * hd block (the fused decode kernel fetches it with ONE bulk copy).  When a row is 64
+// bytes (hd = 32, 16-bit cache) the 16-byte chunk c of token r is stored at chunk c ^ ((r >> 1) & 3): the bank-conflict-free pattern of
+// the fused kernel's ldmatrix reads (what TMA SWIZZLE_64B would produce).  Every writer and reader of the pool uses this layout.
+template <typename TKV, int HD>
+__device__ __forceinline__ int kv_chunk(int r, int c) { return (HD * (int)sizeof(TKV) == 64) ? (c ^ ((r >> 1) & 3)) : c; }
+
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 static inline size_t esize(int dtype) { return dtype == MDC_BF16 ? 2 : 4; }
 

@@ -727,14 +727,7 @@ __device__ __forceinline__ void attend_one(const float* q /*smem, HD, pre-scaled
   __syncwarp();
 }
 
-// self-attention: appends this step's k,v to the paged cache, then attends over slots 0..t.
-// pool layout: [page][layer][head][k|v][page_tokens][hd] -- the K and V rows of one (page, layer, head) are one contiguous
-// 2 * page_tokens * hd block (the fused decode kernel fetches it with ONE bulk copy).  When a row is 64 bytes (hd = 32, 16-bit
-// cache) the 16-byte chunk c of token r is stored at chunk c ^ ((r >> 1) & 3): the bank-conflict-free pattern of the fused kernel's
-// ldmatrix reads (what TMA SWIZZLE_64B would produce), shared by both implementations.
-template <typename TKV, int HD>
-__device__ __forceinline__ int kv_chunk(int r, int c) { return (HD * (int)sizeof(TKV) == 64) ? (c ^ ((r >> 1) & 3)) : c; }
-
+// self-attention: appends this step's k,v to the paged cache (layout: kv_chunk, common.cuh), then attends over slots 0..t.
 template <typename TKV, int HD>
 __global__ void dec_self_attn_kernel(const float* __restrict__ qkv /*[B,3d]*/, TKV* __restrict__ pool,
                                      const int32_t* __restrict__ page_table, int pages_per_seq, int PT, int n_layers, int layer,
@@ -901,11 +894,12 @@ using namespace mdcsel;
 struct StopArgs { int* fin; int* state; int eos; };
 
 // Once per mdc_decode_steps call, before the first step (inside a captured graph: at the start of every replay): the token columns
-// t_begin+1..t_end become PAD and the conf columns of steps t_begin..t_end-1 zero -- the values of every position after an image's
-// EOS, which the select of a step that runs overwrites with the selected token -- and the finished flags and count come from the
-// known prefix (an EOS among columns 1..t_begin).  One CTA.
+// t_begin+1..t_end past the row's prompt (columns > prompt_len[b]) become PAD and the conf columns of steps t_begin..t_end-1 zero -- the
+// values of every position after an image's EOS, which the select of a step that runs overwrites -- and the finished flags and count
+// come from the known prefix (an EOS among columns 1..t_begin).  One CTA.
 __global__ void __launch_bounds__(SEL_THREADS) dec_stop_init_kernel(int32_t* __restrict__ tokens, int tokens_ld, float* __restrict__ confs,
-                                                                     int confs_ld, int B, int t_begin, int t_end, int pad, StopArgs stop) {
+                                                                     int confs_ld, int B, int t_begin, int t_end, int pad, StopArgs stop,
+                                                                     const int32_t* __restrict__ prompt_len) {
   __shared__ int n_fin;
   if (threadIdx.x == 0) n_fin = 0;
   __syncthreads();
@@ -916,8 +910,10 @@ __global__ void __launch_bounds__(SEL_THREADS) dec_stop_init_kernel(int32_t* __r
     if (f) atomicAdd(&n_fin, 1);
   }
   const int nt = t_end - t_begin;
-  for (int64_t i = threadIdx.x; i < (int64_t)B * nt; i += SEL_THREADS)
-    tokens[(i / nt) * tokens_ld + t_begin + 1 + i % nt] = pad;
+  for (int64_t i = threadIdx.x; i < (int64_t)B * nt; i += SEL_THREADS) {
+    const int64_t b = i / nt; const int c = t_begin + 1 + (int)(i % nt);
+    if (prompt_len == nullptr || c > prompt_len[b]) tokens[b * tokens_ld + c] = pad;
+  }
   const int c0 = (t_begin + 3) / 4, nc = (t_end + 3) / 4 - c0;      // conf columns of the steps t % 4 == 0 in [t_begin, t_end)
   if (confs && nc > 0)
     for (int64_t i = threadIdx.x; i < (int64_t)B * nc; i += SEL_THREADS) confs[(i / nc) * confs_ld + c0 + i % nc] = 0.f;
@@ -929,12 +925,14 @@ __global__ void __launch_bounds__(SEL_THREADS) dec_stop_init_kernel(int32_t* __r
 // to the caller's logits tensor, then greedy / top-k / top-p select + max-prob.  One CTA per image.
 // With stop at EOS an image that has finished is left alone (its columns hold PAD / 0 from dec_stop_init_kernel); an image that
 // selects EOS is marked finished and counted, and the count reaching B sets the all-finished flag.  (An image not yet finished keeps
-// the count below B during this launch, so the flag cannot change under a CTA that runs.)
+// the count below B during this launch, so the flag cannot change under a CTA that runs.)  A prompt step (t + 1 <= prompt_len[b])
+// writes its conf but neither the token column, which holds the prompt, nor an EOS count.
 __global__ void __launch_bounds__(SEL_THREADS) dec_select_kernel(const float* __restrict__ step_logits, int V, int Vp2, int t,
                                                                   float* __restrict__ logits_out, int64_t logits_img_stride, int logits_row,
                                                                   int32_t* __restrict__ tokens, int tokens_ld, int forced,
                                                                   float* __restrict__ confs, int confs_ld, const float* __restrict__ uniforms,
-                                                                  int uniforms_ld, int top_k, float top_p, StopArgs stop) {
+                                                                  int uniforms_ld, int top_k, float top_p, StopArgs stop,
+                                                                  const int32_t* __restrict__ prompt_len) {
   extern __shared__ __align__(16) float sm[];
   float* lg = sm;             // V
   float* srt = lg + V;        // Vp2
@@ -952,9 +950,10 @@ __global__ void __launch_bounds__(SEL_THREADS) dec_select_kernel(const float* __
   int token; float conf;
   select_from_logits(lg, srt, V, Vp2, top_k, top_p, sample, u, token, conf);
   if (threadIdx.x == 0) {
-    if (!forced) tokens[(int64_t)b * tokens_ld + t + 1] = token;
+    const bool prompt_step = prompt_len != nullptr && t + 1 <= prompt_len[b];
+    if (!forced && !prompt_step) tokens[(int64_t)b * tokens_ld + t + 1] = token;
     if (confs && (t % 4 == 0)) confs[(int64_t)b * confs_ld + t / 4] = conf;
-    if (stop.fin != nullptr && token == stop.eos) {
+    if (stop.fin != nullptr && token == stop.eos && !prompt_step) {
       stop.fin[b] = 1;
       if (atomicAdd(&stop.state[0], 1) + 1 == (int)gridDim.x) stop.state[1] = 1;
     }
@@ -1188,7 +1187,7 @@ int decode_step_typed(mdc_model* m, const mdc_decode_state* st, int t, cudaStrea
     MDC_ENSURE_SMEM(dec_select_kernel, smem);
     dec_select_kernel<<<B, SEL_THREADS, smem, s>>>(sc.lg, V, Vp2, t, st->logits, (int64_t)st->logits_ld * V, t + st->logits_row_offset,
                                                   st->tokens, st->tokens_ld, st->forced, st->confs, st->confs_ld, st->uniforms,
-                                                  st->uniforms_ld, st->top_k, st->top_p, stop);
+                                                  st->uniforms_ld, st->top_k, st->top_p, stop, st->prompt_len);
     MDC_LAUNCH_CHECK(ctx);
   }
   return 0;
@@ -1218,6 +1217,7 @@ extern "C" int mdc_decode_steps(mdc_model* m, const mdc_decode_state* st, int t_
   if (st->confs) MDC_CHECK_ARG((t_end + 3) / 4 <= st->confs_ld);
   if ((st->top_k != 0 || st->top_p != 1.0f) && !st->forced) MDC_CHECK_ARG(st->uniforms && t_end <= st->uniforms_ld);
   if (st->stop_at_eos) MDC_CHECK_ARG(!st->forced && !st->logits && st->eos_token >= 0 && st->eos_token < m->d.vocab);
+  if (st->prompt_len) MDC_CHECK_ARG(!st->forced && !st->x_override);
   cudaStream_t s = (cudaStream_t)stream;
   if (t_end > t_begin && decode_cluster_supported(m, st, t_end)) {
     Scratch sc = carve(m->d, st->B, st->scratch);      // the cluster kernel only needs the step-logits area
@@ -1226,7 +1226,7 @@ extern "C" int mdc_decode_steps(mdc_model* m, const mdc_decode_state* st, int t_
   if (st->stop_at_eos && t_end > t_begin) {
     Scratch sc = carve(m->d, st->B, st->scratch);
     dec_stop_init_kernel<<<1, SEL_THREADS, 0, s>>>(st->tokens, st->tokens_ld, st->confs, st->confs_ld, st->B, t_begin, t_end, m->d.pad_idx,
-                                                   StopArgs{sc.fin, sc.stop_state, st->eos_token});
+                                                   StopArgs{sc.fin, sc.stop_state, st->eos_token}, st->prompt_len);
     MDC_LAUNCH_CHECK(m->ctx);
   }
   for (int t = t_begin; t < t_end; ++t) {

@@ -89,7 +89,9 @@ struct Lay {
   static constexpr int NBARS = 2 * NS_MAX + 6;
   static constexpr int SMEM_USED = OFF_BARS + NBARS * 8;
   static constexpr int SMEM_BYTES = SMEM_USED + 1024;             // + alignment slack
-  static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
+  static constexpr int OFF_PLEN = SMEM_USED;                      // kPrompt only: [GMX] int32 prompt lengths of the group, past the
+  static constexpr int SMEM_BYTES_PROMPT = SMEM_BYTES + GMX * 4;  // layout of the instantiations without a prompt (which stays as it was)
+  static_assert(SMEM_BYTES_PROMPT <= 227 * 1024, "shared memory budget");
   static_assert(OFF_XH % 16 == 0 && OFF_XRES % 16 == 0 && OFF_F2RECV % 16 == 0 && OFF_QS % 16 == 0 && OFF_OST % 16 == 0 && OFF_BARS % 8 == 0, "alignment");
   static_assert(!OVL || 4 * GMX * 32 * 4 >= SEL_BYTES, "select scratch must fit the q/k/v/y staging it shares");
   static_assert(GMX * 2048 == STAGE, "a 16-key chunk of all images' K and V head slices fills a stage");
@@ -119,6 +121,7 @@ struct __align__(64) FusedParams {
   int t_begin, t_end;
   long long* trace; int trace_t;           // developer aid: phase timestamps of CTA 0 at step trace_t (MDC_DECODE_TRACE_PTR)
   float ref_margin;                        // developer build: softmax reference-maximum margin (MDC_DECODE_REF_MARGIN; the product build uses 64)
+  const int32_t* prompt_len;               // mdc_decode_state.prompt_len (read by the kPrompt instantiations)
 };
 
 __device__ __forceinline__ void cbar() { bar_sync<1, NCT>(); }   // the 8 consumer warps
@@ -297,7 +300,9 @@ __device__ __forceinline__ void warp_greedy_select(const float* lg, int V, int& 
 // i.e. two independent image groups) share an SM, so that one group's dependent phase chain fills the other's stalls.
 // kStop: stop at EOS (mdc_decode_state.stop_at_eos).  A template parameter, so that the instantiations without it compile to the code
 // they had before the option existed (as a run-time flag its few instructions shifted the register allocation: -1.2 % img/s).
-template <bool kTrace, int NB, int NSTG, int MINB, bool kStop>
+// kPrompt: prompted decoding (mdc_decode_state.prompt_len), a template parameter for the same reason: a prompt step publishes the
+// prompt token of column t+1 instead of the selected one and never counts as an EOS.
+template <bool kTrace, int NB, int NSTG, int MINB, bool kStop, bool kPrompt>
 __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fused_kernel(const __grid_constant__ FusedParams P) {
   using Y = Lay<NB, NSTG, NB == 2 || MINB == 2>;
   constexpr int GMX = Y::GMX, NS = Y::NS, STAGE = Y::STAGE;
@@ -322,6 +327,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
   int* haspad = (int*)(smem + Y::OFF_HASPAD);
   uint32_t* finm = (uint32_t*)(smem + Y::OFF_FIN); volatile int* all_fin = (int*)(smem + Y::OFF_FIN + 8);
   uint32_t* ph_step = (uint32_t*)(smem + Y::OFF_FIN + 12);     // in shared memory: a register live across the group loop costs spills
+  int* plen = (int*)(smem + Y::OFF_PLEN);                        // kPrompt only
   const uint32_t bars = sbase + Y::OFF_BARS;
   auto bar = [&](int i) -> uint32_t { return bars + i * 8; };
 
@@ -366,6 +372,8 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
           if (P.tokens[(int64_t)(img0 + g) * P.tokens_ld + w * 32 + b] == P.pad_idx) bits |= 1u << b;
       padbits[i] = bits;
     }
+    if (kPrompt)
+      for (int i = tid; i < GMX; i += NT) plen[i] = i < G ? P.prompt_len[img0 + i] : 0;
     __syncthreads();
     if (tid < GMX) {
       uint32_t any = 0;
@@ -744,7 +752,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
         // ---- stop at EOS: finished mask before step t (bit g: image g has emitted EOS, or had one among columns 1..t_begin) and the
         //      decision whether step t runs.  Every CTA of the cluster received the same tokens, so every CTA decides the same. -------
         if (kStop && warp == 0) {
-          const bool eos_now = t > P.t_begin && lane < G && tokbuf[(t & 1) * GMX + lane] == P.eos;
+          const bool eos_now = t > P.t_begin && lane < G && tokbuf[(t & 1) * GMX + lane] == P.eos && !(kPrompt && t <= plen[lane]);
           const uint32_t f = finm[(t + 1) & 1] | __ballot_sync(0xffffffffu, eos_now);
           if (lane == 0) {
             finm[t & 1] = f;
@@ -819,7 +827,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
             const float4 a = *reinterpret_cast<const float4*>(src), b = *reinterpret_cast<const float4*>(src + 4);
             uint4 o; o.x = pack_bf16x2(a.x, a.y); o.y = pack_bf16x2(a.z, a.w); o.z = pack_bf16x2(b.x, b.y); o.w = pack_bf16x2(b.z, b.w);
             const int page = pages[g * 32 + t / P.PT];
-            const int r = t % P.PT;      // pool: [page][layer][head][k|v][16 tokens][32]; chunk ch of token r at ch ^ ((r >> 1) & 3) (decode.cu kv_chunk)
+            const int r = t % P.PT;      // pool: [page][layer][head][k|v][16 tokens][32]; chunk ch of token r at ch ^ ((r >> 1) & 3) (common.cuh kv_chunk)
             bf16* dst = P.kv_pool + ((((int64_t)page * L + l) * CS + rank) * 2 + which) * (int64_t)(P.PT * HD) + r * HD + ((ch ^ ((r >> 1) & 3)) << 3);
             *reinterpret_cast<uint4*>(dst) = o;
           }
@@ -1024,8 +1032,10 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, MINB) decode_fu
           ph_lg ^= 1;
           auto publish = [&](int img, int token, float conf) {     // one thread: token to the caller's buffer and to every peer
             if (kStop && ((finm[t & 1] >> img) & 1u)) { token = P.pad_idx; conf = 0.f; }    // finished before step t
+            const bool prompt_step = kPrompt && t + 1 <= plen[img];     // column t+1 holds the prompt: exchange it, leave it alone
+            if (prompt_step) token = __ldcg(P.tokens + (int64_t)(img0 + img) * P.tokens_ld + t + 1);
             if (!P.forced) {
-              P.tokens[(int64_t)(img0 + img) * P.tokens_ld + t + 1] = token;
+              if (!prompt_step) P.tokens[(int64_t)(img0 + img) * P.tokens_ld + t + 1] = token;
               const uint32_t off = sbase + Y::OFF_TOK + ((((t + 1) & 1) * GMX) + img) * 4;
 #pragma unroll
               for (int p = 0; p < CS; ++p) st_async_b32(mapa(off, p), (uint32_t)token, mapa(bar(BAR_TOK), p));
@@ -1144,19 +1154,22 @@ bool geometry_ok(const mdc_dims& d) {
 // 2: NB = 1, 4-stage ring (64 KB), compact layout, two CTAs per SM (<= 8 images per cluster; two clusters interleave on the same SMs)
 constexpr int N_VARIANTS = 3;
 template <bool kTrace> struct Variants {
-  template <bool kStop> static const void* fn_(int v) {
+  template <bool kStop, bool kPrompt> static const void* fn_(int v) {
     switch (v) {
-      case 0: return (const void*)decode_fused_kernel<kTrace, 1, 10, 1, kStop>;
-      case 1: return (const void*)decode_fused_kernel<kTrace, 2, 4, 1, kStop>;
-      default: return (const void*)decode_fused_kernel<kTrace, 1, 4, 2, kStop>;
+      case 0: return (const void*)decode_fused_kernel<kTrace, 1, 10, 1, kStop, kPrompt>;
+      case 1: return (const void*)decode_fused_kernel<kTrace, 2, 4, 1, kStop, kPrompt>;
+      default: return (const void*)decode_fused_kernel<kTrace, 1, 4, 2, kStop, kPrompt>;
     }
   }
-  static const void* fn(int v, bool stop) { return stop ? fn_<true>(v) : fn_<false>(v); }
+  static const void* fn(int v, bool stop, bool prompt) {
+    return prompt ? (stop ? fn_<true, true>(v) : fn_<false, true>(v)) : (stop ? fn_<true, false>(v) : fn_<false, false>(v));
+  }
 };
-int variant_smem(int v) { return v == 0 ? Lay<1, 10, false>::SMEM_BYTES : (v == 1 ? Lay<2, 4, true>::SMEM_BYTES : Lay<1, 4, true>::SMEM_BYTES); }
+template <int NB, int NSTG, bool OVL> int lay_smem(bool prompt) { return prompt ? Lay<NB, NSTG, OVL>::SMEM_BYTES_PROMPT : Lay<NB, NSTG, OVL>::SMEM_BYTES; }
+int variant_smem(int v, bool prompt) { return v == 0 ? lay_smem<1, 10, false>(prompt) : (v == 1 ? lay_smem<2, 4, true>(prompt) : lay_smem<1, 4, true>(prompt)); }
 
 // per-context (= per-device) launch state: the dynamic-smem opt-in and the occupancy query are device properties
-struct ClusterCtxState { int max_clusters[N_VARIANTS][2]; };      // [variant][stop at EOS]
+struct ClusterCtxState { int max_clusters[N_VARIANTS][2][2]; };      // [variant][stop at EOS][prompt]
 
 }  // namespace
 
@@ -1246,6 +1259,7 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
   P.confs = st->confs; P.confs_ld = st->confs_ld;
   P.uniforms = st->uniforms; P.uniforms_ld = st->uniforms_ld; P.top_k = st->top_k; P.top_p = st->top_p; P.forced = st->forced;
   P.eos = st->eos_token;
+  P.prompt_len = st->prompt_len;
   P.t_begin = t_begin; P.t_end = t_end;
   P.trace = nullptr; P.trace_t = -1; P.ref_margin = 64.0f;
   int ipc = st->images_per_cluster, cps = st->ctas_per_sm;
@@ -1261,13 +1275,13 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
   const int gmx = variant == 1 ? 16 : 8;
   if (!ctx->decode_state) { ClusterCtxState* cs = new ClusterCtxState(); memset(cs, 0, sizeof(*cs)); ctx->decode_state = cs; }
   ClusterCtxState* cs = (ClusterCtxState*)ctx->decode_state;
-  const int smem = variant_smem(variant);
-  const bool stop = st->stop_at_eos != 0;
-  if (!cs->max_clusters[variant][stop]) {
-    const void* fn = Variants<false>::fn(variant, stop);
+  const bool stop = st->stop_at_eos != 0, prompt = st->prompt_len != nullptr;
+  const int smem = variant_smem(variant, prompt);
+  if (!cs->max_clusters[variant][stop][prompt]) {
+    const void* fn = Variants<false>::fn(variant, stop, prompt);
     MDC_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 #ifdef MDC_DEVTOOLS
-    MDC_CUDA(cudaFuncSetAttribute(Variants<true>::fn(variant, stop), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    MDC_CUDA(cudaFuncSetAttribute(Variants<true>::fn(variant, stop, prompt), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 #endif
     cudaLaunchConfig_t q{}; q.gridDim = dim3(CS * 64); q.blockDim = dim3(NT); q.dynamicSmemBytes = smem;
     cudaLaunchAttribute a[1]; a[0].id = cudaLaunchAttributeClusterDimension; a[0].val.clusterDim.x = CS; a[0].val.clusterDim.y = 1; a[0].val.clusterDim.z = 1;
@@ -1275,9 +1289,9 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
     int n = 0;
     cudaError_t e = cudaOccupancyMaxActiveClusters(&n, fn, &q);
     if (e != cudaSuccess || n < 1) { (void)cudaGetLastError(); n = ctx->sm_count / CS / 2; if (n < 1) n = 1; }
-    cs->max_clusters[variant][stop] = n;
+    cs->max_clusters[variant][stop][prompt] = n;
   }
-  const int max_clusters = cs->max_clusters[variant][stop];
+  const int max_clusters = cs->max_clusters[variant][stop][prompt];
   int G = (P.B + max_clusters - 1) / max_clusters;
   if (ipc > 0 && ipc > G) G = ipc;                                                              // fewer, fuller clusters (batch pipelining)
   if (G > gmx) G = gmx;
@@ -1286,9 +1300,9 @@ int decode_cluster_launch(mdc_model* m, const mdc_decode_state* st, int t_begin,
   P.n_groups = (P.B + G - 1) / G;
   const int n_clusters = P.n_groups < max_clusters ? P.n_groups : max_clusters;
   void* args[1] = {(void*)&P};
-  const void* fn = Variants<false>::fn(variant, stop);
+  const void* fn = Variants<false>::fn(variant, stop, prompt);
 #ifdef MDC_DEVTOOLS
-  if (P.trace) fn = Variants<true>::fn(variant, stop);
+  if (P.trace) fn = Variants<true>::fn(variant, stop, prompt);
 #endif
   MDC_CUDA(cudaLaunchKernel(fn, dim3(n_clusters * CS), dim3(NT), args, (size_t)smem, s));
   MDC_LAUNCH_CHECK(ctx);

@@ -8,8 +8,12 @@
 //   x     = LN2(x + cross . W_co^T + b);  x = LN3(x + W2 relu(W1 x + b1) + b2)
 // and the vocabulary head runs once over all rows.  Mask semantics as the reference builds them (utils.py:7-12,26-30; Q7): -inf above
 // the diagonal, +1.0 (a float mask, not -inf) on PAD keys.
+// The same layer chain serves mdc_decode_prefill_steps (a prompt in one pass): there every layer's self-attention K/V columns are also
+// scattered into the paged pool the decode kernels read, and the head runs only when logits or confidences are wanted.
 #include "common.cuh"
+#include "select.cuh"
 #include <cuda_fp16.h>
+#include <algorithm>
 
 namespace {
 
@@ -236,12 +240,139 @@ __global__ void __launch_bounds__(128) prefill_head_kernel(const __half* __restr
   }
 }
 
+// ---- K/V columns of one layer's in-projection output -> the paged self-attention pool (layout: kv_chunk, common.cuh) ----------------
+// qkv: fp16 [B*n][3*dim] (q | k | v); position i of image b goes to slot i % PT of page page_table[b][i / PT], rounded to the cache type
+// as the decode kernels round it.  One thread per 16-byte chunk of the pool.
+template <int HD>
+__global__ void prefill_kv_scatter_kernel(const __half* __restrict__ qkv, int n, int dim, bf16* __restrict__ pool, const int32_t* __restrict__ page_table,
+                                          int pages_per_seq, int PT, int n_layers, int layer, int64_t total) {
+  constexpr int CPR = HD / 8;                       // 16-byte chunks of one head row in the pool
+  const int heads = dim / HD;
+  for (int64_t id = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; id < total; id += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(id % CPR);
+    const int64_t rest = id / CPR;
+    const int head = (int)(rest % heads), which = (int)((rest / heads) & 1);
+    const int64_t row = rest / heads / 2;
+    const int b = (int)(row / n), i = (int)(row % n), r = i % PT;
+    float v[8]; load8(qkv + row * 3 * dim + (1 + which) * dim + head * HD + c * 8, v);
+    const int64_t page = page_table[(int64_t)b * pages_per_seq + i / PT];
+    bf16* dst = pool + ((((page * n_layers + layer) * heads + head) * 2 + which) * PT + r) * (int64_t)HD + kv_chunk<bf16, HD>(r, c) * 8;
+    store8(dst, v);
+  }
+}
+
+// ---- conf columns of the prefilled steps: max probability of the filtered distribution, as the decode select computes it --------------
+// One CTA per (image, step t < n with t % 4 == 0); logits of step t at logits + b * img_stride + (t + row_offset) * V.
+__global__ void __launch_bounds__(mdcsel::SEL_THREADS) prefill_conf_kernel(const float* __restrict__ logits, int64_t img_stride, int row_offset,
+                                                                           int V, int Vp2, int top_k, float top_p, float* __restrict__ confs,
+                                                                           int confs_ld, int n_conf) {
+  extern __shared__ __align__(16) float sel_sm[];
+  float* lg = sel_sm; float* srt = sel_sm + V;
+  const int b = blockIdx.x / n_conf, t = (blockIdx.x % n_conf) * 4;
+  const float* src = logits + (int64_t)b * img_stride + (int64_t)(t + row_offset) * V;
+  for (int i = threadIdx.x; i < V; i += mdcsel::SEL_THREADS) lg[i] = src[i];
+  __syncthreads();
+  int token; float conf;
+  mdcsel::select_from_logits(lg, srt, V, Vp2, top_k, top_p, false, 0.f, token, conf);
+  if (threadIdx.x == 0) confs[(int64_t)b * confs_ld + t / 4] = conf;
+}
+
 struct Ws { float* x32; __half* x16; __half* qkv; __half* o16; __half* y16; __half* h16; float* kbias; };
 
 size_t ws_bytes(const mdc_dims& d, int B, int n) {
   const size_t R = (size_t)B * n;
   return align_up(R * d.dim * 4, 256) + align_up(R * d.dim * 2, 256) + align_up(R * 3 * d.dim * 2, 256) + align_up(R * d.dim * 2, 256) +
          align_up(R * d.dim * 2, 256) + align_up(R * d.dec_ffn * 2, 256) + align_up(R * 4, 256);
+}
+
+Ws carve(const mdc_dims& d, int B, int n, void* workspace) {
+  const int64_t R = (int64_t)B * n, dim = d.dim;
+  char* p = (char*)workspace; Ws w;
+  w.x32 = (float*)p; p += align_up(R * dim * 4, 256);
+  w.x16 = (__half*)p; p += align_up(R * dim * 2, 256);
+  w.qkv = (__half*)p; p += align_up(R * 3 * dim * 2, 256);
+  w.o16 = (__half*)p; p += align_up(R * dim * 2, 256);
+  w.y16 = (__half*)p; p += align_up(R * dim * 2, 256);
+  w.h16 = (__half*)p; p += align_up(R * d.dec_ffn * 2, 256);
+  w.kbias = (float*)p;
+  return w;
+}
+
+// where the layer chain also writes its self-attention K/V: the paged pool of a decode state (NULL pool = nowhere)
+struct KvSink { bf16* pool; const int32_t* page_table; int pages_per_seq; };
+
+constexpr int ROWS_PER_BLOCK = 8;
+constexpr int HEAD_THREADS = 128;
+
+// Embedding, then every decoder layer over the B*n rows (w.x16 holds the last layer's output for the head).  With kv.pool every layer's
+// K/V columns go to the pool; without `full_last` the last layer stops after that (its output is not needed).
+int run_layers(mdc_model* m, const int32_t* tokens, int tokens_ld, int B, int n, const float* pos, const void* cross_kv, const Ws& w,
+               const KvSink& kv, bool full_last, cudaStream_t s) {
+  mdc_ctx* ctx = m->ctx; const mdc_dims& d = m->d;
+  const int dim = d.dim, S = d.n_patches, heads = d.dec_heads;
+  const void** gw = m->w + MDC_ENC_GLOBAL_SLOTS + d.enc_depth * MDC_ENC_BLOCK_SLOTS;
+  const void** lw0 = gw + MDC_DEC_GLOBAL_SLOTS;
+  const int64_t R = (int64_t)B * n;
+  const int row_blocks = (int)((R + ROWS_PER_BLOCK - 1) / ROWS_PER_BLOCK);
+  prefill_embed_kernel<<<row_blocks, ROWS_PER_BLOCK * 32, 0, s>>>(tokens, tokens_ld, n, dim, (const float*)gw[MDC_EMB], pos, d.pad_idx, w.x32, w.x16, w.kbias, R);
+  MDC_LAUNCH_CHECK(ctx);
+  const int hd = dim / heads;
+  const float scale_log2e = LOG2E / sqrtf((float)hd);
+  const dim3 agrid(heads, B, (n + QCH - 1) / QCH);
+#define MDC_ATTN(TKV_, CAUSAL_, ...)                                                                          \
+  {                                                                                                           \
+    if (hd == 32) prefill_attn_kernel<TKV_, CAUSAL_, 32><<<agrid, 256, 0, s>>>(__VA_ARGS__);                  \
+    else if (hd == 64) prefill_attn_kernel<TKV_, CAUSAL_, 64><<<agrid, 256, 0, s>>>(__VA_ARGS__);             \
+    else prefill_attn_kernel<TKV_, CAUSAL_, 128><<<agrid, 256, 0, s>>>(__VA_ARGS__);                          \
+    MDC_LAUNCH_CHECK(ctx);                                                                                    \
+  }
+#define MDC_ADDLN(...)                                                                                        \
+  {                                                                                                           \
+    if (dim == 256) add_layernorm_kernel<1><<<row_blocks, ROWS_PER_BLOCK * 32, 0, s>>>(__VA_ARGS__);          \
+    else if (dim == 512) add_layernorm_kernel<2><<<row_blocks, ROWS_PER_BLOCK * 32, 0, s>>>(__VA_ARGS__);     \
+    else add_layernorm_kernel<4><<<row_blocks, ROWS_PER_BLOCK * 32, 0, s>>>(__VA_ARGS__);                     \
+    MDC_LAUNCH_CHECK(ctx);                                                                                    \
+  }
+  for (int l = 0; l < d.dec_layers; ++l) {
+    const void** lw = lw0 + l * MDC_DEC_LAYER_SLOTS;
+    // self-attention block
+    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.x16, dim, lw[MDC_SA_IN_W], dim, w.qkv, 3 * dim, (const float*)lw[MDC_SA_IN_B], nullptr, 0, (int)R, 3 * dim, dim, s));
+    if (kv.pool) {
+      const int64_t total = R * 2 * dim / 8;
+      const int grid = (int)std::min<int64_t>((total + 255) / 256, (int64_t)ctx->sm_count * 8);
+      if (hd == 32) prefill_kv_scatter_kernel<32><<<grid, 256, 0, s>>>(w.qkv, n, dim, kv.pool, kv.page_table, kv.pages_per_seq, d.page_tokens, d.dec_layers, l, total);
+      else if (hd == 64) prefill_kv_scatter_kernel<64><<<grid, 256, 0, s>>>(w.qkv, n, dim, kv.pool, kv.page_table, kv.pages_per_seq, d.page_tokens, d.dec_layers, l, total);
+      else prefill_kv_scatter_kernel<128><<<grid, 256, 0, s>>>(w.qkv, n, dim, kv.pool, kv.page_table, kv.pages_per_seq, d.page_tokens, d.dec_layers, l, total);
+      MDC_LAUNCH_CHECK(ctx);
+      if (l + 1 == d.dec_layers && !full_last) break;
+    }
+    MDC_ATTN(__half, true, w.qkv, 3 * dim, w.qkv + dim, w.qkv + 2 * dim, 3 * dim, w.kbias, w.o16, dim, n, n, scale_log2e)
+    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.o16, dim, lw[MDC_SA_OUT_W], dim, w.y16, dim, (const float*)lw[MDC_SA_OUT_B], nullptr, 0, (int)R, dim, dim, s));
+    MDC_ADDLN(w.x32, w.y16, (const float*)lw[MDC_LN1_W], (const float*)lw[MDC_LN1_B], w.x16, R, 1e-5f)
+    // cross-attention block: q from rows [0,dim) of the packed in-projection; K/V = the resident cross-K/V of this layer
+    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.x16, dim, lw[MDC_CA_IN_W], dim, w.qkv, dim, (const float*)lw[MDC_CA_IN_B], nullptr, 0, (int)R, dim, dim, s));
+    const bf16* ckv = (const bf16*)cross_kv + (size_t)l * B * S * 2 * dim;
+    MDC_ATTN(bf16, false, w.qkv, dim, ckv, ckv + dim, 2 * dim, nullptr, w.o16, dim, n, S, scale_log2e)
+    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.o16, dim, lw[MDC_CA_OUT_W], dim, w.y16, dim, (const float*)lw[MDC_CA_OUT_B], nullptr, 0, (int)R, dim, dim, s));
+    MDC_ADDLN(w.x32, w.y16, (const float*)lw[MDC_LN2_W], (const float*)lw[MDC_LN2_B], w.x16, R, 1e-5f)
+    // feed-forward block
+    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS_RELU, w.x16, dim, lw[MDC_FF1_W], dim, w.h16, d.dec_ffn, (const float*)lw[MDC_FF1_B], nullptr, 0, (int)R, d.dec_ffn, dim, s));
+    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.h16, d.dec_ffn, lw[MDC_FF2_W], d.dec_ffn, w.y16, dim, (const float*)lw[MDC_FF2_B], nullptr, 0, (int)R, dim, d.dec_ffn, s));
+    MDC_ADDLN(w.x32, w.y16, (const float*)lw[MDC_LN3_W], (const float*)lw[MDC_LN3_B], w.x16, R, 1e-5f)
+  }
+#undef MDC_ATTN
+#undef MDC_ADDLN
+  return 0;
+}
+
+int launch_head(mdc_model* m, const Ws& w, int B, int n, float* logits, int64_t img_stride, int row_offset, int n_out, cudaStream_t s) {
+  const mdc_dims& d = m->d;
+  const void** gw = m->w + MDC_ENC_GLOBAL_SLOTS + d.enc_depth * MDC_ENC_BLOCK_SLOTS;
+  const int64_t R = (int64_t)B * n;
+  prefill_head_kernel<<<(int)((R + HEAD_ROWS - 1) / HEAD_ROWS), HEAD_THREADS, (size_t)HEAD_ROWS * d.dim * sizeof(float), s>>>(
+      w.x16, (const __half*)gw[MDC_OUT_W], (const float*)gw[MDC_OUT_B], logits, img_stride, row_offset, n, n_out, d.vocab, R, d.dim);
+  MDC_LAUNCH_CHECK(m->ctx);
+  return 0;
 }
 
 bool geometry_ok(const mdc_dims& d) {
@@ -264,65 +395,57 @@ extern "C" int mdc_decoder_prefill(mdc_model* m, const int32_t* tokens, int toke
   MDC_CHECK_ARG(geometry_ok(m->d));
   MDC_CHECK_ARG(workspace_bytes >= ws_bytes(m->d, B, n));
   MDC_CHECK_ARG(n_out >= 0 && n_out <= n && row_offset >= 0 && n_out + row_offset <= logits_ld);
-  mdc_ctx* ctx = m->ctx; const mdc_dims& d = m->d; cudaStream_t s = (cudaStream_t)stream;
-  const int dim = d.dim, S = d.n_patches, heads = d.dec_heads;
+  const mdc_dims& d = m->d; cudaStream_t s = (cudaStream_t)stream;
   const void** gw = m->w + MDC_ENC_GLOBAL_SLOTS + d.enc_depth * MDC_ENC_BLOCK_SLOTS;
-  const void** lw0 = gw + MDC_DEC_GLOBAL_SLOTS;
   if (!pos) { MDC_CHECK_ARG(n <= d.max_pos); pos = (const float*)gw[MDC_DEC_POS]; }
-  const int64_t R = (int64_t)B * n;
-  char* p = (char*)workspace; Ws w;
-  w.x32 = (float*)p; p += align_up(R * dim * 4, 256);
-  w.x16 = (__half*)p; p += align_up(R * dim * 2, 256);
-  w.qkv = (__half*)p; p += align_up(R * 3 * dim * 2, 256);
-  w.o16 = (__half*)p; p += align_up(R * dim * 2, 256);
-  w.y16 = (__half*)p; p += align_up(R * dim * 2, 256);
-  w.h16 = (__half*)p; p += align_up(R * d.dec_ffn * 2, 256);
-  w.kbias = (float*)p;
-  const int rows_per_block = 8;
-  const int row_blocks = (int)((R + rows_per_block - 1) / rows_per_block);
-  prefill_embed_kernel<<<row_blocks, rows_per_block * 32, 0, s>>>(tokens, tokens_ld, n, dim, (const float*)gw[MDC_EMB], pos, d.pad_idx, w.x32, w.x16, w.kbias, R);
-  MDC_LAUNCH_CHECK(ctx);
-  const int hd = dim / heads;
-  const float scale_log2e = LOG2E / sqrtf((float)hd);
-  const dim3 agrid(heads, B, (n + QCH - 1) / QCH);
-#define MDC_ATTN(TKV_, CAUSAL_, ...)                                                                          \
-  {                                                                                                           \
-    if (hd == 32) prefill_attn_kernel<TKV_, CAUSAL_, 32><<<agrid, 256, 0, s>>>(__VA_ARGS__);                  \
-    else if (hd == 64) prefill_attn_kernel<TKV_, CAUSAL_, 64><<<agrid, 256, 0, s>>>(__VA_ARGS__);             \
-    else prefill_attn_kernel<TKV_, CAUSAL_, 128><<<agrid, 256, 0, s>>>(__VA_ARGS__);                          \
-    MDC_LAUNCH_CHECK(ctx);                                                                                    \
+  const Ws w = carve(d, B, n, workspace);
+  MDC_TRY(run_layers(m, tokens, tokens_ld, B, n, pos, cross_kv, w, KvSink{nullptr, nullptr, 0}, true, s));
+  if (n_out > 0) MDC_TRY(launch_head(m, w, B, n, logits, (int64_t)logits_ld * d.vocab, row_offset, n_out, s));
+  return 0;
+}
+
+// logits of the prefilled steps when the caller wants confidences but no logits: [B][n][vocab] f32 behind the layer-chain workspace
+static size_t prefill_steps_ws_bytes(const mdc_dims& d, int B, int n) {
+  return ws_bytes(d, B, n) + align_up((size_t)B * n * d.vocab * sizeof(float), 256);
+}
+
+extern "C" size_t mdc_decode_prefill_workspace_bytes(const mdc_model* m, int B, int n) {
+  if (!m || B <= 0 || n <= 0 || !geometry_ok(m->d)) return 0;
+  return prefill_steps_ws_bytes(m->d, B, n);
+}
+
+extern "C" int mdc_decode_prefill_steps(mdc_model* m, const mdc_decode_state* st, int n, void* workspace, size_t workspace_bytes, void* stream) {
+  MDC_CHECK_ARG(m && st && st->B > 0 && st->tokens && st->kv_pool && st->page_table && st->cross_kv && workspace && n > 0);
+  MDC_CHECK_DEVICE(m->ctx);
+  const mdc_dims& d = m->d; const int B = st->B;
+  MDC_CHECK_ARG(geometry_ok(d));
+  MDC_CHECK_ARG(!st->forced && !st->x_override);
+  MDC_CHECK_ARG(workspace_bytes >= prefill_steps_ws_bytes(d, B, n));
+  MDC_CHECK_ARG(st->pos_override || n <= d.max_pos);
+  MDC_CHECK_ARG(n <= st->pages_per_seq * d.page_tokens && n < st->tokens_ld);
+  if (st->logits) MDC_CHECK_ARG(st->logits_row_offset >= 0 && n + st->logits_row_offset <= st->logits_ld);
+  if (st->confs) MDC_CHECK_ARG((n + 3) / 4 <= st->confs_ld);
+  if (d.vocab > 4096) MDC_CHECK_ARG(!st->confs);
+  cudaStream_t s = (cudaStream_t)stream;
+  const void** gw = m->w + MDC_ENC_GLOBAL_SLOTS + d.enc_depth * MDC_ENC_BLOCK_SLOTS;
+  const float* pos = st->pos_override ? st->pos_override : (const float*)gw[MDC_DEC_POS];
+  const Ws w = carve(d, B, n, workspace);
+  const bool head = st->logits || st->confs;
+  MDC_TRY(run_layers(m, st->tokens, st->tokens_ld, B, n, pos, st->cross_kv, w, KvSink{(bf16*)st->kv_pool, st->page_table, st->pages_per_seq},
+                     head, s));
+  if (!head) return 0;
+  float* lg = st->logits ? st->logits : (float*)((char*)workspace + ws_bytes(d, B, n));
+  const int64_t img_stride = st->logits ? (int64_t)st->logits_ld * d.vocab : (int64_t)n * d.vocab;
+  const int row_offset = st->logits ? st->logits_row_offset : 0;
+  MDC_TRY(launch_head(m, w, B, n, lg, img_stride, row_offset, n, s));
+  if (st->confs) {
+    const int V = d.vocab, n_conf = (n + 3) / 4;
+    int Vp2 = 1; while (Vp2 < V) Vp2 <<= 1;
+    const size_t smem = (size_t)(V + Vp2) * sizeof(float);
+    MDC_ENSURE_SMEM(prefill_conf_kernel, smem);
+    prefill_conf_kernel<<<B * n_conf, mdcsel::SEL_THREADS, smem, s>>>(lg, img_stride, row_offset, V, Vp2, st->top_k, st->top_p, st->confs,
+                                                                       st->confs_ld, n_conf);
+    MDC_LAUNCH_CHECK(m->ctx);
   }
-#define MDC_ADDLN(...)                                                                                        \
-  {                                                                                                           \
-    if (dim == 256) add_layernorm_kernel<1><<<row_blocks, rows_per_block * 32, 0, s>>>(__VA_ARGS__);          \
-    else if (dim == 512) add_layernorm_kernel<2><<<row_blocks, rows_per_block * 32, 0, s>>>(__VA_ARGS__);     \
-    else add_layernorm_kernel<4><<<row_blocks, rows_per_block * 32, 0, s>>>(__VA_ARGS__);                     \
-    MDC_LAUNCH_CHECK(ctx);                                                                                    \
-  }
-  for (int l = 0; l < d.dec_layers; ++l) {
-    const void** lw = lw0 + l * MDC_DEC_LAYER_SLOTS;
-    // self-attention block
-    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.x16, dim, lw[MDC_SA_IN_W], dim, w.qkv, 3 * dim, (const float*)lw[MDC_SA_IN_B], nullptr, 0, (int)R, 3 * dim, dim, s));
-    MDC_ATTN(__half, true, w.qkv, 3 * dim, w.qkv + dim, w.qkv + 2 * dim, 3 * dim, w.kbias, w.o16, dim, n, n, scale_log2e)
-    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.o16, dim, lw[MDC_SA_OUT_W], dim, w.y16, dim, (const float*)lw[MDC_SA_OUT_B], nullptr, 0, (int)R, dim, dim, s));
-    MDC_ADDLN(w.x32, w.y16, (const float*)lw[MDC_LN1_W], (const float*)lw[MDC_LN1_B], w.x16, R, 1e-5f)
-    // cross-attention block: q from rows [0,dim) of the packed in-projection; K/V = the resident cross-K/V of this layer
-    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.x16, dim, lw[MDC_CA_IN_W], dim, w.qkv, dim, (const float*)lw[MDC_CA_IN_B], nullptr, 0, (int)R, dim, dim, s));
-    const bf16* ckv = (const bf16*)cross_kv + (size_t)l * B * S * 2 * dim;
-    MDC_ATTN(bf16, false, w.qkv, dim, ckv, ckv + dim, 2 * dim, nullptr, w.o16, dim, n, S, scale_log2e)
-    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.o16, dim, lw[MDC_CA_OUT_W], dim, w.y16, dim, (const float*)lw[MDC_CA_OUT_B], nullptr, 0, (int)R, dim, dim, s));
-    MDC_ADDLN(w.x32, w.y16, (const float*)lw[MDC_LN2_W], (const float*)lw[MDC_LN2_B], w.x16, R, 1e-5f)
-    // feed-forward block
-    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS_RELU, w.x16, dim, lw[MDC_FF1_W], dim, w.h16, d.dec_ffn, (const float*)lw[MDC_FF1_B], nullptr, 0, (int)R, d.dec_ffn, dim, s));
-    MDC_TRY(mdc_gemm(ctx, MDC_F16, MDC_EPI_BIAS, w.h16, d.dec_ffn, lw[MDC_FF2_W], d.dec_ffn, w.y16, dim, (const float*)lw[MDC_FF2_B], nullptr, 0, (int)R, dim, d.dec_ffn, s));
-    MDC_ADDLN(w.x32, w.y16, (const float*)lw[MDC_LN3_W], (const float*)lw[MDC_LN3_B], w.x16, R, 1e-5f)
-  }
-  if (n_out > 0) {
-    prefill_head_kernel<<<(int)((R + HEAD_ROWS - 1) / HEAD_ROWS), 128, (size_t)HEAD_ROWS * dim * sizeof(float), s>>>(
-        w.x16, (const __half*)gw[MDC_OUT_W], (const float*)gw[MDC_OUT_B], logits, (int64_t)logits_ld * d.vocab, row_offset, n, n_out, d.vocab, R, dim);
-    MDC_LAUNCH_CHECK(ctx);
-  }
-#undef MDC_ATTN
-#undef MDC_ADDLN
   return 0;
 }

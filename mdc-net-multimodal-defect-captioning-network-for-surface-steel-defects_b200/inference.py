@@ -16,7 +16,7 @@ from .model import check_max_len
 
 
 @torch.no_grad()
-def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None, stop_at_eos=False):
+def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None, stop_at_eos=False, prompt=None, prompt_lengths=None):
     """Returns (LongTensor (B, 1+max_len) on CPU, list of ceil(max_len/4) float tensors (B,) on CPU).
 
     `uniforms` (B, max_len) in [0,1) is an optional superset argument: the per-step uniform variates
@@ -24,12 +24,22 @@ def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None, s
     are drawn with torch.rand on the device (the reference uses torch.multinomial, inference_p.py:74).
     `stop_at_eos` (superset argument): stop at tokenizer.EOS_code.  Everything up to and including each
     image's first EOS is bitwise the default result; after it the tokens are PAD and the confidences 0,
-    and decoding ends once every image has finished -- postprocess() returns the same either way."""
+    and decoding ends once every image has finished -- postprocess() returns the same either way.
+    `prompt` int (B,P) / `prompt_lengths` int (B,) (superset arguments): decode each image from BOS followed by its first l_b prompt
+    tokens (default l_b = P), e.g. a caption from tokenizer.caption_prompt() for caption-conditioned detection.  max_len counts the
+    prompt, the output keeps its shape, the prompt columns hold the prompt, and postprocess_with_captions() returns a prompted caption.
+    PAD or tokenizer.EOS_code inside a prompt, tokens outside the vocabulary and lengths outside 0..min(P, max_len) raise ValueError;
+    semantics in EncoderDecoder.generate_tokens and DESIGN.md §3.4d."""
     _check_bos(tokenizer)
     if not hasattr(model, "generate_tokens"):
         raise TypeError("generate() needs the B200 EncoderDecoder; there is no PyTorch fallback path")
     eos = _stop_token(tokenizer) if stop_at_eos else None
-    tokens, confs = model.generate_tokens(x, max_len, top_k=top_k, top_p=top_p, uniforms=uniforms, eos_token=eos)
+    kw = {}
+    if prompt is not None or prompt_lengths is not None:
+        kw = {"prompt": prompt, "prompt_lengths": prompt_lengths}
+        if eos is None:
+            _check_prompt_eos(prompt, prompt_lengths, int(tokenizer.EOS_code))
+    tokens, confs = model.generate_tokens(x, max_len, top_k=top_k, top_p=top_p, uniforms=uniforms, eos_token=eos, **kw)
     host = _to_pinned(tokens, confs)
     torch.cuda.current_stream(tokens.device).synchronize()      # the ONE sync of the whole call
     return _host_result(*host)
@@ -52,6 +62,16 @@ def generate_beam(model, x, tokenizer, max_len=50, num_beams=4, length_penalty=1
     host = _to_pinned(tokens[:, 0], confs[:, 0])
     torch.cuda.current_stream(tokens.device).synchronize()
     return _host_result(*host)
+
+
+def _check_prompt_eos(prompt, prompt_lengths, eos):
+    """The tokenizer's EOS never belongs in a prompt, also without stop_at_eos (generate_tokens checks its own default EOS)."""
+    if prompt is None:
+        return
+    p = torch.as_tensor(prompt).cpu()
+    n = p.shape[-1] if prompt_lengths is None else torch.as_tensor(prompt_lengths).cpu().long().view(-1, 1)
+    if p.dim() == 2 and bool(((p == eos) & (torch.arange(p.shape[-1])[None, :] < n)).any()):
+        raise ValueError(f"a prompt may not hold EOS ({eos})")
 
 
 def _to_pinned(tokens, confs):

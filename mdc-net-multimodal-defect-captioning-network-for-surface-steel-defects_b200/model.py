@@ -296,10 +296,14 @@ class Engine:
 
     def decode(self, cross_kv, tokens, t_begin, t_end, *, max_tokens, forced, logits=None, logits_row_offset=0,
                confs=None, uniforms=None, top_k=0, top_p=1.0, pos_override=None, x_override=None, kv=None, scratch=None,
-               images_per_cluster=None, ctas_per_sm=None, per_op_kernels=None, eos_token=None):
+               images_per_cluster=None, ctas_per_sm=None, per_op_kernels=None, eos_token=None, prompt_len=None, prefill=0,
+               prefill_ws=None):
         """Runs decode steps [t_begin, t_end) back to back on the current stream (no host sync).  `eos_token` (free-running only): stop
         at that token -- after an image's first EOS its token columns are PAD and its confidences 0, and decoding ends once every image
-        has finished (mdc_decode_state.stop_at_eos)."""
+        has finished (mdc_decode_state.stop_at_eos).  `prompt_len` (free-running only): int32 (B,) device tensor; row b's columns
+        1..prompt_len[b] of `tokens` hold its prompt, which the prompt steps keep (mdc_decode_state.prompt_len).  `prefill` = n > 0 (with
+        t_begin 0 and `prefill_ws`, mdc_decode_prefill_workspace_bytes): steps [0, n) run as one all-positions pass
+        (mdc_decode_prefill_steps), the rest step by step."""
         d = self.dims
         B = tokens.shape[0]
         assert tokens.dtype == torch.int32 and tokens.is_contiguous()
@@ -334,7 +338,15 @@ class Engine:
         st.per_op_kernels = int(opt["per_op_kernels"] if per_op_kernels is None else per_op_kernels)
         if eos_token is not None:
             st.stop_at_eos, st.eos_token = 1, int(eos_token)
+        if prompt_len is not None:
+            assert prompt_len.dtype == torch.int32 and prompt_len.shape == (B,)
+            st.prompt_len = prompt_len.data_ptr()
         with torch.cuda.device(self.device):
+            if prefill:
+                assert t_begin == 0 and prefill <= t_end
+                L.check(self.lib.mdc_decode_prefill_steps(self.handle, C.byref(st), int(prefill), L.ptr(prefill_ws), prefill_ws.numel(),
+                                                          L.stream_ptr(self.device)))
+                t_begin = int(prefill)
             L.check(self.lib.mdc_decode_steps(self.handle, C.byref(st), t_begin, t_end, L.stream_ptr(self.device)))
         return kv, scratch
 
@@ -542,12 +554,21 @@ class EncoderDecoder(nn.Module, _EngineOwner):
 
     @torch.no_grad()
     def generate_tokens(self, image, max_new_tokens, top_k=0, top_p=1.0, uniforms=None, return_logits=False, use_graph=None,
-                        eos_token=None):
+                        eos_token=None, prompt=None, prompt_lengths=None):
         """Returns (tokens int32 (B,1+T) on device, confs f32 (B,ceil(T/4)) on device[, logits (B,T,V)]).
-        The whole call (encoder, cross-K/V, T decode steps) is one CUDA graph replay per (B, T, sampler, stop token) shape.
+        The whole call (encoder, cross-K/V, T decode steps) is one CUDA graph replay per (B, T, sampler, stop token, prompt) shape.
         `eos_token`: stop at that token (superset argument).  Up to and including an image's first EOS the result is bitwise the
         no-stop result; after it the tokens are PAD and the confidences 0, and decoding ends once every image has finished.  Not
-        with `return_logits` (steps that do not run have no logits; predict()/forward() serve that use)."""
+        with `return_logits` (steps that do not run have no logits; predict()/forward() serve that use).
+        `prompt` int (B,P) and `prompt_lengths` int (B,), each in 0..P (default P): prompted decoding (superset arguments).  Row b
+        decodes from BOS followed by prompt[b, :l_b]: token columns 1..l_b keep the prompt, the conf column of a prompt step t (t % 4
+        == 0) holds the max probability of the (filtered) distribution at that step, and steps t >= l_b select and sample as without a
+        prompt.  T counts the prompt (l_b <= T).  With a prompt equal to the first l_b tokens an unprompted call returns, the result is
+        bitwise that call's.  PAD or EOS (`eos_token`, default the tokenizer's 301) among the first l_b tokens, tokens outside the
+        vocabulary, l_b outside 0..P or above T are rejected with ValueError.  The prompt and its lengths are read on the host:
+        device tensors cost one synchronisation.  Where the all-positions prefill covers the model, the first min(l_b) steps run as one
+        pass when min(l_b) >= PREFILL_MIN_STEPS (not under decode_options(prefill=False)); its results equal the step path's up to
+        rounding."""
         eng = self._engine(image.device if image.is_cuda else None)
         B, T = image.shape[0], int(max_new_tokens)
         check_max_len(T, eng.dims.max_pos)
@@ -555,10 +576,21 @@ class EncoderDecoder(nn.Module, _EngineOwner):
             if return_logits:
                 raise ValueError("return_logits=True cannot be combined with eos_token: steps that do not run have no logits")
             eos_token = check_eos_token(eos_token, eng.dims.vocab)
-        plan = self._plan(eng, (id(eng), B, T, int(top_k), float(top_p), bool(return_logits), eos_token), use_graph,
-                          lambda graph: GenerationPlan(eng, B, T, top_k, top_p, return_logits, graph, eos_token=eos_token))
+        P = n_prefill = 0
+        if prompt is not None or prompt_lengths is not None:
+            prompt, lengths = check_prompt(prompt, prompt_lengths, B, T, eng.dims.vocab, DEFAULT_EOS if eos_token is None else eos_token)
+            P = prompt.shape[1]
+            n = int(lengths.min())
+            if (n >= PREFILL_MIN_STEPS and _DECODE_OPTIONS["prefill"]
+                    and eng.lib.mdc_decode_prefill_workspace_bytes(eng.handle, B, n)):
+                n_prefill = n
+        plan = self._plan(eng, (id(eng), B, T, int(top_k), float(top_p), bool(return_logits), eos_token, P, n_prefill), use_graph,
+                          lambda graph: GenerationPlan(eng, B, T, top_k, top_p, return_logits, graph, eos_token=eos_token,
+                                                       prompt_width=P, prefill=n_prefill))
         if plan.uniforms is not None and uniforms is None:
             uniforms = torch.rand((B, T), dtype=torch.float32, device=eng.device)
+        if P:
+            plan.set_prompt(prompt, lengths)
         tokens, confs, logits = plan.run(image, uniforms)
         if return_logits:
             return tokens.clone(), confs.clone(), logits.clone()
@@ -589,6 +621,46 @@ def check_max_len(T, max_pos, error=RuntimeError):
     if T > max_pos:
         raise error(f"max_len {T} exceeds CFG.max_len-1 = {max_pos}: the positional table has no more rows "
                     "(reference fails at model.py:93, Q6)")
+
+
+# EOS of the reference tokenizer (data_processing.py:235-239): never allowed inside a prompt
+DEFAULT_EOS = 301
+# prompted generation: the first min(l_b) steps run as one all-positions prefill pass from this many prompt steps on (DESIGN.md §3.4d)
+PREFILL_MIN_STEPS = 6
+
+
+def check_prompt(prompt, prompt_lengths, B, T, vocab, eos_token):
+    """Host copies of a generation prompt, checked: (prompt int32 (B, min(P, T)) with PAD after each row's length, lengths int32 (B,))."""
+    if prompt is None:
+        raise ValueError("prompt_lengths needs a prompt")
+    prompt = torch.as_tensor(prompt).detach().cpu()
+    if prompt.dim() != 2 or prompt.shape[0] != B:
+        raise ValueError(f"prompt must be (B, P) with B = {B} images, got {tuple(prompt.shape)}")
+    if prompt.dtype.is_floating_point or prompt.dtype == torch.bool:
+        raise ValueError("prompt must hold integer token ids")
+    P = prompt.shape[1]
+    if prompt_lengths is None:
+        lengths = torch.full((B,), P, dtype=torch.int64)
+    else:
+        lengths = torch.as_tensor(prompt_lengths).detach().cpu()
+        if lengths.shape != (B,) or lengths.dtype.is_floating_point or lengths.dtype == torch.bool:
+            raise ValueError(f"prompt_lengths must be {B} integers")
+        lengths = lengths.long()
+    if bool((lengths < 0).any()) or bool((lengths > P).any()):
+        raise ValueError(f"prompt_lengths must lie in 0..{P} (the prompt width), got {lengths.tolist()}")
+    if bool((lengths > T).any()):
+        raise ValueError(f"a prompt length exceeds max_len {T}: max_len counts the prompt")
+    prompt = prompt.long()
+    live = torch.arange(P)[None, :] < lengths[:, None]
+    bad = live & ((prompt < 0) | (prompt >= vocab))
+    if bool(bad.any()):
+        raise ValueError(f"prompt tokens must lie in [0, {vocab}): row {int(bad.any(1).nonzero()[0])}")
+    special = live & ((prompt == int(CFG.pad_idx)) | (prompt == int(eos_token)))
+    if bool(special.any()):
+        raise ValueError(f"a prompt may not hold PAD ({int(CFG.pad_idx)}) or EOS ({int(eos_token)}): row {int(special.any(1).nonzero()[0])}")
+    W = min(P, T)
+    out = torch.where(live, prompt, torch.full_like(prompt, int(CFG.pad_idx)))[:, :W]
+    return out.to(torch.int32).contiguous(), lengths.to(torch.int32)
 
 
 def check_eos_token(eos_token, vocab):
@@ -682,7 +754,7 @@ class GenerationPlan(_Plan):
     the others come from decode_options."""
 
     def __init__(self, eng, B, T, top_k=0, top_p=1.0, want_logits=False, use_graph=True, split=False, eos_token=None,
-                 images_per_cluster=None, ctas_per_sm=None):
+                 images_per_cluster=None, ctas_per_sm=None, prompt_width=0, prefill=0):
         super().__init__(eng, B, T, B)
         d, dev = eng.dims, eng.device
         self.top_k, self.top_p, self.eos_token = int(top_k), float(top_p), eos_token
@@ -690,6 +762,15 @@ class GenerationPlan(_Plan):
         self.logits = torch.empty((B, T, d.vocab), dtype=torch.float32, device=dev) if want_logits else None
         if top_k != 0 or top_p != 1:
             self.uniforms = torch.zeros((B, T), dtype=torch.float32, device=dev)
+        # prompted plans: the prompt (B, prompt_width) and its lengths are static buffers set before each run (set_prompt); with
+        # `prefill` = n the first n steps run as one all-positions pass (every row's prompt covers them)
+        self.prompt = self.prompt_len = self.prefill_ws = None
+        self.prefill = int(prefill)
+        if prompt_width:
+            self.prompt = torch.full((B, prompt_width), int(CFG.pad_idx), dtype=torch.int32, device=dev)
+            self.prompt_len = torch.zeros(B, dtype=torch.int32, device=dev)
+        if self.prefill:
+            self.prefill_ws = torch.empty(eng.lib.mdc_decode_prefill_workspace_bytes(eng.handle, B, self.prefill), dtype=torch.uint8, device=dev)
         if split:
             self.enc_graph, self.dec_graph = capture_graphs(dev, self._launch_encode, self._launch_decode)
         elif use_graph:
@@ -704,11 +785,20 @@ class GenerationPlan(_Plan):
         self._encode()
         L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory), self.B, L.ptr(self.ckv), L.stream_ptr(eng.device)))
 
+    def set_prompt(self, prompt, lengths):
+        """Host (or device) prompt int32 (B, prompt_width), PAD past each row's length, and lengths int32 (B,), as check_prompt returns them."""
+        with torch.cuda.device(self.eng.device):
+            self.prompt.copy_(prompt, non_blocking=True)
+            self.prompt_len.copy_(lengths, non_blocking=True)
+
     def _launch_decode(self):
         self._reset_tokens()
+        if self.prompt is not None:
+            self.tokens[:, 1:1 + self.prompt.shape[1]].copy_(self.prompt)
         self.eng.decode(self.ckv, self.tokens, 0, self.T, max_tokens=self.T, forced=False, logits=self.logits, logits_row_offset=0,
                         confs=self.confs, uniforms=self.uniforms, top_k=self.top_k, top_p=self.top_p, kv=self.kv, scratch=self.scratch,
-                        images_per_cluster=self.images_per_cluster, ctas_per_sm=self.ctas_per_sm, eos_token=self.eos_token)
+                        images_per_cluster=self.images_per_cluster, ctas_per_sm=self.ctas_per_sm, eos_token=self.eos_token,
+                        prompt_len=self.prompt_len, prefill=self.prefill, prefill_ws=self.prefill_ws)
 
     def _outputs(self):
         return self.tokens, self.confs, self.logits

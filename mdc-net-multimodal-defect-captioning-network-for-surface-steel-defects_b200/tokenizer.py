@@ -112,6 +112,23 @@ class Tokenizer:
         boxes, _, counts, _, _ = self._run(L.TOK_BBOXES, torch.as_tensor(pred_seq), False)
         return boxes, counts
 
+    def caption_prompt(self, captions):
+        """Prompts for caption-conditioned generation (generate(..., prompt=, prompt_lengths=)): a list of B caption-word-id lists ->
+        (prompt LongTensor (B, P) with row b = [CAPTION_START, *captions[b], CAPTION_END] padded with PAD_code, lengths LongTensor (B,)),
+        P the longest row.  Ids must be caption words, not special tokens."""
+        rows = [[self.CAPTION_START, *[int(i) for i in ids], self.CAPTION_END] for ids in captions]
+        if not rows:
+            raise ValueError("caption_prompt needs at least one caption")
+        special = {self.BOS_code, self.EOS_code, self.PAD_code, self.CAPTION_START, self.CAPTION_END}
+        for b, r in enumerate(rows):
+            if any(i in special or not 0 <= i < self.vocab_size for i in r[1:-1]):
+                raise ValueError(f"caption {b} holds a special or out-of-vocabulary token id")
+        P = max(len(r) for r in rows)
+        prompt = torch.full((len(rows), P), self.PAD_code, dtype=torch.long)
+        for b, r in enumerate(rows):
+            prompt[b, :len(r)] = torch.tensor(r, dtype=torch.long)
+        return prompt, torch.tensor([len(r) for r in rows], dtype=torch.long)
+
     def decode_batch(self, tokens):
         """Batched Tokenizer.decode (data_processing.py:317-391): device tensors (labels (B,N), boxes (B,N,4), counts (B,),
         caption ids (B,L) PAD-padded, caption lengths (B,), -1 = no caption markers)."""
