@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MDC_ABI_VERSION 9
+#define MDC_ABI_VERSION 10
 
 /* element types of activations / weights.  MDC_F16 (IEEE half) is the type of the decode-loop weights under precision MDC_BF16
  * (see the weight table) and of mdc_gemm's fp16 mode. */
@@ -306,8 +306,19 @@ int mdc_decode_prefill_steps(mdc_model* m, const mdc_decode_state* st, int n, vo
  *   own_pages    int32 [B*K, pages_per_seq] the rows' initial, distinct pages (never written)
  *   scores f32 [B*K], finish_step int32 [B*K]; token_logprobs f32 [B*K, token_logprobs_ld] and confs f32 [B*K, confs_ld], either NULL
  *   workspace    mdc_beam_workspace_bytes() (0 for K outside 1..16)
- * mdc_beam_finalize: normalised score s / len^length_penalty, len = f + 1 for a finished beam and T otherwise; order_out int32 [B, K]
- * lists each image's beam indices by normalised score, descending (ties: lower index first), norm_scores_out f32 [B, K] in that order.
+ * Prompted beam search (prompt_len int32 [B], NULL = no prompt): columns 1..l_b (l_b = prompt_len[b]) of all K token rows of image b
+ * hold its prompt before step 0, and l_b <= T - 1 (at least one free step; the host layer checks it).  Step t with t + 1 <= l_b is a
+ * prompt step of image b: its decode window reads column t as any step, and mdc_beam_step selects and reorders nothing for that image
+ * -- beam 0 stays the only running beam at score 0, beams 1..K-1 stay at -inf, column t+1 keeps the prompt token, beam 0's log-prob
+ * column t is 0 and, when t % 4 == 0, its conf column t/4 receives the max probability 1 / sum_u exp(l_u - m) of its distribution, as
+ * a greedy prompt step writes it.  Prompt and free images mix within one step; each image's CTA decides alone.  The first free step
+ * t = l_b is step 0 of an unprompted search: beam 0 is the only parent and its children take its KV through the reorder above.  Scores
+ * count generated tokens only and stay the f32 sums of the per-token log-prob rows (prompt entries are 0).  With every l_b = 0 the
+ * results are bitwise those of prompt_len = NULL.  Steps [0, n) with n <= min(l_b) may instead run as one mdc_decode_prefill_steps pass
+ * over the B*K rows (confs set, no logits); the beam steps then start at t = n and the caller zeroes the log-prob columns t < n.
+ * mdc_beam_finalize: normalised score s / len^length_penalty over the generated tokens, len = f + 1 - l_b for a finished beam and
+ * T - l_b otherwise (l_b = 0 without a prompt); order_out int32 [B, K] lists each image's beam indices by normalised score, descending
+ * (ties: lower index first), norm_scores_out f32 [B, K] in that order.
  * Rejected with a message: K outside 1..16 or above the vocabulary, vocab > 4096, eos_token outside the vocabulary, a t past the
  * positional table, the token columns or the pages, a short workspace. */
 typedef struct mdc_beam_state {
@@ -319,6 +330,7 @@ typedef struct mdc_beam_state {
   float* confs; int32_t confs_ld;
   int32_t eos_token;
   void* workspace; size_t workspace_bytes;
+  const int32_t* prompt_len;        /* int32 [B] or NULL (= no prompt): see "Prompted beam search" above */
 } mdc_beam_state;
 
 size_t mdc_beam_workspace_bytes(const mdc_model* m, int B, int K);

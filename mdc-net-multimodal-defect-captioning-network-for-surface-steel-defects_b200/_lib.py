@@ -75,6 +75,7 @@ class BeamState(C.Structure):
         ("confs", C.c_void_p), ("confs_ld", C.c_int32),
         ("eos_token", C.c_int32),
         ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t),
+        ("prompt_len", C.c_void_p),
     ]
 
 

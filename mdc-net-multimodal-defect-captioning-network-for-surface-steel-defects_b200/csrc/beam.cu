@@ -3,10 +3,13 @@
 //   beam_select_kernel   one CTA per image: log-softmax of each running beam's row, each beam's K best candidates (a warp per beam),
 //                        the merge of the K*K candidates, then the reorder of token rows, scores, finish steps, per-token histories and
 //                        the live page table (parents staged through the workspace first: a destination row can be another child's
-//                        parent).
+//                        parent).  At a prompt step of its image (t + 1 <= prompt_len[b]) the CTA only records beam 0's zero log-prob
+//                        and, when t % 4 == 0, its max probability, and marks every row as its own parent: nothing is selected or moved.
 //   beam_kv_copy_kernel  copy-on-write of the partly filled KV page, twice: parents' valid token slots -> workspace, workspace -> each
-//                        child's own page.  Skipped when the step filled its page (the page is then shared through the table).
-//   beam_finalize_kernel length-normalised scores and the best-first order of each image's beams.
+//                        child's own page.  Skipped when the step filled its page (the page is then shared through the table), and
+//                        for rows that are their own parent (kept places, prompt steps).
+//   beam_finalize_kernel length-normalised scores (the length counts generated tokens only) and the best-first order of each image's
+//                        beams.
 #include "common.cuh"
 
 namespace {
@@ -19,6 +22,7 @@ struct BeamArgs {
   int B, K, V, pad, eos, pt, t, max_pos;
   const float* logits; int64_t logits_ld;
   int32_t* tokens; int32_t tokens_ld;
+  const int32_t* prompt_len;           // int32 [B] or NULL
   int32_t* live; const int32_t* own; int32_t pps;
   float* scores; int32_t* finish;
   float* lps; int32_t lps_ld;
@@ -57,6 +61,23 @@ __global__ void __launch_bounds__(BEAM_SEL_THREADS) beam_select_kernel(BeamArgs 
   const int b = blockIdx.x, K = a.K, t = a.t, tid = threadIdx.x;
   const int warp = tid >> 5, lane = tid & 31;
   const int64_t r0 = (int64_t)b * K;
+  if (a.prompt_len && t < a.prompt_len[b]) {       // a prompt step of this image: column t+1 already holds the prompt token
+    if (warp == 0) {
+      if (a.confs && t % 4 == 0) {                  // beam 0's max probability 1 / sum exp(l - m), the quantity a greedy step reports
+        const float* row = a.logits + r0 * a.logits_ld;
+        float m = -INFINITY;
+        for (int v = lane; v < a.V; v += 32) m = fmaxf(m, row[v]);
+        m = warp_max(m);
+        float sum = 0.f;
+        for (int v = lane; v < a.V; v += 32) sum += expf(row[v] - m);
+        sum = warp_sum(sum);
+        if (lane == 0) a.confs[r0 * a.confs_ld + t / 4] = 1.f / sum;
+      }
+      if (lane == 0 && a.lps) a.lps[r0 * a.lps_ld + t] = 0.f;
+    }
+    if (tid < K) a.parent[r0 + tid] = (int32_t)(r0 + tid);   // the KV copy that follows moves nothing
+    return;
+  }
   if (tid < K) s_win[tid] = 0;        // fewer than K candidates only from a caller's state with no live beam: stay in bounds
 
   // 1. each beam's K best candidates, best first (a warp per beam)
@@ -186,14 +207,16 @@ __global__ void __launch_bounds__(BEAM_COPY_THREADS) beam_kv_copy_kernel(const i
   }
 }
 
-__global__ void beam_finalize_kernel(const float* __restrict__ scores, const int32_t* __restrict__ finish, int K, int T, float alpha,
-                                     int32_t* __restrict__ order_out, float* __restrict__ norm_out) {
+__global__ void beam_finalize_kernel(const float* __restrict__ scores, const int32_t* __restrict__ finish,
+                                     const int32_t* __restrict__ prompt_len, int K, int T, float alpha, int32_t* __restrict__ order_out,
+                                     float* __restrict__ norm_out) {
   __shared__ float s_norm[BEAM_MAX_K];
   const int b = blockIdx.x, k = threadIdx.x;
   float nk = 0.f;
   if (k < K) {
     const int f = finish[(int64_t)b * K + k];
-    const float len = (float)(f >= 0 ? f + 1 : T);
+    const int lb = prompt_len ? prompt_len[b] : 0;  // generated tokens only: the prompt columns are not part of the beam's length
+    const float len = (float)((f >= 0 ? f + 1 : T) - lb);
     nk = scores[(int64_t)b * K + k] / powf(len, alpha);
     s_norm[k] = nk;
   }
@@ -245,6 +268,7 @@ extern "C" int mdc_beam_step(mdc_model* m, const mdc_beam_state* st, const float
   a.B = st->B; a.K = st->K; a.V = d.vocab; a.pad = d.pad_idx; a.eos = st->eos_token; a.pt = d.page_tokens; a.t = t; a.max_pos = d.max_pos;
   a.logits = logits; a.logits_ld = logits_ld;
   a.tokens = st->tokens; a.tokens_ld = st->tokens_ld;
+  a.prompt_len = st->prompt_len;
   a.live = st->page_table; a.own = st->own_pages; a.pps = st->pages_per_seq;
   a.scores = st->scores; a.finish = st->finish_step;
   a.lps = st->token_logprobs; a.lps_ld = st->token_logprobs_ld;
@@ -272,8 +296,8 @@ extern "C" int mdc_beam_finalize(mdc_model* m, const mdc_beam_state* st, int T, 
   MDC_TRY(beam_check_state(m, st));
   MDC_CHECK_ARG(order_out && norm_scores_out && T >= 1 && T <= m->d.max_pos);
   MDC_CHECK_DEVICE(m->ctx);
-  beam_finalize_kernel<<<st->B, 32, 0, (cudaStream_t)stream>>>(st->scores, st->finish_step, st->K, T, length_penalty, order_out,
-                                                                norm_scores_out);
+  beam_finalize_kernel<<<st->B, 32, 0, (cudaStream_t)stream>>>(st->scores, st->finish_step, st->prompt_len, st->K, T, length_penalty,
+                                                                order_out, norm_scores_out);
   MDC_LAUNCH_CHECK(m->ctx);
   return 0;
 }

@@ -46,11 +46,15 @@ def generate(model, x, tokenizer, max_len=50, top_k=0, top_p=1, uniforms=None, s
 
 
 @torch.no_grad()
-def generate_beam(model, x, tokenizer, max_len=50, num_beams=4, length_penalty=1.0):
+def generate_beam(model, x, tokenizer, max_len=50, num_beams=4, length_penalty=1.0, prompt=None, prompt_lengths=None):
     """Beam search (superset function): returns exactly what generate() returns -- LongTensor (B, 1+max_len) and a list of
     ceil(max_len/4) (B,) confidence tensors, on CPU -- for each image's best beam by score / len^length_penalty, so that postprocess()
     and postprocess_with_captions() read it unchanged.  Beams end at tokenizer.EOS_code (the tokens after it are PAD, the confidences 0);
-    there is no early exit once every beam has ended, and no sampling inside beams.  Semantics: DESIGN.md §3.4c."""
+    there is no early exit once every beam has ended, and no sampling inside beams.
+    `prompt` int (B,P) / `prompt_lengths` int (B,) (superset arguments): every beam of image b starts from BOS followed by its first
+    l_b prompt tokens (default l_b = P), e.g. a caption from tokenizer.caption_prompt(); the search starts after the prompt, and scores
+    and the length normalisation count generated tokens only.  max_len counts the prompt and must leave one free step (l_b <= max_len
+    - 1); PAD or tokenizer.EOS_code inside a prompt and tokens outside the vocabulary raise ValueError.  Semantics: DESIGN.md §3.4c."""
     _check_bos(tokenizer)
     if not hasattr(model, "generate_beam_tokens"):
         raise TypeError("generate_beam() needs the B200 EncoderDecoder; there is no PyTorch fallback path")
@@ -58,7 +62,8 @@ def generate_beam(model, x, tokenizer, max_len=50, num_beams=4, length_penalty=1
     if not x.is_cuda:
         raise ValueError("generate_beam() takes the images on a CUDA device; there is no CPU fallback")
     eos = _stop_token(tokenizer)
-    tokens, _, _, confs = model.generate_beam_tokens(x, max_len, num_beams, length_penalty, eos_token=eos)
+    tokens, _, _, confs = model.generate_beam_tokens(x, max_len, num_beams, length_penalty, eos_token=eos, prompt=prompt,
+                                                     prompt_lengths=prompt_lengths)
     host = _to_pinned(tokens[:, 0], confs[:, 0])
     torch.cuda.current_stream(tokens.device).synchronize()
     return _host_result(*host)

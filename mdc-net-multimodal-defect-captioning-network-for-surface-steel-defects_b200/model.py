@@ -597,12 +597,22 @@ class EncoderDecoder(nn.Module, _EngineOwner):
         return tokens.clone(), confs.clone()
 
     @torch.no_grad()
-    def generate_beam_tokens(self, image, max_new_tokens, num_beams, length_penalty=1.0, *, eos_token, use_graph=None):
+    def generate_beam_tokens(self, image, max_new_tokens, num_beams, length_penalty=1.0, *, eos_token, use_graph=None, prompt=None,
+                             prompt_lengths=None):
         """Beam search (superset method; semantics in include/mdc_b200.h and DESIGN.md §3.4c).  Returns, on the device, each image's
         beams best first by length-normalised score: tokens int32 (B,K,1+T), normalised scores f32 (B,K), per-token log-probs f32
         (B,K,T) and confidences f32 (B,K,ceil(T/4)).  Tokens after a beam's EOS are PAD, with log-prob and confidence 0.  The whole
         call (encoder, cross-K/V for the B*K rows, T x (one teacher-forced decode step + one beam step), the final ordering) is one
-        CUDA graph replay per (B, T, K, length penalty, stop token) shape."""
+        CUDA graph replay per (B, T, K, length penalty, stop token, prompt) shape.
+        `prompt` int (B,P) and `prompt_lengths` int (B,), each in 0..P (default P): every beam of image b starts from BOS followed by
+        prompt[b, :l_b].  Steps t < l_b select nothing: the prompt columns are kept, their log-probs are 0, and the conf column of such a
+        step (t % 4 == 0) holds the max probability of beam 0's distribution.  Step l_b is the first beam step.  Scores and the length
+        normalisation count generated tokens only (len = f + 1 - l_b for a beam that ended at step f, T - l_b otherwise).  T counts the
+        prompt, and a beam search needs a free step: l_b <= T - 1.  PAD or `eos_token` among the first l_b tokens, tokens outside the
+        vocabulary and lengths outside 0..min(P, T - 1) raise ValueError before any launch; the prompt is read on the host.  With every
+        l_b = 0 the result is bitwise the unprompted one; with K = 1 the tokens are prompted greedy generate_tokens'.  Where the
+        all-positions prefill covers the model, the first min(l_b) steps of the B*K rows run as one pass when min(l_b) >=
+        PREFILL_MIN_STEPS (not under decode_options(prefill=False)); its results equal the step path's up to rounding."""
         eng = self._engine(image.device if image.is_cuda else None)
         B, T, K = image.shape[0], int(max_new_tokens), int(num_beams)
         if not 1 <= K <= 16:
@@ -611,8 +621,18 @@ class EncoderDecoder(nn.Module, _EngineOwner):
             raise RuntimeError(f"max_len {T}: beam search needs at least one new token")
         check_max_len(T, eng.dims.max_pos)
         eos_token = check_eos_token(eos_token, eng.dims.vocab)
-        plan = self._plan(eng, ("beam", id(eng), B, T, K, float(length_penalty), eos_token), use_graph,
-                          lambda graph: BeamPlan(eng, B, T, K, length_penalty, eos_token, graph))
+        P = n_prefill = 0
+        if prompt is not None or prompt_lengths is not None:
+            prompt, lengths = check_beam_prompt(prompt, prompt_lengths, B, T, eng.dims.vocab, eos_token)
+            P = prompt.shape[1]
+            n = int(lengths.min())
+            if (n >= PREFILL_MIN_STEPS and _DECODE_OPTIONS["prefill"]
+                    and eng.lib.mdc_decode_prefill_workspace_bytes(eng.handle, B * K, n)):
+                n_prefill = n
+        plan = self._plan(eng, ("beam", id(eng), B, T, K, float(length_penalty), eos_token, P, n_prefill), use_graph,
+                          lambda graph: BeamPlan(eng, B, T, K, length_penalty, eos_token, graph, prompt_width=P, prefill=n_prefill))
+        if P:
+            plan.set_prompt(prompt, lengths)
         return tuple(o.clone() for o in plan.run(image))
 
 
@@ -661,6 +681,14 @@ def check_prompt(prompt, prompt_lengths, B, T, vocab, eos_token):
     W = min(P, T)
     out = torch.where(live, prompt, torch.full_like(prompt, int(CFG.pad_idx)))[:, :W]
     return out.to(torch.int32).contiguous(), lengths.to(torch.int32)
+
+
+def check_beam_prompt(prompt, prompt_lengths, B, T, vocab, eos_token):
+    """check_prompt, plus the rule of beam search: every prompt leaves at least one step to search (l_b <= T - 1)."""
+    prompt, lengths = check_prompt(prompt, prompt_lengths, B, T, vocab, eos_token)
+    if bool((lengths > T - 1).any()):
+        raise ValueError(f"a prompt length exceeds max_len - 1 = {T - 1}: beam search needs at least one step after the prompt")
+    return prompt, lengths
 
 
 def check_eos_token(eos_token, vocab):
@@ -746,6 +774,26 @@ class _Plan:
         self.tokens.fill_(int(CFG.pad_idx))
         self.tokens[:, 0].fill_(int(CFG.bos_idx))
 
+    def _init_prompt(self, width, prefill):
+        """Prompted plans: the prompt (B, width) and its lengths are static buffers set before each run (set_prompt); with `prefill` = n
+        the first n steps of every decoded row run as one all-positions pass (every row's prompt covers them)."""
+        eng, dev = self.eng, self.eng.device
+        self.prompt = self.prompt_len = self.prefill_ws = None
+        self.prefill = int(prefill)
+        if width:
+            self.prompt = torch.full((self.B, width), int(CFG.pad_idx), dtype=torch.int32, device=dev)
+            self.prompt_len = torch.zeros(self.B, dtype=torch.int32, device=dev)
+        if self.prefill:
+            rows = self.tokens.shape[0]
+            self.prefill_ws = torch.empty(eng.lib.mdc_decode_prefill_workspace_bytes(eng.handle, rows, self.prefill), dtype=torch.uint8,
+                                          device=dev)
+
+    def set_prompt(self, prompt, lengths):
+        """Host (or device) prompt int32 (B, prompt width), PAD past each row's length, and lengths int32 (B,), as check_prompt returns them."""
+        with torch.cuda.device(self.eng.device):
+            self.prompt.copy_(prompt, non_blocking=True)
+            self.prompt_len.copy_(lengths, non_blocking=True)
+
 
 class GenerationPlan(_Plan):
     """One (batch, new tokens, sampler, stop token) shape: encoder -> memory -> cross-K/V -> T decode steps.  With `use_graph` the
@@ -762,15 +810,7 @@ class GenerationPlan(_Plan):
         self.logits = torch.empty((B, T, d.vocab), dtype=torch.float32, device=dev) if want_logits else None
         if top_k != 0 or top_p != 1:
             self.uniforms = torch.zeros((B, T), dtype=torch.float32, device=dev)
-        # prompted plans: the prompt (B, prompt_width) and its lengths are static buffers set before each run (set_prompt); with
-        # `prefill` = n the first n steps run as one all-positions pass (every row's prompt covers them)
-        self.prompt = self.prompt_len = self.prefill_ws = None
-        self.prefill = int(prefill)
-        if prompt_width:
-            self.prompt = torch.full((B, prompt_width), int(CFG.pad_idx), dtype=torch.int32, device=dev)
-            self.prompt_len = torch.zeros(B, dtype=torch.int32, device=dev)
-        if self.prefill:
-            self.prefill_ws = torch.empty(eng.lib.mdc_decode_prefill_workspace_bytes(eng.handle, B, self.prefill), dtype=torch.uint8, device=dev)
+        self._init_prompt(prompt_width, prefill)
         if split:
             self.enc_graph, self.dec_graph = capture_graphs(dev, self._launch_encode, self._launch_decode)
         elif use_graph:
@@ -784,12 +824,6 @@ class GenerationPlan(_Plan):
         eng = self.eng
         self._encode()
         L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory), self.B, L.ptr(self.ckv), L.stream_ptr(eng.device)))
-
-    def set_prompt(self, prompt, lengths):
-        """Host (or device) prompt int32 (B, prompt_width), PAD past each row's length, and lengths int32 (B,), as check_prompt returns them."""
-        with torch.cuda.device(self.eng.device):
-            self.prompt.copy_(prompt, non_blocking=True)
-            self.prompt_len.copy_(lengths, non_blocking=True)
 
     def _launch_decode(self):
         self._reset_tokens()
@@ -808,9 +842,11 @@ class BeamPlan(_Plan):
     """One beam-search shape (B images, T new tokens, K beams): encoder -> memory repeated K times -> cross-K/V of the B*K rows ->
     T x (teacher-forced decode step t, mdc_beam_step t) -> mdc_beam_finalize, captured as one CUDA graph with `use_graph`.
     The KV pool holds B*K rows of distinct pages (`own`, never rewritten); `kv.page_table` is the live table the decode kernels read,
-    reset to `own` at the start of every run."""
+    reset to `own` at the start of every run.  Prompted plans (`prompt_width` > 0) copy each image's prompt into all K of its token rows
+    after the reset; with `prefill` = n, steps [0, n) of the B*K rows run as one all-positions pass (mdc_decode_prefill_steps) and the
+    decode windows and beam steps start at t = n."""
 
-    def __init__(self, eng, B, T, K, length_penalty, eos_token, use_graph):
+    def __init__(self, eng, B, T, K, length_penalty, eos_token, use_graph, prompt_width=0, prefill=0):
         super().__init__(eng, B, T, B * K)
         d, dev, BK = eng.dims, eng.device, B * K
         self.K, self.length_penalty, self.eos_token = K, float(length_penalty), int(eos_token)
@@ -836,6 +872,9 @@ class BeamPlan(_Plan):
         st.confs, st.confs_ld = self.confs.data_ptr(), self.confs.shape[1]
         st.eos_token = self.eos_token
         st.workspace, st.workspace_bytes = self.beam_ws.data_ptr(), self.beam_ws.numel()
+        self._init_prompt(prompt_width, prefill)
+        if self.prompt is not None:
+            st.prompt_len = self.prompt_len.data_ptr()
         self.state = st
         if use_graph:
             [self.graph] = capture_graphs(dev, self._launch)
@@ -848,11 +887,18 @@ class BeamPlan(_Plan):
         self.memory_k.copy_(self.memory[:, None].expand_as(self.memory_k))
         L.check(eng.lib.mdc_cross_kv_build(eng.handle, L.ptr(self.memory_k), B * K, L.ptr(self.ckv), s))
         self._reset_tokens()
+        if self.prompt is not None:
+            P = self.prompt.shape[1]
+            self.tokens.view(B, K, T + 1)[:, :, 1:1 + P].copy_(self.prompt[:, None].expand(B, K, P))
+            self.lps.zero_()              # the prefill skips the beam steps t < n, which would otherwise write log-prob columns t
         self.kv.page_table.copy_(self.own)
         self.scores.copy_(self.score0.view(-1))
         self.finish.fill_(-1)
+        if self.prefill:
+            eng.decode(self.ckv, self.tokens, 0, self.prefill, max_tokens=T, forced=False, confs=self.confs, kv=self.kv,
+                       scratch=self.scratch, prefill=self.prefill, prefill_ws=self.prefill_ws)
         row_bytes = d.vocab * self.logits.element_size()
-        for t in range(T):
+        for t in range(self.prefill, T):
             eng.decode(self.ckv, self.tokens, t, t + 1, max_tokens=T, forced=True, logits=self.logits, logits_row_offset=0,
                        kv=self.kv, scratch=self.scratch)
             L.check(eng.lib.mdc_beam_step(eng.handle, C.byref(self.state), C.c_void_p(self.logits.data_ptr() + t * row_bytes),
