@@ -74,7 +74,11 @@ int64_t mdc_ctx_launch_count(const mdc_ctx* ctx);
  *          MDC_F16  -> A,W and D IEEE half on the same kernel (bias / bias+ReLU epilogues only: the decoder prefill);
  *          MDC_F32  -> A,W f32, FFMA with fp32 accumulation in K order (the token-exact path).
  *   D is `dtype` for BIAS/GELU/RELU; for LS_RESIDUAL / PATCH the output is the f32 stream R.
- *   aux0: gamma f32[N] (LS_RESIDUAL) or pos f32[period,N] (PATCH); period: PATCH only.
+ *   aux0: gamma f32[N] (LS_RESIDUAL) or, for PATCH, the positional table: `period` rows of N f32 values with the
+ *         row stride of the output, ldd (pos[p][c] at aux0[p * ldd + c]); period: PATCH only.
+ *   Alignment: MDC_F32 needs A and W 16-byte aligned, MDC_BF16 on the FFMA kernel 8-byte aligned; the tensor-core kernel
+ *   (MDC_BF16 with K, lda, ldw, N multiples of 8, and MDC_F16) needs A, W and D 16-byte aligned, ldd % 8 == 0, and for
+ *   PATCH a 16-byte aligned aux0 and period >= 32.  Misaligned operands are rejected before any launch.
  */
 int mdc_gemm(mdc_ctx* ctx, int dtype, int epilogue,
              const void* A, int64_t lda, const void* W, int64_t ldw,
@@ -87,14 +91,18 @@ int mdc_gemm(mdc_ctx* ctx, int dtype, int epilogue,
  *   (ii)  timm Attention inside the ViT blocks (strip = 197 tokens, head_dim 64, scale 1/8),
  *   (iii) true row / column strips of a patch grid (strip_len 14, n_strips = B*14).
  * qkv: [n_strips*strip_len, 3*heads*head_dim] packed q|k|v (row stride ld_qkv), out:
- * [n_strips*strip_len, heads*head_dim].  softmax_over_queries != 0 selects softmax over the query
- * axis (AxialAttention.forward(axis=-2)); it requires strip_len <= 128.
+ * [n_strips*strip_len, heads*head_dim].  qkv must be 16-byte aligned and ld_qkv a multiple of 8.
+ * softmax_over_queries != 0 selects softmax over the query axis (AxialAttention.forward(axis=-2));
+ * it stages a whole strip in shared memory: strip_len <= 128, head_dim <= 128 and
+ * (n(n+1) + 3·n·head_dim)·4 bytes (n = strip_len) within the device's per-block limit (227 KB on
+ * a B200: n = 128 allows head_dim <= 104).
  */
 int mdc_strip_attention(mdc_ctx* ctx, int dtype, const void* qkv, int64_t ld_qkv, void* out, int64_t ld_out,
                         int n_strips, int strip_len, int heads, int head_dim, float scale,
                         int softmax_over_queries, void* stream);
 
-/* LayerNorm over the last axis of an f32 matrix, output `out_dtype` (timm norm1/norm2). */
+/* LayerNorm over the last axis of an f32 matrix, output `out_dtype` (timm norm1/norm2).
+ * x, w and b must be 16-byte aligned, cols and ldx multiples of 4; `out` may have any stride (element alignment only). */
 int mdc_layernorm(mdc_ctx* ctx, const float* x, int64_t ldx, const float* w, const float* b, float eps,
                   void* out, int64_t ldo, int out_dtype, int rows, int cols, void* stream);
 

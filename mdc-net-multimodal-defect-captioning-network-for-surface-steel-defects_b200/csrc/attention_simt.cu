@@ -176,10 +176,13 @@ int launch_rows(mdc_ctx* ctx, const void* qkv, int64_t ld, void* out, int64_t ld
   MDC_LAUNCH_CHECK(ctx); return 0;
 }
 
+// shared memory of strip_attn_colsoftmax_kernel: the score matrix S [n][n+1] and Q, K, V [n][hd]
+size_t cols_smem_bytes(int n, int hd) { return ((size_t)n * (n + 1) + 3 * (size_t)n * hd) * sizeof(float); }
+
 template <typename T>
 int launch_cols(mdc_ctx* ctx, const void* qkv, int64_t ld, void* out, int64_t ldo, int n_strips, int n, int heads, int hd,
                 float scale, cudaStream_t s) {
-  size_t smem = ((size_t)n * (n + 1) + 3 * (size_t)n * hd) * sizeof(float);
+  const size_t smem = cols_smem_bytes(n, hd);
   MDC_ENSURE_SMEM(strip_attn_colsoftmax_kernel<T>, smem);
   strip_attn_colsoftmax_kernel<T><<<dim3(heads, n_strips), 256, smem, s>>>((const T*)qkv, ld, (T*)out, ldo, n, heads, hd, scale);
   MDC_LAUNCH_CHECK(ctx); return 0;
@@ -203,10 +206,18 @@ extern "C" int mdc_strip_attention(mdc_ctx* ctx, int dtype, const void* qkv, int
   MDC_CHECK_ARG(dtype == MDC_F32 || dtype == MDC_BF16);
   MDC_CHECK_ARG(n_strips >= 0 && strip_len > 0 && heads > 0 && heads <= 65535 && n_strips <= 65535 * 32);
   MDC_CHECK_ARG(ld_qkv % 8 == 0 && head_dim % 8 == 0);
+  MDC_CHECK_ARG(((uintptr_t)qkv & 15) == 0);     // rows of q, k and v are read in 16-byte vectors (load8, TMA)
   if (n_strips == 0) return 0;
   cudaStream_t s = (cudaStream_t)stream;
   if (softmax_over_queries) {
     MDC_CHECK_ARG(strip_len <= 128 && head_dim <= 128);
+    // the whole strip is staged in shared memory: checked before any CUDA call that could fail on it
+    int smem_max = 0;
+    MDC_CUDA(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+    const size_t smem = cols_smem_bytes(strip_len, head_dim);
+    if (smem > (size_t)smem_max)
+      MDC_FAIL(-2, "strip_attention: softmax over queries stages (n(n+1) + 3 n head_dim) floats = %zu bytes of shared memory for "
+                   "n = %d, head_dim = %d; a block may use at most %d bytes", smem, strip_len, head_dim, smem_max);
     return dtype == MDC_F32 ? launch_cols<float>(ctx, qkv, ld_qkv, out, ld_out, n_strips, strip_len, heads, head_dim, scale, s)
                             : launch_cols<bf16>(ctx, qkv, ld_qkv, out, ld_out, n_strips, strip_len, heads, head_dim, scale, s);
   }

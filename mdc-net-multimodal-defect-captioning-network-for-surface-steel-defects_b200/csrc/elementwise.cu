@@ -328,10 +328,12 @@ extern "C" int mdc_layernorm(mdc_ctx* ctx, const float* x, int64_t ldx, const fl
   MDC_CHECK_ARG(ctx && x && w && b && out);
   MDC_CHECK_DEVICE(ctx);
   MDC_CHECK_ARG(cols % 4 == 0 && ldx % 4 == 0 && rows >= 0);
+  // both kernels read x, w and b as float4
+  MDC_CHECK_ARG(((uintptr_t)x & 15) == 0 && ((uintptr_t)w & 15) == 0 && ((uintptr_t)b & 15) == 0);
   if (rows == 0) return 0;
   cudaStream_t s = (cudaStream_t)stream;
   int grid = (rows + 7) / 8;
-  const bool vec_ok = ldo % 4 == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)x & 15) == 0 && ((uintptr_t)w & 15) == 0 && ((uintptr_t)b & 15) == 0;
+  const bool vec_ok = ldo % 4 == 0 && ((uintptr_t)out & 15) == 0;     // vector stores (fast path) or scalar stores (generic kernel)
 #define MDC_LN_FAST(NV_)                                                                                                        \
   if (vec_ok && cols == NV_ * 128) {                                                                                            \
     const int grid2 = (rows + 15) / 16;           /* two rows per warp */                                                        \

@@ -123,6 +123,8 @@ int gemm_simt_launch(mdc_ctx* ctx, int dtype, int epilogue, const void* A, int64
                      void* D, int64_t ldd, const float* bias, const float* aux0, int period, int M, int N, int K,
                      cudaStream_t s) {
   MDC_CHECK_ARG(K % 4 == 0 && lda % 4 == 0 && ldw % 4 == 0);
+  const uintptr_t vec_mask = dtype == MDC_F32 ? 15 : 7;      // A and W are read four elements at a time: float4 (f32) or uint2 (bf16)
+  MDC_CHECK_ARG(((uintptr_t)A & vec_mask) == 0 && ((uintptr_t)W & vec_mask) == 0);
   EpiParams ep{D, ldd, bias, aux0, period};
   if (dtype == MDC_F32) return launch_typed<float, float>(ctx, epilogue, A, lda, W, ldw, ep, M, N, K, s);
   return launch_typed<bf16, bf16>(ctx, epilogue, A, lda, W, ldw, ep, M, N, K, s);

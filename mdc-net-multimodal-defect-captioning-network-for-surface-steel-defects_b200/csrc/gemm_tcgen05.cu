@@ -458,6 +458,7 @@ int gemm_tc_launch(mdc_ctx* ctx, int epilogue, const void* A, int64_t lda, const
   MDC_CHECK_ARG(((uintptr_t)A & 15) == 0 && ((uintptr_t)W & 15) == 0 && ((uintptr_t)D & 15) == 0);
   MDC_CHECK_ARG(ldd % 8 == 0);
   if (epilogue == MDC_EPI_PATCH) MDC_CHECK_ARG(period >= 32);      // a 32-row epilogue chunk crosses at most one image boundary
+  if (epilogue == MDC_EPI_PATCH) MDC_CHECK_ARG(((uintptr_t)aux0 & 15) == 0);   // the positional rows are read as float4
   // tile width: the widest tile that still gives every SM one tile (128 x 256 tiles need 1/3 less operand traffic per flop than
   // 128 x 128 ones; with N = 512 that is 1.3 waves instead of 2.7 -- the same time for the kernel alone, ~1 % more images/s in the
   // batch pipeline, where co-scheduled kernels fill the tail and SM-time is what counts); narrow N uses narrow tiles

@@ -124,7 +124,14 @@ def test_layernorm(dtype):
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize("cfg", [(3, 197, 8, 64, 0.125), (2, 99, 8, 32, 0.125), (28, 14, 8, 64, 0.125), (2, 17, 2, 128, 0.3),
-                                 (1, 1025, 8, 64, 0.125), (2, 300, 8, 64, 0.125), (2, 208, 8, 64, 0.125), (2, 209, 8, 64, 0.125), (5, 1, 8, 32, 0.125)])
+                                 (1, 1025, 8, 64, 0.125), (2, 300, 8, 64, 0.125), (2, 208, 8, 64, 0.125), (2, 209, 8, 64, 0.125), (5, 1, 8, 32, 0.125),
+                                 # bf16 head width 64: the mma.sync kernel below 16 and above 256 tokens, the tcgen05 kernel at its bounds
+                                 (3, 1, 4, 64, 0.125), (3, 7, 4, 64, 0.125), (3, 15, 4, 64, 0.125), (3, 16, 4, 64, 0.125),
+                                 (2, 255, 4, 64, 0.125), (2, 256, 4, 64, 0.125), (2, 257, 4, 64, 0.125),
+                                 # many waves: the bench's 64 strips and config 5's 256 strips of 197 tokens
+                                 (64, 197, 8, 64, 0.125), (256, 197, 8, 64, 0.125),
+                                 # head widths 32 and 128 with keys over several 64-key tiles
+                                 (2, 300, 4, 32, 0.125), (2, 300, 2, 128, 0.125)])
 def test_strip_attention(dtype, cfg):
     n_strips, n, H, hd, scale = cfg
     qkv = _mk((n_strips * n, 3 * H * hd), dtype, 4)
